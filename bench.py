@@ -10,6 +10,11 @@ backward (reverse sweep through the solver) -> [gradient all-reduce] -> clip 1.0
 Workload at N=1 = BASELINE.json configs[1] (the C100 shape of SURVEY section 8: 224 px, patch 16,
 D=768, H=12, mlp_ratio 1, 10 registers, N=207 tokens, Euler over 24 grid points, 64 images per
 GPU), weak scaling over N.  One JSON line on stdout (rank 0).
+
+    python bench.py --steps K --dump-outputs DIR   # also write the last timed step's outputs as DIR/<name>.npy
+
+The inputs and the initial weights are seeded, so two builds run with the same arguments can be compared output for
+output (see `dump_outputs`).
 """
 from __future__ import annotations
 
@@ -23,6 +28,7 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 
+import numpy as np  # noqa: E402
 import torch  # noqa: E402
 import torch.distributed as dist  # noqa: E402
 
@@ -133,6 +139,41 @@ def synthetic_batch(cfg, B, seed_off=0):
     px = torch.randn(B, 3, S, S, generator=torch.Generator().manual_seed(1234 + seed_off))
     lb = torch.randint(0, C, (B,), generator=torch.Generator().manual_seed(1235 + seed_off))
     return px, lb
+
+
+DUMP_BUDGET_BYTES = 64 * 10**6
+
+
+def host_arrays(prefix, obj):
+    """{name: float32 host array} of every floating-point tensor in `obj` (a tensor or nested dicts of them)."""
+    if torch.is_tensor(obj):
+        return {prefix: obj.detach().float().cpu().numpy()} if obj.is_floating_point() else {}
+    out = {}
+    if isinstance(obj, dict):
+        for k, v in obj.items():
+            out.update(host_arrays(f"{prefix}.{k}" if prefix else str(k), v))
+    return out
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes every array as out_dir/<name>.npy in float32, DUMP_BUDGET_BYTES in all.  When the arrays are larger than
+    that, each array above a common element count is replaced by a sample of that many of its flattened elements: the
+    same positions (seeded, in ascending order) in every run, so that dumps of two builds still compare element for
+    element."""
+    os.makedirs(out_dir, exist_ok=True)
+    left = DUMP_BUDGET_BYTES // 4 - 32 * len(arrays)         # in elements; an .npy header is 128 bytes
+    sizes = sorted(a.size for a in arrays.values())
+    cap = None
+    for i, n in enumerate(sizes):                             # largest cap with sum(min(size, cap)) <= left
+        if n > left // (len(sizes) - i):
+            cap = left // (len(sizes) - i)
+            break
+        left -= n
+    for name, a in arrays.items():
+        a = np.asarray(a, dtype=np.float32)
+        if cap is not None and a.size > cap:
+            a = a.reshape(-1)[np.sort(np.random.default_rng(0).choice(a.size, cap, replace=False))]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 # ------------------------------------------------------------------------------------------------
@@ -317,12 +358,14 @@ def run_ours(args, wl):
     model = ob.ViTNeuralODE(**cfg).to(dev).train()      # the reference's own init (:494-513), dropout 0
     model.precision = args.precision
     params = [p for p in model.parameters() if p.requires_grad]
+    initial_params = [p.detach().clone() for p in params] if args.dump_outputs else None
     opt = torch.optim.AdamW(params, lr=1e-4, weight_decay=5e-2, fused=True, capturable=True)
     reducer = FlatGradAllReduce(params)
 
     px_h, lb_h = synthetic_batch(cfg, B, seed_off=rank)
     px_h, lb_h = px_h.pin_memory(), lb_h.pin_memory()
     px_d, lb_d = px_h.to(dev), lb_h.to(dev)
+    last = {}          # what the latest step returned (under graph replay: the captured step's output buffers)
 
     if wl.get("distill"):
         # the reference's trainer (loss_trainer.py:305-372 -> odevit_b200.loss_trainer) around the frozen teacher, whose
@@ -331,10 +374,14 @@ def run_ours(args, wl):
         trainer = ob.ImageDistilTrainer(teacher_model=teacher, student_model=model, optimizer=opt, **DISTILL_TRAINER)
 
         def loss_fn(m, px, lb):
-            return trainer.loss_only({"pixel_values": px}, lb, epoch=0)["loss"]
+            out = trainer.loss_only({"pixel_values": px}, lb, epoch=0)
+            last["logits"] = out["student_output"]["logits"].detach()   # not its autograd graph: that would keep the step's tape alive
+            return out["loss"]
     else:
         def loss_fn(m, px, lb):
-            return m(px, labels=lb)["loss"]
+            out = m(px, labels=lb)
+            last["logits"] = out["logits"].detach()   # not its autograd graph: that would keep the step's tape alive
+            return out["loss"]
 
     def step(px, lb):
         opt.zero_grad(set_to_none=True)
@@ -377,7 +424,7 @@ def run_ours(args, wl):
     # The timed steps replay ONE CUDA graph of forward + backward (then all-reduce, clipping, AdamW eagerly):
     # ~1200 launches per step leave sub-microsecond gaps that a replay closes.  Same kernels, same work; the
     # per-class roofline region below stays eager (it brackets every launch with events).
-    stepper, launch_mode, graph_launches = None, "eager", 0
+    stepper, launch_mode, graph_launches, graph_logits = None, "eager", 0, None
     if not args.no_graph and not args.quick:
         try:
             from odevit_b200.graphs import GraphedTrainStep
@@ -386,6 +433,7 @@ def run_ours(args, wl):
             stepper = GraphedTrainStep(model, opt, (px_d, lb_d), clip=1.0, warmup=1, capture_optimizer=False, loss_fn=loss_fn,
                                        grad_hook=(reducer if world > 1 and not os.environ.get("ODEVIT_BENCH_SKIP_ALLREDUCE") else None))
             graph_launches = ob.launch_count() // 2       # one warm-up step + the captured one
+            graph_logits = last["logits"]                 # the capture was the last forward: every replay rewrites it
             launch_mode = "cuda_graph_replay (forward+backward; all-reduce/clip/AdamW eager)"
         except Exception as e:  # noqa: BLE001
             import traceback
@@ -394,7 +442,11 @@ def run_ours(args, wl):
             torch.cuda.synchronize()
 
     def fast_step(px, lb):
-        return stepper(px, lb) if stepper is not None else step(px, lb)
+        if stepper is None:
+            last["loss"] = step(px, lb)
+        else:
+            last["loss"], last["logits"] = stepper(px, lb), graph_logits
+        return last["loss"]
     # per-class event pairs are created here, outside the timed region (cudaEventCreate can stall)
     ob.reset_launch_count()
     step(px_d, lb_d)
@@ -433,8 +485,32 @@ def run_ours(args, wl):
         e2e_region(1)
         ob.reset_launch_count()
     vals_v, vals_e = [], []
-    for _ in range(max(1, args.repeats)):
+    dumped = None
+    for r in range(max(1, args.repeats)):
+        if args.dump_outputs and r == max(1, args.repeats) - 1:
+            # The weight gradients are summed with float atomics, so their last bits vary from run to run, and AdamW's
+            # early updates (~lr * sign(g)) turn that into weight differences that grow step after step.  The dumped
+            # region therefore starts from the seeded weights and a fresh AdamW state (in place: the captured graph
+            # keeps these addresses): its first step has the same inputs in every run; with --steps above 1, the
+            # later steps inherit the rounding of the atomics again.
+            with torch.no_grad():
+                for p, p0 in zip(params, initial_params):
+                    p.copy_(p0)
+                for state in opt.state.values():
+                    for t in state.values():
+                        if torch.is_tensor(t):
+                            t.zero_()
+            torch.cuda.synchronize()
         vals_v.append(timed_once(lambda: fast_step(px_d, lb_d), args.steps))
+        if args.dump_outputs and rank == 0 and r == max(1, args.repeats) - 1:
+            # the last headline step: its loss and logits, the gradients it left and the weights after its AdamW update
+            # (copied now: the regions below keep training the same model)
+            dumped = host_arrays("", {"loss": last["loss"], "logits": last["logits"]})
+            for n, p in model.named_parameters():
+                if p.requires_grad:
+                    dumped.update(host_arrays(f"param.{n}", p))
+                    if p.grad is not None:
+                        dumped.update(host_arrays(f"grad.{n}", p.grad))
         if not args.quick:
             vals_e.append(e2e_region(args.steps))
     repeats_log["value"] = [round(v, 3) for v in vals_v]
@@ -572,6 +648,8 @@ def run_ours(args, wl):
             "cpu_baseline": cpu_baseline,
             "grad_allreduce_bytes": reducer.bucket_bytes if world > 1 else 0,
         }
+        if dumped is not None:
+            dump_outputs(args.dump_outputs, dumped)
         rk.emit(line)
     else:
         rk.emit({})
@@ -618,6 +696,11 @@ def run_infer(args, wl):
     sampler.start()
     rows, regions_log = [], {}
     head = None
+    last = {}
+
+    def forward():
+        last["out"] = model(px_d)
+
     with torch.no_grad():
         for solver, steps in points:
             model = build(solver, steps)
@@ -625,7 +708,7 @@ def run_infer(args, wl):
             for _ in range(max(3, args.warmup)):
                 model(px_d)
             gc.collect()
-            vals = sorted(region(lambda: model(px_d), args.steps) for _ in range(max(1, args.repeats)))
+            vals = sorted(region(forward, args.steps) for _ in range(max(1, args.repeats)))
             ms = vals[len(vals) // 2]
             tf = world * B * nfe * field_flops_fwd(cfg) / (ms * 1e-3) / 1e12
             rows.append({"solver": solver, "steps": steps, "ms_per_step": round(ms, 4), "img_per_s": world * B / ms * 1e3,
@@ -634,6 +717,8 @@ def run_infer(args, wl):
             regions_log[f"{solver}_{steps}"] = [round(v, 4) for v in vals]
             head = (model, solver, steps, nfe, ms)
         model, solver, steps, nfe, ms_step = head
+        # the last timed forward is the headline point's (the last point)
+        dumped = host_arrays("", last["out"]) if args.dump_outputs and rank == 0 else None
         # ---- end to end for the headline point: pinned host images in (prefetched one step ahead), logits out
         feeder = HostBatchPrefetcher(dev)
         out_h = torch.empty(B, cfg["num_classes"], dtype=torch.float32).pin_memory()
@@ -730,6 +815,8 @@ def run_infer(args, wl):
     }
     if sweep:
         line["sweep"] = rows
+    if dumped is not None:
+        dump_outputs(args.dump_outputs, dumped)
     rk.emit(line)
 
 
@@ -749,7 +836,16 @@ def main():
     ap.add_argument("--quick", action="store_true",
                     help="profiling helper (ncu launch lists): only the device-resident timed region, any warm-up count; "
                          "its JSON line is not a bench value")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step returned (training: loss, logits, gradients and the updated "
+                         "weights; inference: the forward's outputs) as DIR/<name>.npy, float32, at most 64 MB in all. "
+                         "Training: the last headline region (and every region after it) then starts from the seeded "
+                         "weights and a fresh AdamW state, so that the dump is comparable between runs")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     if args.quick:
         args.repeats = 1
     if args.impl == "ours" and not args.quick:
