@@ -20,7 +20,8 @@
  *
  * Conventions (SURVEY.md section 8b):
  *   - plain pointers and sizes only; no torch types; every device buffer, including the workspace,
- *     is owned by the caller; the library never allocates device memory and never synchronises;
+ *     is owned by the caller; the library never allocates device memory and never synchronises
+ *     (except odevit_solve_adaptive, which cannot know its number of rounds in advance);
  *   - all work is enqueued on `stream` and is asynchronous with respect to the host;
  *   - `t_grid` is a HOST pointer (the per-step dt = t[i+1]-t[i] is formed on the host in fp32,
  *     exactly as torchdiffeq forms it);
@@ -53,7 +54,9 @@ typedef enum {
   ODEVIT_ERR_WORKSPACE = -2,     /* workspace too small or misaligned                          */
   ODEVIT_ERR_CUDA = -3,          /* a CUDA runtime / driver call failed (sticky errors too)    */
   ODEVIT_ERR_UNSUPPORTED = -4,   /* shape outside what the kernels cover                       */
-  ODEVIT_ERR_NOT_DEVICE_PTR = -5 /* a host pointer was passed where device memory is required  */
+  ODEVIT_ERR_NOT_DEVICE_PTR = -5, /* a host pointer was passed where device memory is required */
+  ODEVIT_ERR_NOT_CONVERGED = -6   /* adaptive solve: max_num_steps, a non-finite error ratio or dt
+                                     underflow (the message names the image)                     */
 } odevit_status;
 
 typedef enum {
@@ -144,7 +147,8 @@ typedef enum {
   ODEVIT_WS_FIELD = 0,     /* odevit_field_fwd                                                 */
   ODEVIT_WS_SOLVE_FWD = 1, /* odevit_solve_fwd                                                 */
   ODEVIT_WS_SOLVE_BWD = 2, /* odevit_solve_bwd                                                 */
-  ODEVIT_WS_ENCODER_FWD = 3 /* odevit_encoder_fwd (method ignored)                             */
+  ODEVIT_WS_ENCODER_FWD = 3, /* odevit_encoder_fwd (method ignored)                            */
+  ODEVIT_WS_SOLVE_ADAPTIVE = 4 /* odevit_solve_adaptive (method ignored)                        */
 } odevit_ws_kind;
 
 /* ABI / build identification. */
@@ -268,6 +272,35 @@ int odevit_solve_fwd_lean(const odevit_desc* desc, const odevit_weights* w, int3
                           const int32_t* row_index_host, int32_t n_rows, float* fd_max, float* p_last,
                           float* jas_traj, int32_t jas_first_eval, int32_t jas_k, void* workspace,
                           size_t workspace_bytes, odevit_stream_t stream);
+
+/* Adaptive Dormand-Prince 5(4) solve with PER-IMAGE step control, inference only.  Replaces
+ * torchdiffeq.odeint(func, x0, t_out, method="dopri5", rtol, atol, options={first_step, max_num_steps}) with one
+ * difference of substance: torchdiffeq takes ONE RMS error norm over the whole batch, here every image b is solved on
+ * its own N*D elements (its own t, dt, accept/reject decisions and dense output), so a batch of one is the published
+ * algorithm and an image's result does not depend on its batch-mates.  Per image (torchdiffeq _impl/dopri5.py,
+ * rk_common.py, interp.py, misc.py): FSAL Dormand-Prince with Shampine's error estimate, ratio = RMS(err / (atol +
+ * rtol max(|y0|, |y1|))), accept iff ratio <= 1, _optimal_step_size(safety 0.9, ifactor 10, dfactor 0.2, order 5),
+ * _select_initial_step(order 4) when first_step <= 0, outputs written from the quartic interpolant of the accepted
+ * step that covers them (the solver does not step to them).  Time and dt are fp64 on the device; stage combines run
+ * in fp32 with dt cast, as torchdiffeq does.
+ *   t_out_host [n_out] fp32 HOST, strictly increasing, 2 <= n_out <= 4096 (decreasing grids are not supported);
+ *   max_num_steps: attempted steps per image over the WHOLE solve (torchdiffeq counts per output interval);
+ *   states [n_out,B,N,D] out: row 0 = x0, row i = the solution at t_out[i];
+ *   nfe, accepted, rejected [B] device int32 or NULL: field evaluations per image
+ *          (1 + (first_step <= 0) + 6 * (accepted + rejected)) and step counts.
+ * desc must have no dropout.  Workspace kind ODEVIT_WS_SOLVE_ADAPTIVE.  Returns ODEVIT_ERR_NOT_CONVERGED when an
+ * image exceeds max_num_steps, meets a non-finite error ratio or a dt that no longer advances t.
+ * SYNCHRONISATION: the one entry point of the library that waits for the device.  Each round (one attempted step of
+ * every image, six field evaluations of the batch) ends with a copy of its active-image count to pinned host memory;
+ * the host enqueues round r + 1 and then waits for round r's count (an event), so the device always has one round
+ * queued, and the last round enqueued is a no-op that the call also waits for.  A finished image keeps dt = 0 (its
+ * rounds are identity steps) until every image has finished.  Refused (ODEVIT_ERR_UNSUPPORTED) while `stream` is being
+ * captured into a CUDA graph. */
+int odevit_solve_adaptive(const odevit_desc* desc, const odevit_weights* w, const float* x0, const float* t_out_host,
+                          int32_t n_out, double rtol, double atol, double first_step /* <= 0: select */,
+                          int32_t max_num_steps, float* states /* [n_out,B,N,D] */, int32_t* nfe, int32_t* accepted,
+                          int32_t* rejected /* [B] device, or NULL */, void* workspace, size_t workspace_bytes,
+                          odevit_stream_t stream);
 
 /* 1 when odevit_solve_fwd runs this inference solve in the on-chip-state kernel (one persistent CTA per image,
  * trajectory rows written from shared memory): the caller then has no reason to prefer the trajectory-free form. */

@@ -104,6 +104,7 @@ const Tableau* tableau_for(int method) {
     default: return nullptr;
   }
 }
+}  // namespace
 
 // ------------------------------------------------------------------------------------------------
 // plan + workspace arena (structs in host.h)
@@ -186,7 +187,7 @@ StageCtx take_ctx(const Plan& p, Arena& a, bool with_hpre) {
   return c;
 }
 
-static void split_scratch(const Plan& p, Arena& a) {
+void split_scratch(const Plan& p, Arena& a) {
   p.split_a = p.split_b = nullptr;
   p.split_a_bytes = p.split_b_bytes = 0;
   static const bool off = [] { const char* e = getenv("ODEVIT_FP32_SPLIT"); return e && e[0] == '0'; }();
@@ -354,6 +355,7 @@ int prepare_weights(const Plan& p, const odevit_weights* w, WeightBufs& wb, cuda
   return fold_weights_parallel(f, s);
 }
 
+namespace {
 // q / k / v views of the packed qkv buffer for batch z = (image b, head h)
 struct HeadView {
   long long bo, bi, rs;
@@ -606,17 +608,14 @@ int attention_vjp(const Plan& p, const void* qkv_v, const void* oh, long long ld
   return 0;
 }
 
-namespace {
-
 // Forward evaluation at stage input `u`.  `rk` (nullable) is the epilogue of the last GEMM.
 // xc_mode: XC_CENTRE forms c.xc = u - mean_D(u); XC_READY: c.xc already holds the activation-type copy of u, written by
 // the epilogue that produced u (see operand_from_epilogue: the rows of W1cat are centred, so the operand needs no
 // centring of its own); XC_COPY forms that same plain copy here (a recomputing reverse sweep reproducing such a forward
 // from a trajectory row).
-enum { XC_CENTRE = 0, XC_READY = 1, XC_COPY = 2 };
 int eval_forward(const Plan& p, const WeightBufs& wb, const StageCtx& c, const float* u, float* P,
                  float* p_copy, float* sq, float* tmp, long long e, const Epi* rk, cudaStream_t s,
-                 float* jas_out = nullptr, int jas_k = 0, int xc_mode = XC_CENTRE) {
+                 float* jas_out, int jas_k, int xc_mode) {
   if (p.variant == ODEVIT_FIELD_MACARON) return macaron_forward(p, wb, c, u, P, rk, e, s);
   const int D = p.D, hid = p.hid, R = 3 * D + hid, K2 = D + hid;
   if (xc_mode != XC_READY) ODV_TRY(center_rows(u, c.xc, p.act, nullptr, 0.f, p.M, D, s, xc_mode == XC_CENTRE));
@@ -688,6 +687,7 @@ int eval_forward(const Plan& p, const WeightBufs& wb, const StageCtx& c, const f
   return 0;
 }
 
+namespace {
 // The stage-combine epilogue can write the NEXT evaluation's GEMM operand (the bf16 copy of the stage input it produces)
 // next to the fp32 value: with the centring folded into W1cat's rows (rows.cu::fold_w1_kernel) that copy needs no
 // `center_rows` pass (-10.6 us per evaluation for +1.5 us in the GEMM when timed kernel by kernel; the whole bench step does
@@ -1030,6 +1030,8 @@ size_t odevit_workspace_bytes(const odevit_desc* desc, int32_t ws_kind, int32_t 
   } else if (ws_kind == ODEVIT_WS_ENCODER_FWD) {
     if (encoder_plan(desc, &p)) return 0;
     layout_encoder(p, a);
+  } else if (ws_kind == ODEVIT_WS_SOLVE_ADAPTIVE) {
+    a.off = solve_adaptive_workspace_bytes(p);
   } else {
     const Tableau* tb = tableau_for(method);
     if (!tb) { set_error(ODEVIT_ERR_INVALID_ARG, "unknown method %d", method); return 0; }

@@ -73,10 +73,12 @@ __device__ __forceinline__ void epi_apply(const Epi& e, int m, int n, float acc,
     if (e.resid) v = fmaf(e.resid_coef, e.resid[idx], v);
     if (e.k_store) e.k_store[idx] = v;
     float r = e.c_new * v;
-    if (e.y) r = fmaf(e.y_coef, e.y[idx], r);
+    if constexpr ((EPI & EPI_ROWDT) == 0)
+      if (e.y) r = fmaf(e.y_coef, e.y[idx], r);
 #pragma unroll
     for (int i = 0; i < Epi::kMaxTerms; ++i)
       if (e.kin[i]) r = fmaf(e.c_k[i], e.kin[i][idx], r);
+    if constexpr ((EPI & EPI_ROWDT) != 0) r = fmaf((float)e.row_dt[m / e.rows_per_image], r, e.y_coef * e.y[idx]);
     if (e.out) reinterpret_cast<float*>(e.out)[idx] = r;
     if (e.out2) store_elem(e.out2, idx, e.aux_type, e.out2_scale * r);
     if (e.fd_out)   // (CUDA-core path: one atomic per element; the tcgen05 epilogue reduces over the row first)
@@ -200,10 +202,12 @@ __device__ __forceinline__ void epi_chunk16(const Epi& e, int m, int n, float* v
     if (e.k_store) store16(e.k_store, idx, DT_F32, v);
 #pragma unroll
     for (int j = 0; j < 16; ++j) r[j] = e.c_new * v[j];
-    if (e.y) {
-      load16(e.y, idx, DT_F32, t);
+    if constexpr ((EPI & EPI_ROWDT) == 0) {
+      if (e.y) {
+        load16(e.y, idx, DT_F32, t);
 #pragma unroll
-      for (int j = 0; j < 16; ++j) r[j] = fmaf(e.y_coef, t[j], r[j]);
+        for (int j = 0; j < 16; ++j) r[j] = fmaf(e.y_coef, t[j], r[j]);
+      }
     }
 #pragma unroll
     for (int i = 0; i < Epi::kMaxTerms; ++i) {
@@ -212,6 +216,12 @@ __device__ __forceinline__ void epi_chunk16(const Epi& e, int m, int n, float* v
 #pragma unroll
         for (int j = 0; j < 16; ++j) r[j] = fmaf(e.c_k[i], t[j], r[j]);
       }
+    }
+    if constexpr ((EPI & EPI_ROWDT) != 0) {
+      const float dtb = (float)e.row_dt[m / e.rows_per_image];
+      load16(e.y, idx, DT_F32, t);
+#pragma unroll
+      for (int j = 0; j < 16; ++j) r[j] = fmaf(dtb, r[j], e.y_coef * t[j]);
     }
     if (e.out) store16(e.out, idx, DT_F32, r);
     if (e.out2) {
@@ -572,9 +582,11 @@ __device__ __forceinline__ void epi8_finish(const Epi& e, int m0, int M, int n, 
       }
 #pragma unroll
       for (int i = 0; i < 4; ++i) r[i] = scale4(e.c_new, v[i]);
-      if (e.y) {
+      if constexpr ((EPI & EPI_ROWDT) == 0) {
+        if (e.y) {
 #pragma unroll
-        for (int i = 0; i < 4; ++i) r[i] = fma4(e.y_coef, raw_f32(pre.a[4 * h + i]), r[i]);
+          for (int i = 0; i < 4; ++i) r[i] = fma4(e.y_coef, raw_f32(pre.a[4 * h + i]), r[i]);
+        }
       }
 #pragma unroll 1   // (rolled: ONE operand batch live at a time)
       for (int k = 0; k < Epi::kMaxTerms; ++k) {
@@ -585,6 +597,14 @@ __device__ __forceinline__ void epi8_finish(const Epi& e, int m0, int M, int n, 
           const float ck = e.c_k[k];
 #pragma unroll
           for (int i = 0; i < 4; ++i) r[i] = fma4(ck, raw_f32(t[i]), r[i]);
+        }
+      }
+      if constexpr ((EPI & EPI_ROWDT) != 0) {   // r = y_coef*y + dt_b*(c_new*v + sum c_k k); rows past M read image 0
+#pragma unroll
+        for (int i = 0; i < 4; ++i) {
+          const int m = m0 + 4 * (4 * h + i);
+          const float dtb = (float)e.row_dt[row_in<FULL>(m0, 4 * h + i, M) ? m / e.rows_per_image : 0];
+          r[i] = fma4(dtb, r[i], scale4(e.y_coef, raw_f32(pre.a[4 * h + i])));
         }
       }
       if constexpr ((EPI & EPI_FD) != 0) {

@@ -108,7 +108,11 @@ int gemm_simt(const GemmArgs& g, cudaStream_t s) {
       else gemm_simt_kernel<EPI_FWD1><<<grid, 256, 0, s>>>(g);
       break;
     case EPI_RK:
-      if (g.epi.drop.thresh) gemm_simt_kernel<EPI_RK | EPI_DROP><<<grid, 256, 0, s>>>(g);
+      if (g.epi.row_dt) {
+        if (g.epi.drop.thresh || !g.epi.y)
+          return set_error(ODEVIT_ERR_INVALID_ARG, "gemm_simt: the per-image step epilogue needs y and no dropout");
+        gemm_simt_kernel<EPI_RK | EPI_ROWDT><<<grid, 256, 0, s>>>(g);
+      } else if (g.epi.drop.thresh) gemm_simt_kernel<EPI_RK | EPI_DROP><<<grid, 256, 0, s>>>(g);
       else gemm_simt_kernel<EPI_RK><<<grid, 256, 0, s>>>(g);
       break;
     case EPI_BWD3:

@@ -464,6 +464,11 @@ int launch_epi(int epi_mode, bool mn, const CUtensorMap& ta, const CUtensorMap& 
           return set_error(ODEVIT_ERR_INVALID_ARG, "gemm_tc: the finite-difference epilogue needs y, fd_prev, N %% 32 == 0 and no dropout");
         return launch_major<CG, BN, EPI_RK | EPI_FD>(mn, ta, tb, d, units, s);
       }
+      if (d.epi.row_dt) {
+        if (d.epi.drop.thresh || !d.epi.y)
+          return set_error(ODEVIT_ERR_INVALID_ARG, "gemm_tc: the per-image step epilogue needs y and no dropout");
+        return launch_major<CG, BN, EPI_RK | EPI_ROWDT>(mn, ta, tb, d, units, s);
+      }
       if (d.epi.drop.thresh) return launch_major<CG, BN, EPI_RK | EPI_DROP>(mn, ta, tb, d, units, s);
       return launch_major<CG, BN, EPI_RK>(mn, ta, tb, d, units, s);
     case EPI_BWD3:
@@ -556,6 +561,7 @@ bool gemm_tc_supports(const GemmArgs& g) {
   if (g.M <= 0 || g.N <= 0 || g.K <= 0) return false;
   if (g.N % 16) return false;
   if (g.epi.fd_out && (g.N % 32 || g.epi.drop.thresh)) return false;
+  if (g.epi.row_dt && (g.epi.fd_out || g.epi.drop.thresh)) return false;   // (those combinations are not instantiated)
   if (g.epi.exact_gelu && g.epi.drop.thresh) return false;   // (that combination is not instantiated)
   if ((g.epi.colsum_a || g.epi.colsum_b) && (g.epi_mode != EPI_BWD3 || g.N % 32 || g.epi.split % 32)) return false;   // whole warps reduce over rows: no dead lanes
   const bool a_k = (g.a_cs == 1), a_mn = (g.a_rs == 1 && g.a_cs != 1);

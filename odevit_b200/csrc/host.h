@@ -86,6 +86,22 @@ struct BwdBufs {
 // GEMM dispatch: tcgen05 in bf16 mode where the kernel covers the problem, FFMA otherwise.
 int gemm(const Plan& p, const GemmArgs& g, cudaStream_t s);
 
+// Plan, workspace pieces, argument checks and weight preparation shared by the solve entry points (api.cu).
+int make_plan(const odevit_desc* desc, Plan* p);
+WeightBufs take_weights(const Plan& p, Arena& a);
+StageCtx take_ctx(const Plan& p, Arena& a, bool with_hpre);
+void split_scratch(const Plan& p, Arena& a);   // fp32 mode: bf16 split scratch of the tensor-core GEMMs
+int check_ws(const void* ws, size_t have, size_t need);
+int check_device_ptr(const void* p, const char* what);
+int check_weights(const Plan& p, const odevit_weights* w);
+int prepare_weights(const Plan& p, const odevit_weights* w, WeightBufs& wb, cudaStream_t s);
+
+// One forward field evaluation at `u` (api.cu); `rk` (nullable) is the epilogue of its last GEMM.
+enum { XC_CENTRE = 0, XC_READY = 1, XC_COPY = 2 };
+int eval_forward(const Plan& p, const WeightBufs& wb, const StageCtx& c, const float* u, float* P,
+                 float* p_copy, float* sq, float* tmp, long long e, const Epi* rk, cudaStream_t s,
+                 float* jas_out = nullptr, int jas_k = 0, int xc_mode = XC_CENTRE);
+
 // softmax(q k^T) v per (image, head) from the packed qkv buffer into oh[:, h*d ...] (leading dim ld_oh).
 // P: [B,H,N,N] fp32 scratch (unfused path); p_copy: optional export; lse: optional row log-sum-exp.
 int attention_forward(const Plan& p, const void* qkv, void* oh, long long ld_oh, float* P, float* p_copy,
@@ -106,6 +122,9 @@ size_t solve_resident_scratch_floats(const Plan& p);
 int solve_resident(const Plan& p, const WeightBufs& wb, int S, const float (*ta)[4], const float* tbv, const float* x0,
                    const float* t_host, int n_grid, float* states, float* final_state, float* p_last, float* kbuf,
                    cudaStream_t s);
+
+// Adaptive Dormand-Prince solve (solve_adaptive.cu): bytes of its workspace layout (ODEVIT_WS_SOLVE_ADAPTIVE)
+size_t solve_adaptive_workspace_bytes(const Plan& p);
 
 // MACARON field (field_macaron.cu)
 int macaron_forward(const Plan& p, const WeightBufs& wb, const StageCtx& c, const float* u, float* P,

@@ -107,7 +107,10 @@ enum EpiMode : int {
   // Epi::fd_out (trajectory-free inference: ode_transformer_gpt.py:529-543 without the [T,B,N,D] tensor)
   EPI_FD = 16,
   // template-only flag (EPI_FWD1 / EPI_BWD3): erf-form GELU instead of the fitted logistic form (the fp32 mode)
-  EPI_EXACT = 32
+  EPI_EXACT = 32,
+  // template-only flag (EPI_RK): per-image step size, r = y_coef*y + dt_b*(c_new*v + sum_i c_k[i]*kin[i]) with
+  // dt_b = (float)Epi::row_dt[m / rows_per_image] (the adaptive solve: the host passes the tableau without dt)
+  EPI_ROWDT = 64
 };
 
 // One dropout site of one field evaluation: element (r, c) is kept iff hash(key, r, c) >= thresh and then
@@ -170,6 +173,10 @@ struct Epi {
   // needs N % 32 == 0 and split % 32 == 0: whole warps reduce)
   float* colsum_a = nullptr;
   float* colsum_b = nullptr;
+  // EPI_RK with EPI_ROWDT: per-image step sizes [B] (fp64, cast to fp32 as torchdiffeq casts dt to the state's type);
+  // row m belongs to image m / rows_per_image.  Needs y.
+  const double* row_dt = nullptr;
+  int rows_per_image = 1;
 };
 
 struct GemmArgs {

@@ -565,11 +565,12 @@ __global__ void __launch_bounds__(256) ln_bwd_rows_kernel(LnBwdArgs a, int rows,
   }
 }
 
+template <int EPI>
 __global__ void __launch_bounds__(256) rk_apply_kernel(const __grid_constant__ Epi e, const float* __restrict__ v,
                                                        long long n, int D) {
   long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   const long long stride = (long long)gridDim.x * blockDim.x;
-  for (; i < n; i += stride) epi_apply<EPI_RK, false>(e, (int)(i / D), (int)(i % D), v[i], 0, 0);
+  for (; i < n; i += stride) epi_apply<EPI, false>(e, (int)(i / D), (int)(i % D), v[i], 0, 0);
 }
 
 // ---- L2 attention pieces ---------------------------------------------------------------------
@@ -1184,7 +1185,12 @@ int rk_apply_rows(const Epi& e, const float* v, int rows, int D, cudaStream_t s)
   e2.alpha = 1.f; e2.bias = nullptr; e2.dev_scale = nullptr; e2.resid = nullptr; e2.ld_out = D;
   const long long n = (long long)rows * D;
   const int blocks = (int)((n + 255) / 256 < 148 * 8 ? (n + 255) / 256 : 148 * 8);
-  rk_apply_kernel<<<blocks > 0 ? blocks : 1, 256, 0, s>>>(e2, v, n, D);
+  if (e2.row_dt) {
+    if (!e2.y) return set_error(ODEVIT_ERR_INVALID_ARG, "rk_apply_rows: the per-image step combine needs y");
+    rk_apply_kernel<EPI_RK | EPI_ROWDT><<<blocks > 0 ? blocks : 1, 256, 0, s>>>(e2, v, n, D);
+  } else {
+    rk_apply_kernel<EPI_RK><<<blocks > 0 ? blocks : 1, 256, 0, s>>>(e2, v, n, D);
+  }
   ODV_LAUNCH_CHECK();
   return 0;
 }

@@ -19,7 +19,7 @@ import torch.nn as nn
 import torch.nn.functional as F
 
 from . import _lib, ops
-from .vit_ode import DEFAULT_PRECISION, _next_drop_seed
+from .vit_ode import DEFAULT_PRECISION, _next_drop_seed, adaptive_solve_args
 
 
 class PatchEmbed(nn.Module):
@@ -178,6 +178,9 @@ class ViTMacaron(nn.Module):
         self.time_interval = time_interval
         self.num_eval_steps = num_eval_steps
         self.t_grid = torch.linspace(0.0, time_interval, num_eval_steps)
+        # None, or {"rtol", "atol"[, "first_step", "max_num_steps"]}: forward integrates over t_grid with the per-image
+        # adaptive Dormand-Prince solve (inference only; a plain attribute like `precision`, not a config key)
+        self.adaptive_solve = None
         self._init_weights()
 
     # -- precision switch (not in the reference) -------------------------------------------------
@@ -238,6 +241,8 @@ class ViTMacaron(nn.Module):
                 t_grid: Optional[torch.Tensor] = None, temperature: Optional[float] = 100.0):
         """:302-352."""
         block = self.odefunc.block
+        if self.adaptive_solve is not None:
+            cfg = adaptive_solve_args(self, {})
         tokens = self.embed(pixel_values)
         if t_grid is None:
             num_eval_steps, t = self.num_eval_steps, self.t_grid
@@ -251,10 +256,19 @@ class ViTMacaron(nn.Module):
                 raise IndexError(f"control point index {int(idx.max())} is out of bounds for a trajectory of "
                                  f"{num_eval_steps} states (the reference's states[control_points] fails alike)")
             idx = idx % num_eval_steps
-        res = ops.ode_solve(tokens, t, block.field_spec(self.odefunc.scaler), self.solver, block.field_weights(),
-                            row_index=idx.tolist() if idx is not None else ())
+        if self.adaptive_solve is not None:
+            res = ops.ode_solve_adaptive(tokens, t, block.field_spec(self.odefunc.scaler), block.field_weights(),
+                                         cfg["rtol"], cfg["atol"], first_step=cfg.get("first_step"),
+                                         max_num_steps=cfg.get("max_num_steps", ops.DOPRI5_MAX_NUM_STEPS))
+            if idx is not None:
+                res["rows"] = res["states"][idx]
+        else:
+            res = ops.ode_solve(tokens, t, block.field_spec(self.odefunc.scaler), self.solver, block.field_weights(),
+                                row_index=idx.tolist() if idx is not None else ())
         states, final = res["states"], res["final"]
         out = {"logits": self.head(self.norm_head(final[:, 0]))}
+        if self.adaptive_solve is not None:
+            out["nfe"] = res["nfe"]
         if self.add_distillation_token:
             out["logits_dist"] = self.dist_head(self.norm_dist(final[:, 1]))
         if labels is not None:

@@ -5,6 +5,7 @@ current CUDA stream.  PyTorch is plumbing here (device memory, streams, autograd
 Replaces, for CUDA tensors:
   * `ViT_ODEFunc.forward(t, x)`                         models/ode_transformer_gpt.py:317-330
   * `torchdiffeq.odeint(func, y0, t, method=...)`        models/ode_transformer_gpt.py:571-578
+  * `torchdiffeq.odeint(..., method="dopri5")` with the error norm taken per image (ode_solve_adaptive)
   * autograd through both (backprop-through-solver)      train.py:57-67
 """
 from __future__ import annotations
@@ -510,6 +511,57 @@ def ode_solve_lean(x0: torch.Tensor, t: torch.Tensor, spec: FieldSpec, method: s
     _lib.check(st, "odevit_solve_fwd_lean")
     return {"states": None, "final": final, "rows": rows, "fd_max": fd_max, "p_last": p_last, "p_traj": None,
             "jas_traj": jas_traj}
+
+
+class NotConvergedError(OdevitError):
+    """The adaptive solve stopped: an image exceeded max_num_steps, met a non-finite error ratio or a dt that no longer
+    advances t (the message names the image)."""
+
+
+DOPRI5_MAX_NUM_STEPS = 2 ** 31 - 1   # torchdiffeq's default
+
+
+def ode_solve_adaptive(x0: torch.Tensor, t: torch.Tensor, spec: FieldSpec, weights: Dict[str, Optional[torch.Tensor]],
+                       rtol: float, atol: float, first_step: Optional[float] = None,
+                       max_num_steps: int = DOPRI5_MAX_NUM_STEPS):
+    """Adaptive Dormand-Prince 5(4) solve with per-image step control (odevit_solve_adaptive), inference only.
+
+    torchdiffeq's dopri5 run on every image on its own: the error norm, the accept / reject decisions, the step sizes
+    and the dense output of image b depend on image b alone (torchdiffeq takes one norm over the whole batch).  `t`
+    must be strictly increasing; `max_num_steps` bounds the attempted steps per image over the whole solve (torchdiffeq
+    counts them per output interval).  Synchronises with the device once per round (one attempted step of every image).
+
+    Returns dict(states [len(t),B,N,D] (row i = solution at t[i]), final [B,N,D], nfe [B], accepted [B], rejected [B]
+    (int32, device), rounds (int: rounds with at least one image still stepping = max_b accepted + rejected))."""
+    names = tuple(k for k, v in weights.items() if v is not None)
+    if torch.is_grad_enabled() and (x0.requires_grad or any(weights[k].requires_grad for k in names)):
+        raise OdevitError("the adaptive solve is inference-only (no backward is built): run it under torch.no_grad() "
+                          "or detach x0 and the weights")
+    if spec.has_dropout:
+        raise OdevitError("the adaptive solve is inference-only: the field's dropout must be 0 (call .eval())")
+    x0 = _require_cuda(x0.detach(), "x0")
+    B, N, D = x0.shape
+    t_host = t.detach().to("cpu", torch.float32).contiguous()
+    T = int(t_host.numel())
+    t_c = (ctypes.c_float * max(1, T))(*t_host.tolist())
+    desc = spec.desc(B, N)
+    w, keep = _pack_weights(names, [weights[k].detach() for k in names])
+    states = torch.empty(T, B, N, D, device=x0.device, dtype=torch.float32)
+    counts = torch.zeros(3, B, device=x0.device, dtype=torch.int32)
+    buf, ws, ws_bytes = _workspace(desc, _lib.WS_SOLVE_ADAPTIVE, 0, x0.device)
+    fs = 0.0 if first_step is None else float(first_step)
+    if first_step is not None and not fs > 0:
+        raise ValueError(f"first_step must be > 0, got {first_step}")
+    with torch.cuda.device(x0.device):
+        st = _lib.lib().odevit_solve_adaptive(ctypes.byref(desc), ctypes.byref(w), _ptr(x0), t_c, T, float(rtol),
+                                              float(atol), fs, int(max_num_steps), _ptr(states), _ptr(counts[0]),
+                                              _ptr(counts[1]), _ptr(counts[2]), ws, ws_bytes, _stream())
+    if st == _lib.ERR_NOT_CONVERGED:
+        raise NotConvergedError(_lib.lib().odevit_last_error_string().decode("utf-8", "replace"))
+    _lib.check(st, "odevit_solve_adaptive")
+    rounds = int((counts[1] + counts[2]).max().item())
+    return {"states": states, "final": states[-1], "nfe": counts[0], "accepted": counts[1], "rejected": counts[2],
+            "rounds": rounds}
 
 
 def fd_curvature(states: torch.Tensor, delta_t: float) -> torch.Tensor:

@@ -228,6 +228,48 @@ def odeint(func: ViT_ODEFunc, y0: torch.Tensor, t: torch.Tensor, *, method: str 
     return res["states"]
 
 
+def _check_field_module(func, who: str) -> None:
+    if not (hasattr(func, "block") and hasattr(func.block, "field_spec") and hasattr(func, "scaler")):
+        raise TypeError(f"odevit_b200.{who} integrates odevit_b200 vector-field modules only "
+                        "(there is no generic / CPU solver in this package)")
+
+
+def odeint_adaptive(func, y0: torch.Tensor, t: torch.Tensor, *, rtol: float = 1e-7, atol: float = 1e-9,
+                    options: Optional[dict] = None, return_stats: bool = False):
+    """`torchdiffeq.odeint(func, y0, t, method="dopri5", rtol, atol, options)` for the fused vector field, with the
+    step size controlled PER IMAGE (ops.ode_solve_adaptive): image b's error norm, steps and dense output depend on
+    image b alone, where torchdiffeq takes one norm over the batch.  Inference only; `t` strictly increasing;
+    options: `first_step`, `max_num_steps` (attempted steps per image over the whole solve, not per output interval).
+    Exports no attention maps.  Returns the trajectory [len(t), *y0.shape], or (trajectory, stats) with stats =
+    dict(nfe, accepted, rejected: int32 [B] device tensors, rounds: int) when `return_stats`."""
+    _check_field_module(func, "odeint_adaptive")
+    options = dict(options or {})
+    unknown = set(options) - {"first_step", "max_num_steps"}
+    if unknown:
+        raise ValueError(f"unsupported dopri5 options {sorted(unknown)}; first_step and max_num_steps are built")
+    res = ops.ode_solve_adaptive(y0, t, func.block.field_spec(func.scaler), func.block.field_weights(), rtol, atol,
+                                 first_step=options.get("first_step"),
+                                 max_num_steps=options.get("max_num_steps", ops.DOPRI5_MAX_NUM_STEPS))
+    if return_stats:
+        return res["states"], {k: res[k] for k in ("nfe", "accepted", "rejected", "rounds")}
+    return res["states"]
+
+
+def adaptive_solve_args(model: nn.Module, output_flags: Dict[str, bool]) -> dict:
+    """Checks a model's `adaptive_solve` request (a dict with rtol, atol and optionally first_step, max_num_steps) and
+    the forward's arguments against what the adaptive solve can give."""
+    cfg = dict(model.adaptive_solve)
+    unknown = set(cfg) - {"rtol", "atol", "first_step", "max_num_steps"}
+    if unknown or "rtol" not in cfg or "atol" not in cfg:
+        raise ValueError(f"adaptive_solve takes rtol, atol [, first_step, max_num_steps], got {sorted(model.adaptive_solve)}")
+    for name, on in output_flags.items():
+        if on:
+            raise ValueError(f"{name} is not available with adaptive_solve (the adaptive solve exports no attention maps)")
+    if torch.is_grad_enabled() and any(p.requires_grad for p in model.parameters()):
+        raise RuntimeError("adaptive_solve is inference-only (no backward is built): run the model under torch.no_grad()")
+    return cfg
+
+
 class PatchEmbed(nn.Module):
     """ode_transformer_gpt.py:86-182 -- conv patchify, [cls | (dist) | patches | registers], learned
     positional embedding over all tokens or over cls+patches only.  (Row f1 of SURVEY section 8:
@@ -321,6 +363,9 @@ class ViTNeuralODE(nn.Module):
         self.time_interval = time_interval
         self.num_eval_steps = num_eval_steps
         self.t_grid = torch.linspace(0.0, time_interval, num_eval_steps)  # plain attribute, not a buffer
+        # None, or {"rtol", "atol"[, "first_step", "max_num_steps"]}: forward integrates over t_grid with the per-image
+        # adaptive Dormand-Prince solve (inference only; a plain attribute like `precision`, not a config key)
+        self.adaptive_solve = None
         self.patch_embed.precision = self.odefunc.block.precision
         self.apply(self._spectral_init)
 
@@ -437,11 +482,17 @@ class ViTNeuralODE(nn.Module):
         caller can observe (last one for `attentions`, the JaSMin window, all on request)."""
         block = self.odefunc.block
         R = self.patch_embed.num_register_tokens
+        if self.adaptive_solve is not None:
+            cfg = adaptive_solve_args(self, {"output_attentions": output_attentions,
+                                             "output_attention_trajectory": output_attention_trajectory})
         tokens = self.patch_embed(pixel_values)
         if t_grid is None:
             num_eval_steps, t = self.num_eval_steps, self.t_grid
         else:
             num_eval_steps, t = len(t_grid), t_grid
+        if self.adaptive_solve is not None:
+            return self._forward_adaptive(tokens, t, num_eval_steps, cfg, labels, output_hidden_states,
+                                          output_control_points, temperature, jasmin_k)
         stages = _lib.STAGES.get(self.solver)
         if stages is None:
             raise ValueError(f"unsupported solver {self.solver!r}")
@@ -531,4 +582,35 @@ class ViTNeuralODE(nn.Module):
         if output_control_points:
             out["control_points"] = res["rows"][:, :, :-R]
         self.odefunc.attention_trajectory = []   # :641-643
+        return out
+
+    def _forward_adaptive(self, tokens, t, num_eval_steps, cfg, labels, output_hidden_states, output_control_points,
+                          temperature, jasmin_k):
+        """forward() with `adaptive_solve` set: the trajectory over t comes from the dense output of the per-image
+        adaptive solve; the finite-difference bound is taken on it; `nfe` [B] is added to the output."""
+        R = self.patch_embed.num_register_tokens
+        res = ops.ode_solve_adaptive(tokens, t, self.odefunc.block.field_spec(self.odefunc.scaler),
+                                     self.odefunc.block.field_weights(), cfg["rtol"], cfg["atol"],
+                                     first_step=cfg.get("first_step"),
+                                     max_num_steps=cfg.get("max_num_steps", ops.DOPRI5_MAX_NUM_STEPS))
+        states, final = res["states"], res["final"]
+        logits = self.head(final[:, 0])
+        out = {
+            "logits": logits,
+            "second_derivative_upper_bound": self.compute_upper_bound_by_second_derivative(R=jasmin_k, L=1 / 2),
+            "finite_difference_upper_bound": self.compute_upper_bound_by_fininte_difference(
+                states, 0.5, 1 / self.num_eval_steps),
+            "nfe": res["nfe"],
+        }
+        if self.add_distillation_token:
+            out["logits_dist"] = self.dist_head(final[:, 1])
+        if labels is not None:
+            out["loss"] = F.cross_entropy(logits, labels, label_smoothing=0.05)
+        if output_hidden_states:
+            out["states"] = states
+        if output_control_points:
+            idx = self.get_proportional_control_points_with_temperature(temperature=temperature,
+                                                                        num_eval_steps=num_eval_steps)
+            out["control_points"] = states[idx][:, :, :-R]
+        self.odefunc.attention_trajectory = []
         return out
