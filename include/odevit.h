@@ -17,11 +17,14 @@
  *   odevit_solve_bwd   <-  loss.backward() through that call     train.py:57-67, loss_trainer.py:365
  *                          (reference gradient mode: autograd through the unrolled solver; here a
  *                           reverse sweep that recomputes each step from the stored trajectory row)
+ *   odevit_solve_adaptive[_record] / odevit_solve_adaptive_bwd
+ *                      <-  odeint(..., method="dopri5") with the error norm taken per image, and loss.backward()
+ *                          through it with the accepted steps frozen (not part of the reference)
  *
  * Conventions (SURVEY.md section 8b):
  *   - plain pointers and sizes only; no torch types; every device buffer, including the workspace,
  *     is owned by the caller; the library never allocates device memory and never synchronises
- *     (except odevit_solve_adaptive, which cannot know its number of rounds in advance);
+ *     (except odevit_solve_adaptive[_record], which cannot know its number of rounds in advance);
  *   - all work is enqueued on `stream` and is asynchronous with respect to the host;
  *   - `t_grid` is a HOST pointer (the per-step dt = t[i+1]-t[i] is formed on the host in fp32,
  *     exactly as torchdiffeq forms it);
@@ -148,7 +151,8 @@ typedef enum {
   ODEVIT_WS_SOLVE_FWD = 1, /* odevit_solve_fwd                                                 */
   ODEVIT_WS_SOLVE_BWD = 2, /* odevit_solve_bwd                                                 */
   ODEVIT_WS_ENCODER_FWD = 3, /* odevit_encoder_fwd (method ignored)                            */
-  ODEVIT_WS_SOLVE_ADAPTIVE = 4 /* odevit_solve_adaptive (method ignored)                        */
+  ODEVIT_WS_SOLVE_ADAPTIVE = 4, /* odevit_solve_adaptive[_record] (method ignored)              */
+  ODEVIT_WS_SOLVE_ADAPTIVE_BWD = 5 /* odevit_solve_adaptive_bwd (method ignored)                */
 } odevit_ws_kind;
 
 /* ABI / build identification. */
@@ -301,6 +305,45 @@ int odevit_solve_adaptive(const odevit_desc* desc, const odevit_weights* w, cons
                           int32_t max_num_steps, float* states /* [n_out,B,N,D] */, int32_t* nfe, int32_t* accepted,
                           int32_t* rejected /* [B] device, or NULL */, void* workspace, size_t workspace_bytes,
                           odevit_stream_t stream);
+
+/* odevit_solve_adaptive that also records every image's ACCEPTED steps, the schedule odevit_solve_adaptive_bwd
+ * differentiates.  step_t0, step_dt [step_cap, B] fp64 and step_out [step_cap, B] int32, device: entry [s, b] is image
+ * b's s-th accepted step (its start time, its dt, the first output index not yet written after it); entries past an
+ * image's count are zero, so row s of step_dt is the per-image dt of reverse step s.  Everything else, including the
+ * states and counts, is bitwise what odevit_solve_adaptive gives.  An image that accepts more than step_cap steps stops
+ * the solve with ODEVIT_ERR_WORKSPACE (the message names the image); the solve is deterministic, so a retry with a
+ * larger record gives the same result. */
+int odevit_solve_adaptive_record(const odevit_desc* desc, const odevit_weights* w, const float* x0,
+                                 const float* t_out_host, int32_t n_out, double rtol, double atol, double first_step,
+                                 int32_t max_num_steps, float* states, int32_t* nfe, int32_t* accepted,
+                                 int32_t* rejected, int32_t step_cap, double* step_t0, double* step_dt,
+                                 int32_t* step_out, void* workspace, size_t workspace_bytes, odevit_stream_t stream);
+
+/* Bytes of the tape of odevit_solve_adaptive_bwd for S = max accepted steps: 6 S + 1 field evaluations. */
+size_t odevit_adaptive_tape_bytes(const odevit_desc* desc, int32_t S);
+
+/* Reverse sweep through the adaptive solve with the recorded steps FROZEN (discretise-then-optimise): the exact
+ * derivative, with respect to x0 and the field's weights, of the computation that maps x0 to `states` along each
+ * image's accepted steps -- FSAL Dormand-Prince stages, stage combines in fp32 with dt cast, the quartic dense output at
+ * x = (t_out[j] - t0) / dt (fp64, cast).  The step times, dt, x and the choice of step per output are constants: rejected
+ * attempts, the error estimate, the step-size controller and the initial-step selection contribute nothing.  (Neither
+ * the continuous adjoint nor autograd through an unrolled torchdiffeq dopri5, whose graph also reaches y through the
+ * error ratio that sets the next dt.)
+ *   x0, t_out_host, n_out: as given to odevit_solve_adaptive_record;  step_t0, step_dt, step_out, step_cap: its record;
+ *   n_steps_host [B] HOST int32: accepted steps per image (0 <= n_b <= step_cap);  S = max n_b >= 1;
+ *   g_states [n_out,B,N,D]: cotangent of states;  g_x0 [B,N,D] out;  gw: weight-gradient accumulators (+=);
+ *   ckpt [S+1,B,N,D] fp32 caller scratch: the state at the start of every reverse step (a replay of the recorded steps
+ *        writes it; a finished image's rows repeat its last state);
+ *   tape (odevit_adaptive_tape_bytes(desc, S) bytes, 1024-aligned) or NULL: the replay keeps every evaluation's
+ *        intermediates there; with NULL the reverse sweep recomputes each step from its checkpoint.
+ * 6 S + 1 evaluations replay the steps, 6 S + 1 VJPs run the reverse sweep, plus 6 S recomputed evaluations without a
+ * tape.  desc must have no dropout.  Workspace kind ODEVIT_WS_SOLVE_ADAPTIVE_BWD.  Does not synchronise. */
+int odevit_solve_adaptive_bwd(const odevit_desc* desc, const odevit_weights* w, const float* x0,
+                              const float* t_out_host, int32_t n_out, const double* step_t0, const double* step_dt,
+                              const int32_t* step_out, int32_t step_cap, const int32_t* n_steps_host,
+                              const float* g_states, float* g_x0, const odevit_weight_grads* gw, float* ckpt,
+                              void* tape, size_t tape_bytes, void* workspace, size_t workspace_bytes,
+                              odevit_stream_t stream);
 
 /* 1 when odevit_solve_fwd runs this inference solve in the on-chip-state kernel (one persistent CTA per image,
  * trajectory rows written from shared memory): the caller then has no reason to prefer the trajectory-free form. */

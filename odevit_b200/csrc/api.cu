@@ -730,6 +730,7 @@ Epi rk_epilogue(const Tableau& tb, int st, float dt, const float* y, float* cons
   e.k_store = (!last && st < 3) ? k[st] : nullptr;
   return e;
 }
+}  // namespace
 
 // VJP of one field evaluation: given dd = scaler * lambda (cotangent of the pre-scaler output, in
 // the activation type) and the stage intermediates `c`, accumulate G1, c1, G2, c2 and deliver
@@ -883,7 +884,6 @@ int finish_grads(const Plan& p, const odevit_weights* w, const odevit_weight_gra
 
 bool wants_c2(const odevit_weight_grads* gw) { return gw && (gw->out_proj_b || gw->fc2_b); }
 
-}  // namespace
 }  // namespace odevit
 
 // ================================================================================================
@@ -1032,6 +1032,8 @@ size_t odevit_workspace_bytes(const odevit_desc* desc, int32_t ws_kind, int32_t 
     layout_encoder(p, a);
   } else if (ws_kind == ODEVIT_WS_SOLVE_ADAPTIVE) {
     a.off = solve_adaptive_workspace_bytes(p);
+  } else if (ws_kind == ODEVIT_WS_SOLVE_ADAPTIVE_BWD) {
+    a.off = solve_adaptive_bwd_workspace_bytes(p);
   } else {
     const Tableau* tb = tableau_for(method);
     if (!tb) { set_error(ODEVIT_ERR_INVALID_ARG, "unknown method %d", method); return 0; }

@@ -123,8 +123,21 @@ int solve_resident(const Plan& p, const WeightBufs& wb, int S, const float (*ta)
                    const float* t_host, int n_grid, float* states, float* final_state, float* p_last, float* kbuf,
                    cudaStream_t s);
 
-// Adaptive Dormand-Prince solve (solve_adaptive.cu): bytes of its workspace layout (ODEVIT_WS_SOLVE_ADAPTIVE)
+// Reverse-sweep pieces shared by odevit_solve_bwd and odevit_solve_adaptive_bwd (api.cu):
+//   layout_bwd: the fixed-grid workspace for S stages;  tape_ctx: slot e of a tape of n_evals evaluations (its byte count
+//   into *total_bytes when given);  eval_vjp: VJP of one field evaluation, mu delivered through `mu_epi` (the EPI_RK
+//   epilogue of its last GEMM);  finish_grads: the accumulators unfolded into the caller's gradients, once per call
+BwdBufs layout_bwd(const Plan& p, Arena& a, int S);
+StageCtx tape_ctx(const Plan& p, void* tape, long long e, size_t* total_bytes, long long n_evals);
+int eval_vjp(const Plan& p, const WeightBufs& wb, const StageCtx& c, BwdBufs& b, const float* g_p, bool need_c2,
+             const odevit_weight_grads* gw, long long ev, const Epi& mu_epi, cudaStream_t s);
+int finish_grads(const Plan& p, const odevit_weights* w, const odevit_weight_grads* gw, const BwdBufs& b, cudaStream_t s);
+bool wants_c2(const odevit_weight_grads* gw);
+
+// Adaptive Dormand-Prince solve (solve_adaptive.cu): bytes of its workspace layouts (ODEVIT_WS_SOLVE_ADAPTIVE,
+// ODEVIT_WS_SOLVE_ADAPTIVE_BWD)
 size_t solve_adaptive_workspace_bytes(const Plan& p);
+size_t solve_adaptive_bwd_workspace_bytes(const Plan& p);
 
 // MACARON field (field_macaron.cu)
 int macaron_forward(const Plan& p, const WeightBufs& wb, const StageCtx& c, const float* u, float* P,

@@ -1,4 +1,5 @@
-// Adaptive Dormand-Prince 5(4) inference solve with per-image step control (odevit_solve_adaptive).
+// Adaptive Dormand-Prince 5(4) solve with per-image step control (odevit_solve_adaptive[_record]) and its reverse
+// sweep over the accepted steps (odevit_solve_adaptive_bwd).
 //
 // Every image b runs torchdiffeq's dopri5 (_impl/dopri5.py, rk_common.py, interp.py, misc.py) on its own N*D
 // elements: its own t, dt, error norm, accept/reject decision and dense output.  A batch of one is the published
@@ -21,6 +22,11 @@
 // The host cannot know the number of rounds: after enqueuing round r + 1 it waits for round r's active-image count
 // (copied to pinned host memory right after round r, before round r + 1's launches), so the GPU always has the next
 // round queued while the host decides.
+//
+// odevit_solve_adaptive_record also records every image's accepted steps (ad_control_kernel); odevit_solve_adaptive_bwd
+// differentiates the solve along them, frozen: it replays the steps into checkpoints (optionally onto a tape), then runs
+// the reverse sweep step by step -- the dense output's VJP (ad_interp_vjp_kernel), the stage VJPs whose mu epilogues form
+// the next lambda with the per-image dt (EPI_RK | EPI_ROWDT), and one VJP at the step's start row (DESIGN.md 4.5).
 #include <cmath>
 #include <vector>
 
@@ -48,7 +54,7 @@ __constant__ float kCMid[7] = {(float)(6025192743. / 30085553152. / 2), 0.f, (fl
 
 constexpr int kMaxOut = 4096;        // output times a workspace holds (32 KB of fp64)
 constexpr int kRedThreads = 256;     // per-image reductions: one block per image
-constexpr int kErrMax = 0, kErrNonFinite = 1, kErrUnderflow = 2;
+constexpr int kErrMax = 0, kErrNonFinite = 1, kErrUnderflow = 2, kErrRecord = 3;
 constexpr int kNoError = 0x7fffffff;
 
 // sync words: [0], [1] active-image count of rounds with r & 1 == 0 / 1; [2] min(b * 4 + kind) over failed images
@@ -203,10 +209,12 @@ __global__ void __launch_bounds__(kRedThreads) ad_init_step_kernel(int phase, co
 
 // Per image: error ratio from the row partials (fixed order), accept / reject, the next t / dt / output index into the
 // other half of the double buffer, counters, limits.  One block per image.
+// rec_t0 != null: an accepted step is recorded at [n_acc[b], b] of rec_t0 / rec_dt / rec_out ([rec_cap, B]).
 __global__ void __launch_bounds__(kRedThreads) ad_control_kernel(
     const double* row0, int N, int D, int B, const double* t_cur, const double* dt_cur, const int* on_cur,
     double* t_nxt, double* dt_nxt, int* on_nxt, int* accept, int* attempts, int* n_acc, int* n_rej, const double* t_out,
-    int n_out, int max_steps, int nfe_base, int* nfe, int* acc_out, int* rej_out, int* active_slot, int* err) {
+    int n_out, int max_steps, int nfe_base, int* nfe, int* acc_out, int* rej_out, int* active_slot, int* err,
+    double* rec_t0, double* rec_dt, int* rec_out, int rec_cap) {
   __shared__ double red[kRedThreads];
   const int b = blockIdx.x;
   const double dt = dt_cur[b];
@@ -230,6 +238,16 @@ __global__ void __launch_bounds__(kRedThreads) ad_control_kernel(
     if (ok) {
       t1 = t0 + dt;
       while (on < n_out && t_out[on] <= t1) ++on;
+      if (rec_t0) {
+        const int i = n_acc[b];
+        if (i >= rec_cap) {
+          fail = kErrRecord;
+        } else {
+          rec_t0[(long long)i * B + b] = t0;
+          rec_dt[(long long)i * B + b] = dt;
+          rec_out[(long long)i * B + b] = on;
+        }
+      }
       n_acc[b] += 1;
     } else {
       n_rej[b] += 1;
@@ -237,7 +255,7 @@ __global__ void __launch_bounds__(kRedThreads) ad_control_kernel(
     // _optimal_step_size(dt, ratio, safety 0.9, ifactor 10, dfactor 0.2, order 5)
     if (ratio == 0.0) dt_new = dt * 10.0;
     else dt_new = dt * fmin(10.0, fmax(0.9 * pow(ratio, -1.0 / 5.0), ratio < 1.0 ? 1.0 : 0.2));
-    if (on < n_out) {
+    if (fail < 0 && on < n_out) {
       if (att >= max_steps) fail = kErrMax;
       else if (t1 + dt_new == t1) fail = kErrUnderflow;
     }
@@ -293,6 +311,59 @@ __global__ void __launch_bounds__(256) ad_commit_kernel(float* y0, const float* 
   }
 }
 
+// Cotangents the dense output of one reverse step hands to the stages.  Row r = ckpt[s] is y0 of step s and y1 of step
+// s - 1, and its evaluation f(ckpt[s]) is k1 of step s and k7 of step s - 1 (FSAL): one buffer each.
+struct InterpCot {
+  float* y;      // of row s: g_y0 of step s + g_y1 of step s - 1 (+ g_states[0] when s == 0)
+  float* k17;    // of f(row s): g_k1 of step s + g_k7 of step s - 1
+  float* k[4];   // g_k3 .. g_k6 of step s
+};
+
+// VJP of the quartic dense output of step s (interp._interp_fit / _interp_evaluate, as ad_commit_kernel forms it).  With
+// S_p = sum_j x_j^p g_j over the outputs j of the step (step_out of steps s - 1 and s bound them) and the coefficients
+// [e, d, c, b, a] of interp_fit:  g_a = S4, g_b = S3, g_c = S2, g_d = S1, g_e = S0, hence
+//   g_y0 = S0 - 11 S2 + 18 S3 - 8 S4,  g_y1 = -5 S2 + 14 S3 - 8 S4,  g_ymid = 16 S2 - 32 S3 + 16 S4,
+//   g_f0 = dt (S1 - 4 S2 + 5 S3 - 2 S4),  g_f1 = dt (S2 - 3 S3 + 2 S4),
+// and y_mid = y0 + dt sum_l c_mid[l] k_l spreads g_ymid onto y0 and onto k_l with dt c_mid[l].  Writes `cur` (step s's
+// own cotangents; zeros for an image without an output in the step) and adds g_y1, g_k7 into `nxt` (row s + 1).
+__global__ void __launch_bounds__(256) ad_interp_vjp_kernel(const float* __restrict__ g_states, const double* t_out,
+                                                            const double* step_t0, const double* step_dt,
+                                                            const int* step_out, int s, int B, InterpCot cur,
+                                                            InterpCot nxt, long long MD, long long per_image) {
+  const long long stride = (long long)gridDim.x * blockDim.x;
+  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < MD; i += stride) {
+    const int b = (int)(i / per_image);
+    const long long sb = (long long)s * B + b;
+    const int lo = s == 0 ? 1 : step_out[sb - B], hi = step_out[sb];
+    float S0 = 0.f, S1 = 0.f, S2 = 0.f, S3 = 0.f, S4 = 0.f;
+    if (lo < hi) {
+      const double t0 = step_t0[sb], dtd = step_dt[sb];
+      for (int j = lo; j < hi; ++j) {
+        const float x = (float)((t_out[j] - t0) / dtd);
+        const float g = g_states[(long long)j * MD + i];
+        const float x2 = x * x;
+        S0 += g;
+        S1 = fmaf(x, g, S1);
+        S2 = fmaf(x2, g, S2);
+        S3 = fmaf(x2 * x, g, S3);
+        S4 = fmaf(x2 * x2, g, S4);
+      }
+    }
+    const float dt = lo < hi ? (float)step_dt[sb] : 0.f;
+    const float gm = 16.f * S2 - 32.f * S3 + 16.f * S4;
+    const float dgm = dt * gm;
+    float gy0 = S0 - 11.f * S2 + 18.f * S3 - 8.f * S4 + gm;
+    if (s == 0) gy0 += g_states[i];
+    cur.y[i] = gy0;
+    cur.k17[i] = fmaf(kCMid[0], dgm, dt * (S1 - 4.f * S2 + 5.f * S3 - 2.f * S4));
+    for (int l = 0; l < 4; ++l) cur.k[l][i] = kCMid[l + 2] * dgm;
+    if (lo < hi) {
+      nxt.y[i] += -5.f * S2 + 14.f * S3 - 8.f * S4;
+      nxt.k17[i] += fmaf(kCMid[6], dgm, dt * (S2 - 3.f * S3 + 2.f * S4));
+    }
+  }
+}
+
 int grid_for(long long n) {
   const long long b = (n + 255) / 256;
   return (int)(b < 148 * 8 ? (b > 0 ? b : 1) : 148 * 8);
@@ -330,6 +401,49 @@ int* pinned_slots() {
   return p;
 }
 
+// the output times as fp64, checked: 2..kMaxOut finite, strictly increasing values
+int read_t_out(const float* t_out_host, int n_out, std::vector<double>& t_out) {
+  if (!t_out_host || n_out < 2 || n_out > kMaxOut)
+    return set_error(ODEVIT_ERR_INVALID_ARG, "t_out must hold 2..%d host values, got %d", kMaxOut, (int)n_out);
+  t_out.resize(n_out);
+  for (int i = 0; i < n_out; ++i) {
+    t_out[i] = (double)t_out_host[i];
+    if (!std::isfinite(t_out[i])) return set_error(ODEVIT_ERR_INVALID_ARG, "t_out[%d] is not finite", i);
+    if (i > 0 && !(t_out[i] > t_out[i - 1]))
+      return set_error(ODEVIT_ERR_INVALID_ARG, "t_out must be strictly increasing (t_out[%d]=%g, t_out[%d]=%g)", i - 1,
+                       t_out[i - 1], i, t_out[i]);
+  }
+  return 0;
+}
+
+// ---- reverse sweep (odevit_solve_adaptive_bwd) ---------------------------------------------------------------------
+struct AdBwdBufs {
+  BwdBufs b;          // the fixed-grid reverse-sweep buffers: folded weights, VJP scratch, G (b.gy), dd, accumulators
+  StageCtx ctx[6];    // without a tape: f(ckpt[s]) (ctx[0] = b.ctx[0], also every replay evaluation) and k2..k6 of step s
+  float* k[6];        // k1..k6 of the step being replayed or recomputed
+  float* mu[6];       // [1..5]: mu of the evaluations k2..k6 of the reverse step
+  InterpCot cot[2];   // dense-output cotangents of rows with s & 1 == 0 / 1
+  double* t_out;      // [kMaxOut]
+};
+
+AdBwdBufs layout_adaptive_bwd(const Plan& p, Arena& a) {
+  AdBwdBufs f;
+  const size_t MD = (size_t)p.M * p.D;
+  f.b = layout_bwd(p, a, 1);
+  f.ctx[0] = f.b.ctx[0];
+  for (int i = 1; i < 6; ++i) f.ctx[i] = take_ctx(p, a, true);
+  for (int i = 0; i < 6; ++i) f.k[i] = a.f32(MD);
+  f.mu[0] = nullptr;
+  for (int i = 1; i < 6; ++i) f.mu[i] = a.f32(MD);
+  for (InterpCot& c : f.cot) {
+    c.y = a.f32(MD);
+    c.k17 = a.f32(MD);
+    for (float*& k : c.k) k = a.f32(MD);
+  }
+  f.t_out = reinterpret_cast<double*>(a.take((size_t)kMaxOut * 8));
+  return f;
+}
+
 }  // namespace
 
 size_t solve_adaptive_workspace_bytes(const Plan& p) {
@@ -338,15 +452,29 @@ size_t solve_adaptive_workspace_bytes(const Plan& p) {
   return a.off;
 }
 
+size_t solve_adaptive_bwd_workspace_bytes(const Plan& p) {
+  Arena a(nullptr);
+  layout_adaptive_bwd(p, a);
+  return a.off;
+}
+
 }  // namespace odevit
 
 using namespace odevit;
 
-extern "C" int odevit_solve_adaptive(const odevit_desc* desc, const odevit_weights* w, const float* x0,
-                                     const float* t_out_host, int32_t n_out, double rtol, double atol,
-                                     double first_step, int32_t max_num_steps, float* states, int32_t* nfe,
-                                     int32_t* accepted, int32_t* rejected, void* workspace, size_t workspace_bytes,
-                                     odevit_stream_t stream) {
+namespace {
+// The accepted-step record of odevit_solve_adaptive_record ([cap, B] each; t0 == nullptr: no record).
+struct StepRecord {
+  double* t0 = nullptr;
+  double* dt = nullptr;
+  int32_t* out = nullptr;
+  int cap = 0;
+};
+
+int solve_adaptive_impl(const odevit_desc* desc, const odevit_weights* w, const float* x0, const float* t_out_host,
+                        int32_t n_out, double rtol, double atol, double first_step, int32_t max_num_steps,
+                        float* states, int32_t* nfe, int32_t* accepted, int32_t* rejected, const StepRecord& rec,
+                        void* workspace, size_t workspace_bytes, odevit_stream_t stream) {
   Plan p{};
   ODV_TRY(make_plan(desc, &p));
   ODV_TRY(check_weights(p, w));
@@ -356,16 +484,14 @@ extern "C" int odevit_solve_adaptive(const odevit_desc* desc, const odevit_weigh
   if (nfe) ODV_TRY(check_device_ptr(nfe, "nfe"));
   if (accepted) ODV_TRY(check_device_ptr(accepted, "accepted"));
   if (rejected) ODV_TRY(check_device_ptr(rejected, "rejected"));
-  if (!t_out_host || n_out < 2 || n_out > kMaxOut)
-    return set_error(ODEVIT_ERR_INVALID_ARG, "t_out must hold 2..%d host values, got %d", kMaxOut, (int)n_out);
-  std::vector<double> t_out(n_out);
-  for (int i = 0; i < n_out; ++i) {
-    t_out[i] = (double)t_out_host[i];
-    if (!std::isfinite(t_out[i])) return set_error(ODEVIT_ERR_INVALID_ARG, "t_out[%d] is not finite", i);
-    if (i > 0 && !(t_out[i] > t_out[i - 1]))
-      return set_error(ODEVIT_ERR_INVALID_ARG, "t_out must be strictly increasing (t_out[%d]=%g, t_out[%d]=%g)", i - 1,
-                       t_out[i - 1], i, t_out[i]);
+  if (rec.t0) {
+    if (rec.cap < 1) return set_error(ODEVIT_ERR_INVALID_ARG, "step_cap %d < 1", rec.cap);
+    ODV_TRY(check_device_ptr(rec.t0, "step_t0"));
+    ODV_TRY(check_device_ptr(rec.dt, "step_dt"));
+    ODV_TRY(check_device_ptr(rec.out, "step_out"));
   }
+  std::vector<double> t_out;
+  ODV_TRY(read_t_out(t_out_host, n_out, t_out));
   if (!(rtol >= 0.0 && atol >= 0.0 && rtol + atol > 0.0 && std::isfinite(rtol) && std::isfinite(atol)))
     return set_error(ODEVIT_ERR_INVALID_ARG, "rtol %g / atol %g: both >= 0, finite, not both 0", rtol, atol);
   if (!std::isfinite(first_step)) return set_error(ODEVIT_ERR_INVALID_ARG, "first_step is not finite");
@@ -390,6 +516,12 @@ extern "C" int odevit_solve_adaptive(const odevit_desc* desc, const odevit_weigh
   ODV_CUDA(cudaMemcpyAsync(f.t_out, t_out.data(), (size_t)n_out * 8, cudaMemcpyHostToDevice, s));
   ODV_CUDA(cudaMemcpyAsync(states, x0, (size_t)MD * 4, cudaMemcpyDeviceToDevice, s));
   ODV_CUDA(cudaMemcpyAsync(f.y0, x0, (size_t)MD * 4, cudaMemcpyDeviceToDevice, s));
+  if (rec.t0) {   // entries past an image's count stay zero: row s of step_dt is then the dt of reverse step s
+    const size_t n = (size_t)rec.cap * B;
+    ODV_CUDA(cudaMemsetAsync(rec.t0, 0, n * 8, s));
+    ODV_CUDA(cudaMemsetAsync(rec.dt, 0, n * 8, s));
+    ODV_CUDA(cudaMemsetAsync(rec.out, 0, n * 4, s));
+  }
   ad_init_kernel<<<(B + 255) / 256, 256, 0, s>>>(f.t, f.dt, f.out_next, f.accept, f.sync, f.t_out,
                                                   first_step > 0 ? first_step : 0.0, B);
   ODV_LAUNCH_CHECK();
@@ -436,7 +568,8 @@ extern "C" int odevit_solve_adaptive(const odevit_desc* desc, const odevit_weigh
     ad_control_kernel<<<B, kRedThreads, 0, s>>>(f.row0, N, D, B, f.t + (size_t)c * B, dt, f.out_next + (size_t)c * B,
                                                 f.t + (size_t)n * B, f.dt + (size_t)n * B, f.out_next + (size_t)n * B,
                                                 f.accept, f.attempts, f.n_acc, f.n_rej, f.t_out, n_out, max_num_steps,
-                                                nfe_base, nfe, accepted, rejected, f.sync + c, f.sync + 2);
+                                                nfe_base, nfe, accepted, rejected, f.sync + c, f.sync + 2, rec.t0,
+                                                rec.dt, rec.out, rec.cap);
     ODV_LAUNCH_CHECK();
     ad_commit_kernel<<<grid_for(MD), 256, 0, s>>>(f.y0, f.y1, f.k[0], f.k[2], f.k[3], f.k[4], f.k[5], f.k[6], f.accept,
                                                   f.t + (size_t)c * B, dt, f.out_next + (size_t)c * B,
@@ -460,6 +593,9 @@ extern "C" int odevit_solve_adaptive(const odevit_desc* desc, const odevit_weigh
         return set_error(ODEVIT_ERR_NOT_CONVERGED, "image %d: max_num_steps (%d) exceeded before t_out[-1]", b,
                          (int)max_num_steps);
       if (kind == kErrNonFinite) return set_error(ODEVIT_ERR_NOT_CONVERGED, "image %d: non-finite error ratio", b);
+      if (kind == kErrRecord)
+        return set_error(ODEVIT_ERR_WORKSPACE, "image %d: more than step_cap (%d) accepted steps: the step record is full",
+                         b, rec.cap);
       return set_error(ODEVIT_ERR_NOT_CONVERGED, "image %d: underflow in dt (t + dt == t)", b);
     }
     if (active == 0) {
@@ -474,4 +610,202 @@ extern "C" int odevit_solve_adaptive(const odevit_desc* desc, const odevit_weigh
     }
   }
   return 0;
+}
+}  // namespace
+
+extern "C" int odevit_solve_adaptive(const odevit_desc* desc, const odevit_weights* w, const float* x0,
+                                     const float* t_out_host, int32_t n_out, double rtol, double atol,
+                                     double first_step, int32_t max_num_steps, float* states, int32_t* nfe,
+                                     int32_t* accepted, int32_t* rejected, void* workspace, size_t workspace_bytes,
+                                     odevit_stream_t stream) {
+  return solve_adaptive_impl(desc, w, x0, t_out_host, n_out, rtol, atol, first_step, max_num_steps, states, nfe,
+                             accepted, rejected, StepRecord{}, workspace, workspace_bytes, stream);
+}
+
+extern "C" int odevit_solve_adaptive_record(const odevit_desc* desc, const odevit_weights* w, const float* x0,
+                                            const float* t_out_host, int32_t n_out, double rtol, double atol,
+                                            double first_step, int32_t max_num_steps, float* states, int32_t* nfe,
+                                            int32_t* accepted, int32_t* rejected, int32_t step_cap, double* step_t0,
+                                            double* step_dt, int32_t* step_out, void* workspace,
+                                            size_t workspace_bytes, odevit_stream_t stream) {
+  if (!step_t0 || !step_dt || !step_out) return set_error(ODEVIT_ERR_INVALID_ARG, "step_t0 / step_dt / step_out is NULL");
+  StepRecord rec;
+  rec.t0 = step_t0; rec.dt = step_dt; rec.out = step_out; rec.cap = step_cap;
+  return solve_adaptive_impl(desc, w, x0, t_out_host, n_out, rtol, atol, first_step, max_num_steps, states, nfe,
+                             accepted, rejected, rec, workspace, workspace_bytes, stream);
+}
+
+extern "C" size_t odevit_adaptive_tape_bytes(const odevit_desc* desc, int32_t S) {
+  Plan p{};
+  if (make_plan(desc, &p)) return 0;
+  if (S < 1) { set_error(ODEVIT_ERR_INVALID_ARG, "S %d < 1", (int)S); return 0; }
+  size_t need = 0;
+  tape_ctx(p, nullptr, 0, &need, 6LL * S + 1);
+  return need;
+}
+
+// Reverse sweep with the recorded steps frozen.  Evaluation e = 6 s + i of the replay is f(ckpt[s]) for i = 0 (k1 of step
+// s, k7 of step s - 1) and k_{i+1} of step s for i = 1..5.  With G the cotangent of ckpt[s + 1] (everything downstream of
+// it), reverse step s runs
+//   lambda_6 = g_k6 + dt_b c_sol[5] G                                   (a row pass: rk_apply_rows with EPI_ROWDT)
+//   VJP of k6 .. k2: mu_m, and in the mu GEMM's EPI_RK | EPI_ROWDT epilogue
+//     lambda_{m-1} = g_k{m-1} + dt_b (beta[m-1][m-1] mu_m + sum_{l>m} beta[l-1][m-1] mu_l + c_sol[m-1] G)
+//   VJP of f(ckpt[s]) with lambda_1 + g_k7 of step s - 1 (the same evaluation):  G <- G + sum mu + g of row s
+// where the g_* are the dense output's cotangents (ad_interp_vjp_kernel).  Reverse step S is that last VJP alone, at each
+// image's end state.  A finished image has dt_b = 0 and no outputs in its remaining steps: lambda = 0 there.
+extern "C" int odevit_solve_adaptive_bwd(const odevit_desc* desc, const odevit_weights* w, const float* x0,
+                                         const float* t_out_host, int32_t n_out, const double* step_t0,
+                                         const double* step_dt, const int32_t* step_out, int32_t step_cap,
+                                         const int32_t* n_steps_host, const float* g_states, float* g_x0,
+                                         const odevit_weight_grads* gw, float* ckpt, void* tape, size_t tape_bytes,
+                                         void* workspace, size_t workspace_bytes, odevit_stream_t stream) {
+  Plan p{};
+  ODV_TRY(make_plan(desc, &p));
+  ODV_TRY(check_weights(p, w));
+  if (p.any_drop) return set_error(ODEVIT_ERR_INVALID_ARG, "the adaptive solve has no dropout: dropout must be 0");
+  if (!gw) return set_error(ODEVIT_ERR_INVALID_ARG, "weight-gradient struct is NULL");
+  ODV_TRY(check_device_ptr(x0, "x0"));
+  ODV_TRY(check_device_ptr(g_states, "g_states"));
+  ODV_TRY(check_device_ptr(g_x0, "g_x0"));
+  ODV_TRY(check_device_ptr(ckpt, "ckpt"));
+  ODV_TRY(check_device_ptr(step_t0, "step_t0"));
+  ODV_TRY(check_device_ptr(step_dt, "step_dt"));
+  ODV_TRY(check_device_ptr(step_out, "step_out"));
+  std::vector<double> t_out;
+  ODV_TRY(read_t_out(t_out_host, n_out, t_out));
+  if (step_cap < 1) return set_error(ODEVIT_ERR_INVALID_ARG, "step_cap %d < 1", (int)step_cap);
+  if (!n_steps_host) return set_error(ODEVIT_ERR_INVALID_ARG, "n_steps_host is NULL");
+  int S = 0;
+  for (int b = 0; b < p.B; ++b) {
+    const int n = n_steps_host[b];
+    if (n < 0 || n > step_cap)
+      return set_error(ODEVIT_ERR_INVALID_ARG, "n_steps[%d] = %d outside [0, step_cap = %d]", b, n, (int)step_cap);
+    S = n > S ? n : S;
+  }
+  if (S < 1) return set_error(ODEVIT_ERR_INVALID_ARG, "no image has an accepted step");
+  if (tape) {
+    size_t need = 0;
+    tape_ctx(p, nullptr, 0, &need, 6LL * S + 1);
+    ODV_TRY(check_device_ptr(tape, "tape"));
+    ODV_TRY(check_ws(tape, tape_bytes, need));
+  }
+  Arena a(workspace);
+  AdBwdBufs f = layout_adaptive_bwd(p, a);
+  ODV_TRY(check_ws(workspace, workspace_bytes, a.off));
+  cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
+  BwdBufs& b = f.b;
+  const int B = p.B, N = p.N;
+  const long long MD = (long long)p.M * p.D;
+  const bool need_c2 = wants_c2(gw);
+  float* G = b.gy;
+  ODV_TRY(prepare_weights(p, w, b.w, s));
+  ODV_CUDA(cudaMemcpyAsync(f.t_out, t_out.data(), (size_t)n_out * 8, cudaMemcpyHostToDevice, s));
+  ODV_CUDA(cudaMemsetAsync(b.G1, 0, b.acc_bytes, s));
+  ODV_CUDA(cudaMemcpyAsync(ckpt, x0, (size_t)MD * 4, cudaMemcpyDeviceToDevice, s));
+
+  auto row = [&](int r) { return ckpt + (size_t)r * MD; };
+  auto dt_of = [&](int st) { return step_dt + (size_t)st * B; };
+  // context of evaluation 6 st + i: its tape slot, else the recompute buffer (the replay's own evaluations all go to
+  // ctx[0], which leaves f(ckpt[S]) there for reverse step S)
+  auto ctx_of = [&](int st, int i) -> StageCtx {
+    return tape ? tape_ctx(p, tape, 6LL * st + i, nullptr, 0) : f.ctx[i];
+  };
+  auto eval_k1 = [&](int r, const StageCtx& c) -> int {   // k1 = f(ckpt[r])
+    Epi e;
+    e.out = f.k[0]; e.c_new = 1.f;
+    return eval_forward(p, b.w, c, row(r), b.P, nullptr, b.sq, nullptr, 0, &e, s);
+  };
+  // the stages k2..k6 of step st from ckpt[st] and k1 (as a round of the forward forms them).  replay: the k6
+  // evaluation's epilogue writes ckpt[st + 1]; recompute: only the contexts are needed, k6's output GEMM is skipped
+  auto stages = [&](int st, bool replay) -> int {
+    const double* dt = dt_of(st);
+    const float* y0 = row(st);
+    ODV_TRY(row_axpy(p, y0, f.k[0], (float)kBeta[0][0], dt, b.u, s));   // u2
+    for (int m = 1; m <= 5; ++m) {
+      const StageCtx c = tape ? ctx_of(st, m) : f.ctx[replay ? 0 : m];
+      if (!replay && m == 5) return eval_forward(p, b.w, c, b.u, b.P, nullptr, b.sq, nullptr, 0, nullptr, s);
+      Epi e;
+      e.y = y0; e.y_coef = 1.f;
+      e.row_dt = dt; e.rows_per_image = N;
+      e.k_store = f.k[m];
+      e.c_new = (float)kBeta[m][m];
+      for (int l = 0, slot = 0; l < m; ++l)
+        if (kBeta[m][l] != 0.0) { e.kin[slot] = f.k[l]; e.c_k[slot] = (float)kBeta[m][l]; ++slot; }
+      e.out = (m == 5) ? row(st + 1) : b.u;
+      ODV_TRY(eval_forward(p, b.w, c, b.u, b.P, nullptr, b.sq, nullptr, 0, &e, s));
+    }
+    return 0;
+  };
+
+  // ---- replay: ckpt[1..S] (and the tape) ----
+  ODV_TRY(eval_k1(0, tape ? ctx_of(0, 0) : f.ctx[0]));
+  for (int st = 0; st < S; ++st) {
+    ODV_TRY(stages(st, true));
+    ODV_TRY(eval_k1(st + 1, tape ? ctx_of(st + 1, 0) : f.ctx[0]));
+  }
+
+  // ---- reverse ----
+  auto interp_vjp = [&](int st) -> int {   // step st's own cotangents into cot[st & 1], g_y1 / g_k7 added to row st + 1's
+    ad_interp_vjp_kernel<<<grid_for(MD), 256, 0, s>>>(g_states, f.t_out, step_t0, step_dt, step_out, st, B,
+                                                      f.cot[st & 1], f.cot[(st + 1) & 1], MD, (long long)N * p.D);
+    ODV_LAUNCH_CHECK();
+    return 0;
+  };
+  auto seed = [&](const float* gk, float c, const double* dt) -> int {   // dd = scaler * (gk + dt_b c G)
+    Epi e;
+    e.y = gk; e.y_coef = 1.f; e.c_new = c;
+    e.row_dt = dt; e.rows_per_image = N;
+    e.out2 = b.dd; e.out2_scale = p.scaler; e.aux_type = p.dd_type;
+    return rk_apply_rows(e, G, p.M, p.D, s);
+  };
+  auto stage_vjps = [&](int st) -> int {   // k6 .. k2 of step st; dd holds scaler * lambda_6
+    const InterpCot& cot = f.cot[st & 1];
+    for (int m = 5; m >= 1; --m) {
+      const int t = m - 1;   // the epilogue forms lambda of k[t]
+      Epi e;
+      e.aux_type = p.dd_type;
+      e.row_dt = dt_of(st); e.rows_per_image = N;
+      e.k_store = f.mu[m];
+      e.c_new = (float)kBeta[m - 1][t];
+      int n = 0;
+      for (int q = m + 1; q <= 5; ++q)
+        if (kBeta[q - 1][t] != 0.0) { e.kin[n] = f.mu[q]; e.c_k[n] = (float)kBeta[q - 1][t]; ++n; }
+      if (kBeta[5][t] != 0.0) { e.kin[n] = G; e.c_k[n] = (float)kBeta[5][t]; ++n; }
+      // the dense output's cotangent of k[t] enters unscaled; k2 has no dense-output weight (c_mid[1] = 0)
+      e.y = t == 0 ? cot.k17 : t == 1 ? G : cot.k[t - 2];
+      e.y_coef = t == 1 ? 0.f : 1.f;
+      e.out2 = b.dd; e.out2_scale = p.scaler;
+      ODV_TRY(eval_vjp(p, b.w, ctx_of(st, m), b, nullptr, need_c2, gw, 6LL * st + m, e, s));
+    }
+    return 0;
+  };
+  auto final_vjp = [&](int st) -> int {   // f(ckpt[st]): G <- G + its mu + the stage mus of step st + g of row st
+    Epi e;
+    e.aux_type = p.dd_type;
+    e.y = G; e.y_coef = 1.f; e.c_new = 1.f;
+    int n = 0;
+    if (st < S)
+      for (int m = 1; m <= 5; ++m) { e.kin[n] = f.mu[m]; e.c_k[n] = 1.f; ++n; }
+    e.kin[n] = f.cot[st & 1].y; e.c_k[n] = 1.f;
+    e.out = st == 0 ? g_x0 : G;
+    return eval_vjp(p, b.w, ctx_of(st, 0), b, nullptr, need_c2, gw, 6LL * st, e, s);
+  };
+
+  ODV_CUDA(cudaMemsetAsync(G, 0, (size_t)MD * 4, s));
+  ODV_CUDA(cudaMemsetAsync(f.cot[S & 1].y, 0, (size_t)MD * 4, s));
+  ODV_CUDA(cudaMemsetAsync(f.cot[S & 1].k17, 0, (size_t)MD * 4, s));
+  ODV_TRY(interp_vjp(S - 1));
+  ODV_TRY(seed(f.cot[S & 1].k17, 0.f, dt_of(S - 1)));   // G = 0: dd = scaler * g_k7 of step S - 1
+  ODV_TRY(final_vjp(S));
+  for (int st = S - 1; st >= 0; --st) {
+    ODV_TRY(seed(f.cot[st & 1].k[3], (float)kBeta[5][5], dt_of(st)));   // lambda_6
+    if (!tape) {
+      ODV_TRY(eval_k1(st, f.ctx[0]));
+      ODV_TRY(stages(st, false));
+    }
+    if (st > 0) ODV_TRY(interp_vjp(st - 1));
+    ODV_TRY(stage_vjps(st));
+    ODV_TRY(final_vjp(st));
+  }
+  return finish_grads(p, w, gw, b, s);
 }

@@ -178,8 +178,9 @@ class ViTMacaron(nn.Module):
         self.time_interval = time_interval
         self.num_eval_steps = num_eval_steps
         self.t_grid = torch.linspace(0.0, time_interval, num_eval_steps)
-        # None, or {"rtol", "atol"[, "first_step", "max_num_steps"]}: forward integrates over t_grid with the per-image
-        # adaptive Dormand-Prince solve (inference only; a plain attribute like `precision`, not a config key)
+        # None, or {"rtol", "atol"[, "first_step", "max_num_steps", "differentiable"]}: forward integrates over t_grid
+        # with the per-image adaptive Dormand-Prince solve (inference only unless "differentiable" is True; a plain
+        # attribute like `precision`, not a config key)
         self.adaptive_solve = None
         self._init_weights()
 
@@ -259,7 +260,8 @@ class ViTMacaron(nn.Module):
         if self.adaptive_solve is not None:
             res = ops.ode_solve_adaptive(tokens, t, block.field_spec(self.odefunc.scaler), block.field_weights(),
                                          cfg["rtol"], cfg["atol"], first_step=cfg.get("first_step"),
-                                         max_num_steps=cfg.get("max_num_steps", ops.DOPRI5_MAX_NUM_STEPS))
+                                         max_num_steps=cfg.get("max_num_steps", ops.DOPRI5_MAX_NUM_STEPS),
+                                         differentiable=cfg.get("differentiable", False))
             if idx is not None:
                 res["rows"] = res["states"][idx]
         else:

@@ -6,7 +6,8 @@ Replaces, for CUDA tensors:
   * `ViT_ODEFunc.forward(t, x)`                         models/ode_transformer_gpt.py:317-330
   * `torchdiffeq.odeint(func, y0, t, method=...)`        models/ode_transformer_gpt.py:571-578
   * `torchdiffeq.odeint(..., method="dopri5")` with the error norm taken per image (ode_solve_adaptive)
-  * autograd through both (backprop-through-solver)      train.py:57-67
+  * autograd through all three (backprop-through-solver)  train.py:57-67; the adaptive solve's with its accepted
+    steps frozen
 """
 from __future__ import annotations
 
@@ -151,8 +152,13 @@ def _alloc_tape(desc: _lib.Desc, method: int, n_grid: int, mode: str, device: to
     tensors are in the reference), or None -> the reverse sweep recomputes each step."""
     if mode == "recompute" or n_grid < 2:
         return None
-    n = int(_lib.lib().odevit_tape_bytes(ctypes.byref(desc), method, n_grid))
-    if n == 0:
+    return _tape_buffer(int(_lib.lib().odevit_tape_bytes(ctypes.byref(desc), method, n_grid)), mode, device)
+
+
+def _tape_buffer(n: int, mode: str, device: torch.device):
+    """A tape of n bytes under the backward mode `mode` ("tape" | "recompute" | "auto": when it fits
+    TAPE_BUDGET_FRACTION of the free memory), or None."""
+    if mode == "recompute" or n == 0:
         return None
     if mode == "auto":
         key = (device.index, n)
@@ -521,44 +527,137 @@ class NotConvergedError(OdevitError):
 DOPRI5_MAX_NUM_STEPS = 2 ** 31 - 1   # torchdiffeq's default
 
 
+ADAPTIVE_STEP_CAP = 1024   # first size of the accepted-step record of a differentiable adaptive solve (grown 4x on demand)
+
+
+def _adaptive_call(x0, t_c, T: int, spec: FieldSpec, names, weights, rtol: float, atol: float, fs: float,
+                   max_num_steps: int, record=None):
+    """One odevit_solve_adaptive call, or odevit_solve_adaptive_record with record = (cap, t0, dt, out).
+    Returns (status, states [T,B,N,D], counts [3,B] int32 = nfe, accepted, rejected)."""
+    B, N, D = x0.shape
+    desc = spec.desc(B, N)
+    w, keep = _pack_weights(names, weights)
+    states = torch.empty(T, B, N, D, device=x0.device, dtype=torch.float32)
+    counts = torch.zeros(3, B, device=x0.device, dtype=torch.int32)
+    buf, ws, ws_bytes = _workspace(desc, _lib.WS_SOLVE_ADAPTIVE, 0, x0.device)
+    with torch.cuda.device(x0.device):
+        if record is None:
+            st = _lib.lib().odevit_solve_adaptive(ctypes.byref(desc), ctypes.byref(w), _ptr(x0), t_c, T, float(rtol),
+                                                  float(atol), fs, int(max_num_steps), _ptr(states), _ptr(counts[0]),
+                                                  _ptr(counts[1]), _ptr(counts[2]), ws, ws_bytes, _stream())
+        else:
+            cap, t0, dt, out = record
+            st = _lib.lib().odevit_solve_adaptive_record(ctypes.byref(desc), ctypes.byref(w), _ptr(x0), t_c, T,
+                                                         float(rtol), float(atol), fs, int(max_num_steps), _ptr(states),
+                                                         _ptr(counts[0]), _ptr(counts[1]), _ptr(counts[2]), int(cap),
+                                                         _vp(t0.data_ptr()), _vp(dt.data_ptr()), _vp(out.data_ptr()),
+                                                         ws, ws_bytes, _stream())
+    return st, states, counts
+
+
+def _adaptive_check(st: int, what: str) -> None:
+    if st == _lib.ERR_NOT_CONVERGED:
+        raise NotConvergedError(_lib.lib().odevit_last_error_string().decode("utf-8", "replace"))
+    _lib.check(st, what)
+
+
+class _AdaptiveSolve(torch.autograd.Function):
+    """(states, counts) = the adaptive solve of x0; its backward is odevit_solve_adaptive_bwd over the accepted steps
+    the forward recorded (frozen: the step sizes, the output times' positions in them and the rejected attempts carry
+    no gradient)."""
+
+    @staticmethod
+    def forward(ctx, x0, spec: FieldSpec, t_c, T: int, rtol: float, atol: float, fs: float, max_num_steps: int,
+                names: Tuple[str, ...], *weights):
+        B = x0.shape[0]
+        cap = max(1, min(int(max_num_steps), int(ADAPTIVE_STEP_CAP)))
+        while True:
+            rec = (cap, torch.empty(cap, B, device=x0.device, dtype=torch.float64),
+                   torch.empty(cap, B, device=x0.device, dtype=torch.float64),
+                   torch.empty(cap, B, device=x0.device, dtype=torch.int32))
+            st, states, counts = _adaptive_call(x0, t_c, T, spec, names, weights, rtol, atol, fs, max_num_steps, rec)
+            # a full record: the solve is deterministic, so a larger one gives the same result
+            if st == _lib.ERR_WORKSPACE and cap < max_num_steps and b"step record" in _lib.lib().odevit_last_error_string():
+                cap = min(4 * cap, int(max_num_steps))
+                continue
+            break
+        _adaptive_check(st, "odevit_solve_adaptive_record")
+        ctx.spec, ctx.names, ctx.t_c, ctx.T, ctx.cap = spec, names, t_c, T, cap
+        ctx.n_steps = counts[1].cpu().tolist()   # (the solve has synchronised already)
+        ctx.save_for_backward(x0, rec[1], rec[2], rec[3], *weights)
+        ctx.mark_non_differentiable(counts)
+        ctx.set_materialize_grads(False)
+        return states, counts
+
+    @staticmethod
+    def backward(ctx, g_states, _g_counts):
+        x0, step_t0, step_dt, step_out, *weights = ctx.saved_tensors
+        spec, names = ctx.spec, ctx.names
+        B, N, D = x0.shape
+        if g_states is None:
+            return (None,) * (9 + len(weights))
+        gw, gts = _alloc_grads(names, weights, ctx.needs_input_grad[9:])
+        g_states = _require_cuda(g_states, "g_states")
+        desc = spec.desc(B, N)
+        w, keep = _pack_weights(names, weights)
+        S = max(ctx.n_steps)
+        ckpt = torch.empty(S + 1, B, N, D, device=x0.device, dtype=torch.float32)
+        tape = _tape_buffer(int(_lib.lib().odevit_adaptive_tape_bytes(ctypes.byref(desc), S)), spec.backward, x0.device)
+        tape_p, tape_n = _aligned(tape)
+        g_x0 = torch.empty_like(x0)
+        n_c = (ctypes.c_int32 * B)(*ctx.n_steps)
+        buf, ws, ws_bytes = _workspace(desc, _lib.WS_SOLVE_ADAPTIVE_BWD, 0, x0.device)
+        with torch.cuda.device(x0.device):
+            st = _lib.lib().odevit_solve_adaptive_bwd(ctypes.byref(desc), ctypes.byref(w), _ptr(x0), ctx.t_c, ctx.T,
+                                                      _vp(step_t0.data_ptr()), _vp(step_dt.data_ptr()),
+                                                      _vp(step_out.data_ptr()), ctx.cap, n_c, _ptr(g_states),
+                                                      _ptr(g_x0), ctypes.byref(gw), _ptr(ckpt), tape_p, tape_n, ws,
+                                                      ws_bytes, _stream())
+        _lib.check(st, "odevit_solve_adaptive_bwd")
+        return (g_x0 if ctx.needs_input_grad[0] else None,) + (None,) * 8 + tuple(gts)
+
+
 def ode_solve_adaptive(x0: torch.Tensor, t: torch.Tensor, spec: FieldSpec, weights: Dict[str, Optional[torch.Tensor]],
                        rtol: float, atol: float, first_step: Optional[float] = None,
-                       max_num_steps: int = DOPRI5_MAX_NUM_STEPS):
-    """Adaptive Dormand-Prince 5(4) solve with per-image step control (odevit_solve_adaptive), inference only.
+                       max_num_steps: int = DOPRI5_MAX_NUM_STEPS, differentiable: bool = False):
+    """Adaptive Dormand-Prince 5(4) solve with per-image step control (odevit_solve_adaptive).
 
     torchdiffeq's dopri5 run on every image on its own: the error norm, the accept / reject decisions, the step sizes
     and the dense output of image b depend on image b alone (torchdiffeq takes one norm over the whole batch).  `t`
     must be strictly increasing; `max_num_steps` bounds the attempted steps per image over the whole solve (torchdiffeq
     counts them per output interval).  Synchronises with the device once per round (one attempted step of every image).
 
+    differentiable=False: inference only, a gradient request raises.  differentiable=True: when grad mode is on and x0
+    or a weight requires grad, `states` is differentiable with respect to them, with each image's accepted steps frozen
+    (discretise-then-optimise: odevit_solve_adaptive_record / odevit_solve_adaptive_bwd).  Gradients with respect to
+    `t` are not built.
+
     Returns dict(states [len(t),B,N,D] (row i = solution at t[i]), final [B,N,D], nfe [B], accepted [B], rejected [B]
     (int32, device), rounds (int: rounds with at least one image still stepping = max_b accepted + rejected))."""
     names = tuple(k for k, v in weights.items() if v is not None)
-    if torch.is_grad_enabled() and (x0.requires_grad or any(weights[k].requires_grad for k in names)):
+    track = torch.is_grad_enabled() and (x0.requires_grad or any(weights[k].requires_grad for k in names))
+    if track and not differentiable:
         raise OdevitError("the adaptive solve is inference-only (no backward is built): run it under torch.no_grad() "
                           "or detach x0 and the weights")
     if spec.has_dropout:
+        if differentiable:
+            raise OdevitError("the adaptive solve has no dropout: the field's dropout must be 0")
         raise OdevitError("the adaptive solve is inference-only: the field's dropout must be 0 (call .eval())")
-    x0 = _require_cuda(x0.detach(), "x0")
-    B, N, D = x0.shape
     t_host = t.detach().to("cpu", torch.float32).contiguous()
     T = int(t_host.numel())
     t_c = (ctypes.c_float * max(1, T))(*t_host.tolist())
-    desc = spec.desc(B, N)
-    w, keep = _pack_weights(names, [weights[k].detach() for k in names])
-    states = torch.empty(T, B, N, D, device=x0.device, dtype=torch.float32)
-    counts = torch.zeros(3, B, device=x0.device, dtype=torch.int32)
-    buf, ws, ws_bytes = _workspace(desc, _lib.WS_SOLVE_ADAPTIVE, 0, x0.device)
     fs = 0.0 if first_step is None else float(first_step)
     if first_step is not None and not fs > 0:
         raise ValueError(f"first_step must be > 0, got {first_step}")
-    with torch.cuda.device(x0.device):
-        st = _lib.lib().odevit_solve_adaptive(ctypes.byref(desc), ctypes.byref(w), _ptr(x0), t_c, T, float(rtol),
-                                              float(atol), fs, int(max_num_steps), _ptr(states), _ptr(counts[0]),
-                                              _ptr(counts[1]), _ptr(counts[2]), ws, ws_bytes, _stream())
-    if st == _lib.ERR_NOT_CONVERGED:
-        raise NotConvergedError(_lib.lib().odevit_last_error_string().decode("utf-8", "replace"))
-    _lib.check(st, "odevit_solve_adaptive")
+    if track:
+        x0 = _require_cuda(x0, "x0")
+        states, counts = _AdaptiveSolve.apply(x0, spec, t_c, T, float(rtol), float(atol), fs, int(max_num_steps),
+                                              names, *[weights[k] for k in names])
+    else:
+        x0 = _require_cuda(x0.detach(), "x0")
+        st, states, counts = _adaptive_call(x0, t_c, T, spec, names, [weights[k].detach() for k in names], rtol, atol,
+                                            fs, max_num_steps)
+        _adaptive_check(st, "odevit_solve_adaptive")
     rounds = int((counts[1] + counts[2]).max().item())
     return {"states": states, "final": states[-1], "nfe": counts[0], "accepted": counts[1], "rejected": counts[2],
             "rounds": rounds}

@@ -235,12 +235,14 @@ def _check_field_module(func, who: str) -> None:
 
 
 def odeint_adaptive(func, y0: torch.Tensor, t: torch.Tensor, *, rtol: float = 1e-7, atol: float = 1e-9,
-                    options: Optional[dict] = None, return_stats: bool = False):
+                    options: Optional[dict] = None, return_stats: bool = False, differentiable: bool = False):
     """`torchdiffeq.odeint(func, y0, t, method="dopri5", rtol, atol, options)` for the fused vector field, with the
     step size controlled PER IMAGE (ops.ode_solve_adaptive): image b's error norm, steps and dense output depend on
-    image b alone, where torchdiffeq takes one norm over the batch.  Inference only; `t` strictly increasing;
-    options: `first_step`, `max_num_steps` (attempted steps per image over the whole solve, not per output interval).
-    Exports no attention maps.  Returns the trajectory [len(t), *y0.shape], or (trajectory, stats) with stats =
+    image b alone, where torchdiffeq takes one norm over the batch.  `t` strictly increasing; options: `first_step`,
+    `max_num_steps` (attempted steps per image over the whole solve, not per output interval).  Exports no attention
+    maps.  Inference only unless `differentiable`: then the trajectory is differentiable with respect to y0 and the
+    field's weights, with each image's accepted steps frozen (not the continuous adjoint, and not autograd through an
+    unrolled torchdiffeq solve).  Returns the trajectory [len(t), *y0.shape], or (trajectory, stats) with stats =
     dict(nfe, accepted, rejected: int32 [B] device tensors, rounds: int) when `return_stats`."""
     _check_field_module(func, "odeint_adaptive")
     options = dict(options or {})
@@ -249,23 +251,26 @@ def odeint_adaptive(func, y0: torch.Tensor, t: torch.Tensor, *, rtol: float = 1e
         raise ValueError(f"unsupported dopri5 options {sorted(unknown)}; first_step and max_num_steps are built")
     res = ops.ode_solve_adaptive(y0, t, func.block.field_spec(func.scaler), func.block.field_weights(), rtol, atol,
                                  first_step=options.get("first_step"),
-                                 max_num_steps=options.get("max_num_steps", ops.DOPRI5_MAX_NUM_STEPS))
+                                 max_num_steps=options.get("max_num_steps", ops.DOPRI5_MAX_NUM_STEPS),
+                                 differentiable=differentiable)
     if return_stats:
         return res["states"], {k: res[k] for k in ("nfe", "accepted", "rejected", "rounds")}
     return res["states"]
 
 
 def adaptive_solve_args(model: nn.Module, output_flags: Dict[str, bool]) -> dict:
-    """Checks a model's `adaptive_solve` request (a dict with rtol, atol and optionally first_step, max_num_steps) and
-    the forward's arguments against what the adaptive solve can give."""
+    """Checks a model's `adaptive_solve` request (a dict with rtol, atol and optionally first_step, max_num_steps,
+    differentiable) and the forward's arguments against what the adaptive solve can give."""
     cfg = dict(model.adaptive_solve)
-    unknown = set(cfg) - {"rtol", "atol", "first_step", "max_num_steps"}
+    unknown = set(cfg) - {"rtol", "atol", "first_step", "max_num_steps", "differentiable"}
     if unknown or "rtol" not in cfg or "atol" not in cfg:
-        raise ValueError(f"adaptive_solve takes rtol, atol [, first_step, max_num_steps], got {sorted(model.adaptive_solve)}")
+        raise ValueError(f"adaptive_solve takes rtol, atol [, first_step, max_num_steps, differentiable], "
+                         f"got {sorted(model.adaptive_solve)}")
     for name, on in output_flags.items():
         if on:
             raise ValueError(f"{name} is not available with adaptive_solve (the adaptive solve exports no attention maps)")
-    if torch.is_grad_enabled() and any(p.requires_grad for p in model.parameters()):
+    if (not cfg.get("differentiable", False) and torch.is_grad_enabled()
+            and any(p.requires_grad for p in model.parameters())):
         raise RuntimeError("adaptive_solve is inference-only (no backward is built): run the model under torch.no_grad()")
     return cfg
 
@@ -363,8 +368,9 @@ class ViTNeuralODE(nn.Module):
         self.time_interval = time_interval
         self.num_eval_steps = num_eval_steps
         self.t_grid = torch.linspace(0.0, time_interval, num_eval_steps)  # plain attribute, not a buffer
-        # None, or {"rtol", "atol"[, "first_step", "max_num_steps"]}: forward integrates over t_grid with the per-image
-        # adaptive Dormand-Prince solve (inference only; a plain attribute like `precision`, not a config key)
+        # None, or {"rtol", "atol"[, "first_step", "max_num_steps", "differentiable"]}: forward integrates over t_grid
+        # with the per-image adaptive Dormand-Prince solve (inference only unless "differentiable" is True; a plain
+        # attribute like `precision`, not a config key)
         self.adaptive_solve = None
         self.patch_embed.precision = self.odefunc.block.precision
         self.apply(self._spectral_init)
@@ -592,14 +598,15 @@ class ViTNeuralODE(nn.Module):
         res = ops.ode_solve_adaptive(tokens, t, self.odefunc.block.field_spec(self.odefunc.scaler),
                                      self.odefunc.block.field_weights(), cfg["rtol"], cfg["atol"],
                                      first_step=cfg.get("first_step"),
-                                     max_num_steps=cfg.get("max_num_steps", ops.DOPRI5_MAX_NUM_STEPS))
+                                     max_num_steps=cfg.get("max_num_steps", ops.DOPRI5_MAX_NUM_STEPS),
+                                     differentiable=cfg.get("differentiable", False))
         states, final = res["states"], res["final"]
         logits = self.head(final[:, 0])
         out = {
             "logits": logits,
             "second_derivative_upper_bound": self.compute_upper_bound_by_second_derivative(R=jasmin_k, L=1 / 2),
             "finite_difference_upper_bound": self.compute_upper_bound_by_fininte_difference(
-                states, 0.5, 1 / self.num_eval_steps),
+                states.detach(), 0.5, 1 / self.num_eval_steps),
             "nfe": res["nfe"],
         }
         if self.add_distillation_token:
