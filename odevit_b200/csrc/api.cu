@@ -194,7 +194,7 @@ void split_scratch(const Plan& p, Arena& a) {
   if (p.precision != ODEVIT_FP32 || off) return;
   const size_t R = 3 * (size_t)p.D + p.hid, K2 = (size_t)p.D + p.hid;
   const size_t mk2 = (size_t)p.M * K2, rd = R * (size_t)p.D;
-  p.split_a_bytes = 3 * (size_t)p.M * R * 2;   // >= 6 M (D + hid): the forward GEMMs take six segments
+  p.split_a_bytes = 3 * (size_t)p.M * R * 2;   // three segments of the mu GEMM's K = 3D + hid
   p.split_b_bytes = 3 * (mk2 > 2 * rd ? mk2 : 2 * rd) * 2;
   p.split_a = a.take(p.split_a_bytes);
   p.split_b = a.take(p.split_b_bytes);
@@ -410,15 +410,9 @@ static int gemm_split3(const Plan& p, const GemmArgs& g, cudaStream_t s, bool* t
   // products kept: (hi,hi) (hi,mid) (mid,hi).  Six products (adding (hi,lo) (mid,mid) (lo,hi): 2^-26 per term) were
   // measured and are NOT more accurate here: the tensor core's fp32 accumulation is not round-to-nearest, its error
   // grows with the length of the contraction, and the doubled axis cost more than the extra terms bought (exported
-  // attention map of the 224 px RK4 case: 1.6e-4 with three segments, 2.2e-4 with six).  ODEVIT_FP32_SEGMENTS=6 keeps
-  // the variant reachable for experiments.
-  static const int a3[3] = {0, 0, 1}, b3[3] = {0, 1, 0};
-  static const int a6[6] = {0, 0, 1, 0, 1, 2}, b6[6] = {0, 1, 0, 2, 1, 0};
-  static const bool six_env = [] { const char* e = getenv("ODEVIT_FP32_SEGMENTS"); return e && atoi(e) == 6; }();
-  const bool six = six_env && (g.kclass == KC_GEMM_IN || g.kclass == KC_GEMM_OUT);
-  const int ns = six ? 6 : 3;
-  const int* pa = six ? a6 : a3;
-  const int* pb = six ? b6 : b3;
+  // attention map of the 224 px RK4 case: 1.6e-4 with three segments, 2.2e-4 with six).
+  static const int pa[3] = {0, 0, 1}, pb[3] = {0, 1, 0};
+  constexpr int ns = 3;
   if ((size_t)ns * g.M * g.K * 2 > p.split_a_bytes || (size_t)ns * g.N * g.K * 2 > p.split_b_bytes) return 0;
   GemmArgs t = g;
   t.K = ns * g.K;
@@ -609,16 +603,12 @@ int attention_vjp(const Plan& p, const void* qkv_v, const void* oh, long long ld
 }
 
 // Forward evaluation at stage input `u`.  `rk` (nullable) is the epilogue of the last GEMM.
-// xc_mode: XC_CENTRE forms c.xc = u - mean_D(u); XC_READY: c.xc already holds the activation-type copy of u, written by
-// the epilogue that produced u (see operand_from_epilogue: the rows of W1cat are centred, so the operand needs no
-// centring of its own); XC_COPY forms that same plain copy here (a recomputing reverse sweep reproducing such a forward
-// from a trajectory row).
 int eval_forward(const Plan& p, const WeightBufs& wb, const StageCtx& c, const float* u, float* P,
                  float* p_copy, float* sq, float* tmp, long long e, const Epi* rk, cudaStream_t s,
-                 float* jas_out, int jas_k, int xc_mode) {
+                 float* jas_out, int jas_k) {
   if (p.variant == ODEVIT_FIELD_MACARON) return macaron_forward(p, wb, c, u, P, rk, e, s);
   const int D = p.D, hid = p.hid, R = 3 * D + hid, K2 = D + hid;
-  if (xc_mode != XC_READY) ODV_TRY(center_rows(u, c.xc, p.act, nullptr, 0.f, p.M, D, s, xc_mode == XC_CENTRE));
+  ODV_TRY(center_rows(u, c.xc, p.act, nullptr, 0.f, p.M, D, s));
   {
     GemmArgs g;
     g.M = p.M; g.N = R; g.K = D;
@@ -688,32 +678,6 @@ int eval_forward(const Plan& p, const WeightBufs& wb, const StageCtx& c, const f
 }
 
 namespace {
-// The stage-combine epilogue can write the NEXT evaluation's GEMM operand (the bf16 copy of the stage input it produces)
-// next to the fp32 value: with the centring folded into W1cat's rows (rows.cu::fold_w1_kernel) that copy needs no
-// `center_rows` pass (-10.6 us per evaluation for +1.5 us in the GEMM when timed kernel by kernel; the whole bench step does
-// NOT get faster -- 9.92 vs 9.81 ms, inference 13.4 k vs 15.7 k img/s: center_rows reads a state the GEMM has just left in
-// L2, while the extra bf16 store rides an epilogue that already waits on its operand feed).
-// bf16 mode only, and OPT-IN (ODEVIT_OPERAND_FROM_EPILOGUE=1).  The forward error against the oracle does not move
-// (tools/operand_probe.py on the D=128 distillation student, training mode: final state 2.23e-2 -> 2.17e-2, state 12
-// 3.4e-3 -> 4.0e-3 -- row means are <= 0.25 sigma there; the bench model at depth (224 px, T=24): final state 4.37e-3 ->
-// 4.42e-3, gradients 3.9e-3 -> 4.0e-3), but it IS a different rounding: that fixture's badly conditioned loss terms and
-// gradients land 2-3x further from the reference trainer's with it (kl 6e-3 -> 1.3e-2, worst gradient 0.10 -> 0.20, over
-// the test's bound), and every forward path must switch together (tape / recompute / trajectory-free solves are held
-// bitwise equal by the tests), so the measured parity numbers keep the exact centring as the default.
-// `with_tape` is kept for callers that want to tell the two kinds of solve apart.
-bool operand_from_epilogue(const Plan& p, bool with_tape) {
-  (void)with_tape;
-  static const bool on = [] { const char* v = getenv("ODEVIT_OPERAND_FROM_EPILOGUE"); return v && v[0] == '1'; }();
-  return on && p.variant != ODEVIT_FIELD_MACARON && p.precision == ODEVIT_BF16 && p.act == DT_BF16;
-}
-
-// arms `rk` to write the operand of evaluation e + 1 (the activation-type copy of the stage input it produces) into `xc_next`.
-// (A per-row shift by the previous input's row mean, with row sums accumulated by atomics in the epilogue, was built
-// and measured: +8 us per GEMM and a forward that is no longer bitwise reproducible -- dropped.)
-void arm_operand_epilogue(const Plan& p, Epi& rk, void* xc_next) {
-  rk.out2 = xc_next; rk.out2_scale = 1.f; rk.aux_type = p.act;
-}
-
 // Epilogue of stage `st` of a step starting at y with step dt: produces the next stage input
 // (or the step result when st == S-1) into `out`; stores k_st when a later stage needs it.
 Epi rk_epilogue(const Tableau& tb, int st, float dt, const float* y, float* const* k, float* out) {
@@ -746,9 +710,8 @@ int eval_vjp(const Plan& p, const WeightBufs& wb, const StageCtx& c, BwdBufs& b,
   const int D = p.D, hid = p.hid, R = 3 * D + hid, K2 = D + hid;
   const size_t e = dtype_size(p.act);
   char* dz = reinterpret_cast<char*>(b.dz);
-  static const bool colsum_fuse_off = [] { const char* v = getenv("ODEVIT_FUSED_COLSUM"); return v && v[0] == '0'; }();
   // (softmax attention, no attention-map dropout, the single-GEMM form of d[O|h]: see below)
-  bool fused_colsum = !colsum_fuse_off && p.variant == ODEVIT_FIELD_PARALLEL && p.p_attn == 0.f && !p.split_out;
+  bool fused_colsum = p.variant == ODEVIT_FIELD_PARALLEL && p.p_attn == 0.f && !p.split_out;
   if (p.split_out) {
     // the cotangent enters the out-proj branch under the proj mask and the fc2 branch under the mlp-output mask
     if (gw->fc2_b) return set_error(ODEVIT_ERR_UNSUPPORTED, "dropout with an fc2 bias is not built (the reference has none)");
@@ -1163,7 +1126,6 @@ int solve_fwd_impl(const odevit_desc* desc, const odevit_weights* w, int32_t met
     const long long n_evals = (long long)(n_grid - 1) * S;
     const float* row_prev = nullptr;   // row j - 1
     const float* row_cur = x0;         // row j
-    const bool from_epi = operand_from_epilogue(p, false);
     for (int j = 0; j + 1 < n_grid; ++j) {
       const float dt = t_grid_host[j + 1] - t_grid_host[j];
       float* y_next = slot_of(j + 1);
@@ -1176,8 +1138,7 @@ int solve_fwd_impl(const odevit_desc* desc, const odevit_weights* w, int32_t met
         if (st == S - 1 && row_prev && lean->fd_max) { rk.fd_prev = row_prev; rk.fd_out = lean->fd_max; }
         float* p_copy = (p_last && e == n_evals - 1) ? p_last : nullptr;
         float* jas_out = (jas_traj && e >= jas_first_eval) ? jas_traj + (size_t)(e - jas_first_eval) * p.B * p.H : nullptr;
-        if (from_epi && e + 1 < n_evals) arm_operand_epilogue(p, rk, f.ctx.xc);
-        ODV_TRY(eval_forward(p, f.w, f.ctx, u, f.P, p_copy, f.sq, f.tmp, e, &rk, s, jas_out, jas_k, from_epi && e > 0 ? XC_READY : XC_CENTRE));
+        ODV_TRY(eval_forward(p, f.w, f.ctx, u, f.P, p_copy, f.sq, f.tmp, e, &rk, s, jas_out, jas_k));
       }
       ODV_TRY(fan_out(j + 1, y_next));
       row_prev = row_cur;
@@ -1192,7 +1153,6 @@ int solve_fwd_impl(const odevit_desc* desc, const odevit_weights* w, int32_t met
   }
   const int S = tb->S;
   const long long n_evals = (long long)(n_grid - 1) * S;
-  const bool from_epi = operand_from_epilogue(p, tape != nullptr);
   for (int j = 0; j + 1 < n_grid; ++j) {
     const float dt = t_grid_host[j + 1] - t_grid_host[j];
     float* y_next = states ? states + (size_t)(j + 1) * MD
@@ -1207,9 +1167,7 @@ int solve_fwd_impl(const odevit_desc* desc, const odevit_weights* w, int32_t met
       else if (p_last && e == n_evals - 1) p_copy = p_last;
       const StageCtx ctx = tape ? tape_ctx(p, tape, e, nullptr, n_evals) : f.ctx;
       float* jas_out = (jas_traj && e >= jas_first_eval) ? jas_traj + (size_t)(e - jas_first_eval) * p.B * p.H : nullptr;
-      if (from_epi && e + 1 < n_evals)   // the next evaluation's operand (its own tape slot, or the shared context)
-        arm_operand_epilogue(p, rk, tape ? tape_ctx(p, tape, e + 1, nullptr, n_evals).xc : f.ctx.xc);
-      ODV_TRY(eval_forward(p, f.w, ctx, u, f.P, p_copy, f.sq, f.tmp, e, &rk, s, jas_out, jas_k, from_epi && e > 0 ? XC_READY : XC_CENTRE));
+      ODV_TRY(eval_forward(p, f.w, ctx, u, f.P, p_copy, f.sq, f.tmp, e, &rk, s, jas_out, jas_k));
       if (p_last && e == n_evals - 1 && p_copy != p_last)
         ODV_CUDA(cudaMemcpyAsync(p_last, p_copy, (size_t)p.BHNN * 4, cudaMemcpyDeviceToDevice, s));
     }
@@ -1342,17 +1300,12 @@ int odevit_solve_bwd(const odevit_desc* desc, const odevit_weights* w, int32_t m
       ctx[st] = tape ? tape_ctx(p, const_cast<void*>(tape), (long long)j * S + st, nullptr, 0) : b.ctx[st];
     for (int st = 0; st < S && !tape; ++st) {
       const float* u = (st == 0) ? y : b.u;
-      // the operands as the (tape-less) forward formed them: centred for the very first evaluation, else the plain copy --
-      // of the trajectory row (st = 0), or written by the previous stage's epilogue
-      const bool from_epi = operand_from_epilogue(p, false);
       const long long e = (long long)j * S + st;
-      const int xc_mode = !from_epi || e == 0 ? XC_CENTRE : (st == 0 ? XC_COPY : XC_READY);
       if (st < S - 1) {
         Epi rk = rk_epilogue(*tb, st, dt, y, b.k, b.u);
-        if (from_epi) arm_operand_epilogue(p, rk, b.ctx[st + 1].xc);
-        ODV_TRY(eval_forward(p, b.w, b.ctx[st], u, b.P, nullptr, b.sq, b.tmp, e, &rk, s, nullptr, 0, xc_mode));
+        ODV_TRY(eval_forward(p, b.w, b.ctx[st], u, b.P, nullptr, b.sq, b.tmp, e, &rk, s));
       } else {
-        ODV_TRY(eval_forward(p, b.w, b.ctx[st], u, b.P, nullptr, b.sq, b.tmp, e, nullptr, s, nullptr, 0, xc_mode));
+        ODV_TRY(eval_forward(p, b.w, b.ctx[st], u, b.P, nullptr, b.sq, b.tmp, e, nullptr, s));
       }
     }
     // (2) reverse through the stages

@@ -436,32 +436,6 @@ __device__ __forceinline__ void epi8_issue(const Epi& e, int m0, int M, int n, E
   }
 }
 
-// ---- L2 prefetch of the operand rows phase 1 will load for a LATER tile: lane = one row of the 32-row slab,
-//      `cols` consecutive columns from n0 (a 128-byte line per row and 32-column fp32 chunk) ----
-// (plain prefetch instructions, one per 32-byte sector: `cp.async.bulk.prefetch.L2` per lane queued ~800 tiny
-// operations per tile in front of the producer's operand loads in the TMA unit and made every GEMM slower)
-__device__ __forceinline__ void prefetch_l2_row(const char* p, int bytes) {
-#pragma unroll
-  for (int o = 0; o < 128; o += 32)
-    if (o < bytes) asm volatile("prefetch.global.L2 [%0];" ::"l"(p + o));
-}
-template <int EPI, bool ATOMIC>
-__device__ __forceinline__ void epi_prefetch_rows(const Epi& e, int m, int M, int n0, int N) {
-  if (m >= M || n0 >= N) return;
-  const int cols = min(32, N - n0);
-  if constexpr ((EPI & 7) == EPI_RK) {
-    if (e.y) prefetch_l2_row(reinterpret_cast<const char*>(e.y + (long long)m * e.ld_out + n0), cols * 4);
-  } else if constexpr ((EPI & 7) == EPI_BWD3) {
-    if (n0 >= e.split) {
-      const long long idx = (long long)m * e.ld_aux + (n0 - e.split);
-      if (e.aux_type == DT_F32) prefetch_l2_row(reinterpret_cast<const char*>(reinterpret_cast<const float*>(e.aux) + idx), cols * 4);
-      else prefetch_l2_row(reinterpret_cast<const char*>(reinterpret_cast<const __nv_bfloat16*>(e.aux) + idx), cols * 2);
-    }
-  } else if constexpr ((EPI & 7) == EPI_ACCUM && !ATOMIC) {
-    prefetch_l2_row(reinterpret_cast<const char*>(reinterpret_cast<const float*>(e.out) + (long long)m * e.ld_out + n0), cols * 4);
-  }
-}
-
 // column sums of the lane's 8 rows x 4 columns, reduced over the four lanes that hold the same columns (lane, lane ^ 8,
 // lane ^ 16, lane ^ 24), one float4 atomic per column group.  Every lane of the warp must call it.
 __device__ __forceinline__ void colsum_rows8(float* dst, const float4 (&w)[8]) {

@@ -19,10 +19,9 @@
 //   warps 2-9 epilogue (TMEM lane quarter x 2 column groups): tcgen05.ld 32 columns of 32 accumulator rows
 //            (thread = row), transpose through a swizzled shared-memory scratch so that 8 consecutive lanes
 //            hold 128 contiguous bytes of one output row, apply the fused epilogue on float4s with coalesced
-//            global loads / stores (epilogue.cuh: loads issued before the accumulator wait, operand rows of the
-//            next tile prefetched to L2).  Two accumulator buffers in TMEM let the epilogue of tile i overlap
-//            the main loop of tile i+1; the peer CTA's epilogue warps release the buffer with a remote arrive
-//            on the leader's `acc_empty` barrier.
+//            global loads / stores (epilogue.cuh: loads issued before the accumulator wait).  Two accumulator
+//            buffers in TMEM let the epilogue of tile i overlap the main loop of tile i+1; the peer CTA's epilogue
+//            warps release the buffer with a remote arrive on the leader's `acc_empty` barrier.
 // Operands may be K-major (row-major [rows, K]) or MN-major (row-major [K, rows], i.e. the
 // transposed products of the weight-gradient GEMMs); out-of-range rows / K are zero-filled by TMA.
 #include <cuda.h>
@@ -91,8 +90,6 @@ struct DevArgs {
   // stall the main loop on its accumulator buffers.  The skew makes that stride coprime with tiles_n (every unit cycles
   // through all N tiles, the expensive ones spread out); the set of tiles in flight per wave is unchanged.
   int tile_skew;
-  int l2_prefetch;   // epilogue operand rows of the next tile -> L2 (experiment switch ODEVIT_GEMM_PREFETCH)
-  int dbg;           // diagnostic builds only (ODEVIT_GEMM_DBG): 1 = skip the shared-memory transposition (wrong results)
   Epi epi;
 };
 
@@ -143,16 +140,6 @@ __device__ __forceinline__ void epilogue_role(const DevArgs& g, float* scratch, 
       const uint32_t acc_phase = (it >> 1) & 1;
       const uint32_t taddr = tmem_base + acc * C::ACC2 + (static_cast<uint32_t>(q * 32) << 16);
       const int m0 = m_base + rsub;
-      // the operand rows the NEXT tile's epilogue will load (state / GELU input / accumulator) -> L2, one tile ahead
-      const int tile_next = (it + 1) * num_units + (unit + g.tile_skew * (it + 1)) % num_units;
-      if (g.l2_prefetch && tile_next < total_tiles) {
-        int mb2, nt2;
-        tile_coords(tile_next, mb2, nt2);
-        for (int k = 0; k < my_chunks; ++k) {
-          if (atomic) epi_prefetch_rows<EPI, true>(g.epi, mb2 + lane, g.M, nt2 + (grp + k * EPI_GROUPS) * 32, g.N);
-          else epi_prefetch_rows<EPI, false>(g.epi, mb2 + lane, g.M, nt2 + (grp + k * EPI_GROUPS) * 32, g.N);
-        }
-      }
       // FULL: the 32-row slab lies inside M (no row predicates); ATOMIC: split-K accumulation
       auto chunks = [&](auto full_c, auto atomic_c) {
         constexpr bool FULL = decltype(full_c)::value, ATOMIC = decltype(atomic_c)::value;
@@ -169,9 +156,8 @@ __device__ __forceinline__ void epilogue_role(const DevArgs& g, float* scratch, 
           }
           GT_T0();
           // the chunk's global operand loads are issued behind the (asynchronous) accumulator load and overlap it and
-          // the transposition; their rows were prefetched to L2 one tile ago.  (Issued in FRONT of the accumulator wait
-          // they would be spilled at once: tcgen05.ld wants 32 consecutive registers and ptxas evicts whatever sits
-          // there to local memory.)
+          // the transposition.  (Issued in FRONT of the accumulator wait they would be spilled at once: tcgen05.ld wants
+          // 32 consecutive registers and ptxas evicts whatever sits there to local memory.)
           float v[32];
           ptx::tmem_ld32(taddr + c * 32, v);
           EpiPre pre;
@@ -190,20 +176,12 @@ __device__ __forceinline__ void epilogue_role(const DevArgs& g, float* scratch, 
           }
           // transpose: lane = row  ->  (row = i*4 + lane/8, 4 columns at (lane%8)*4)
           float4 w[8];
-#ifdef GEMM_TRACE
-          if (g.dbg & 1) {
 #pragma unroll
-            for (int i = 0; i < 8; ++i) w[i] = make_float4(v[4 * i], v[4 * i + 1], v[4 * i + 2], v[4 * i + 3]);
-          } else
-#endif
-          {
+          for (int j = 0; j < 8; ++j) ptx::sts_f32x4(st_base ^ (uint32_t)(j << 4), v[4 * j], v[4 * j + 1], v[4 * j + 2], v[4 * j + 3]);
+          __syncwarp();
 #pragma unroll
-            for (int j = 0; j < 8; ++j) ptx::sts_f32x4(st_base ^ (uint32_t)(j << 4), v[4 * j], v[4 * j + 1], v[4 * j + 2], v[4 * j + 3]);
-            __syncwarp();
-#pragma unroll
-            for (int i = 0; i < 8; ++i) w[i] = ptx::lds_f32x4(((i & 1) ? ld_base1 : ld_base0) + (uint32_t)(512 * i));
-            __syncwarp();
-          }
+          for (int i = 0; i < 8; ++i) w[i] = ptx::lds_f32x4(((i & 1) ? ld_base1 : ld_base0) + (uint32_t)(512 * i));
+          __syncwarp();
           if (live) epi8_finish<EPI, ATOMIC, FULL>(g.epi, m0, g.M, n, w, pre);
           GT_ADD(2);
         }
@@ -604,12 +582,6 @@ int gemm_tc(const GemmArgs& g, cudaStream_t s) {
   d.split_k = (d.num_kb + d.kb_per_split - 1) / d.kb_per_split;
   d.epi = g.epi;
   d.tile_skew = 0;
-  {
-    static const int pf = [] { const char* e = getenv("ODEVIT_GEMM_PREFETCH"); return e ? atoi(e) : 0; }();
-    d.l2_prefetch = pf;   // off: measured neutral to slightly negative (the operand loads are not what the epilogues wait for)
-    static const int dbg = [] { const char* e = getenv("ODEVIT_GEMM_DBG"); return e ? atoi(e) : 0; }();
-    d.dbg = dbg;
-  }
   CUtensorMap ta, tb;
   const int brows = bn / cg;
   if (!mn) {
@@ -624,9 +596,8 @@ int gemm_tc(const GemmArgs& g, cudaStream_t s) {
   const int units = total < max_units ? total : max_units;
   if ((g.epi_mode == EPI_FWD1 || g.epi_mode == EPI_BWD3) && d.tiles_n > 2 && total > units) {
     // epilogues whose cost depends on the N tile (GELU / GELU' on the fc1 columns only): see DevArgs::tile_skew
-    static const bool off = [] { const char* e = getenv("ODEVIT_GEMM_SKEW"); return e && e[0] == '0'; }();
     auto gcd = [](int a, int b) { while (b) { const int t = a % b; a = b; b = t; } return a; };
-    for (int sk = 0; sk < d.tiles_n && !off; ++sk) {
+    for (int sk = 0; sk < d.tiles_n; ++sk) {
       const int stride = (units + sk) % d.tiles_n;
       if (gcd(stride, d.tiles_n) == 1 && stride != 1 && stride != d.tiles_n - 1) { d.tile_skew = sk; break; }
     }

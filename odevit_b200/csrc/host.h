@@ -97,10 +97,9 @@ int check_weights(const Plan& p, const odevit_weights* w);
 int prepare_weights(const Plan& p, const odevit_weights* w, WeightBufs& wb, cudaStream_t s);
 
 // One forward field evaluation at `u` (api.cu); `rk` (nullable) is the epilogue of its last GEMM.
-enum { XC_CENTRE = 0, XC_READY = 1, XC_COPY = 2 };
 int eval_forward(const Plan& p, const WeightBufs& wb, const StageCtx& c, const float* u, float* P,
                  float* p_copy, float* sq, float* tmp, long long e, const Epi* rk, cudaStream_t s,
-                 float* jas_out = nullptr, int jas_k = 0, int xc_mode = XC_CENTRE);
+                 float* jas_out = nullptr, int jas_k = 0);
 
 // softmax(q k^T) v per (image, head) from the packed qkv buffer into oh[:, h*d ...] (leading dim ld_oh).
 // P: [B,H,N,N] fp32 scratch (unfused path); p_copy: optional export; lse: optional row log-sum-exp.

@@ -218,9 +218,8 @@ int attn_bwd_tc(const void* qkv, const void* dO, const void* oh, long long ld_oh
 // row-wise / elementwise kernels (odevit_rows.cu)
 // ---------------------------------------------------------------------------------------------
 // xc[r,:] = x[r,:] - mean(x[r,:]);  if rstd_out: also divide by sqrt(var+eps) (LayerNorm core)
-// subtract_mean = false (bf16 vector path only): xc = the plain copy of x in the activation type
 int center_rows(const float* x, void* xc, int xc_type, float* rstd_out, float eps, int rows,
-                int D, cudaStream_t s, bool subtract_mean = true);
+                int D, cudaStream_t s);
 // in-place softmax over rows of length n (fp32); optional second copy
 int softmax_rows(float* p, float* copy_to, long long rows, int n, cudaStream_t s);
 // ds = p * (dp + dpx - sum_j p*(dp+dpx)), written over dp.  dpx nullable.

@@ -66,7 +66,7 @@ __global__ void __launch_bounds__(256) center_rows_kernel(const float* __restric
 // bf16 field evaluation; the affine and D/(D-1) live in the folded weights)
 template <int CH>
 __global__ void __launch_bounds__(256) center_rows_bf16_vec_kernel(const float* __restrict__ x, __nv_bfloat16* __restrict__ xc,
-                                                                   int rows, int D, bool subtract_mean) {
+                                                                   int rows, int D) {
   const int row = blockIdx.x * 8 + (threadIdx.x >> 5);
   const int lane = threadIdx.x & 31;
   if (row >= rows) return;
@@ -80,7 +80,7 @@ __global__ void __launch_bounds__(256) center_rows_bf16_vec_kernel(const float* 
     v[i] = (c < n4) ? __ldg(xr + c) : make_float4(0.f, 0.f, 0.f, 0.f);
     s += (v[i].x + v[i].y) + (v[i].z + v[i].w);
   }
-  const float mean = subtract_mean ? warp_sum(s) / (float)D : 0.f;   // (false: the plain bf16 copy -- see api.cu::operand_from_epilogue)
+  const float mean = warp_sum(s) / (float)D;
   uint2* out = reinterpret_cast<uint2*>(xc + (long long)row * D);
 #pragma unroll
   for (int i = 0; i < CH; ++i) {
@@ -920,19 +920,18 @@ __global__ void __launch_bounds__(128) unfold_w2_kernel(UnfoldArgs a, odevit_wei
 }  // namespace
 
 int center_rows(const float* x, void* xc, int xc_type, float* rstd_out, float eps, int rows, int D,
-                cudaStream_t s, bool subtract_mean) {
+                cudaStream_t s) {
   ProfScope prof(KC_CENTER, s);
   if (D > 32 * MAX_PER_LANE) return set_error(ODEVIT_ERR_UNSUPPORTED, "center_rows: D=%d > 1024", D);
   if (xc_type == DT_BF16 && !rstd_out && D % 4 == 0 && (reinterpret_cast<uintptr_t>(x) & 15) == 0 &&
       (reinterpret_cast<uintptr_t>(xc) & 7) == 0) {
     __nv_bfloat16* o = reinterpret_cast<__nv_bfloat16*>(xc);
     const int ch = (D / 4 + 31) / 32;
-    if (ch <= 2) center_rows_bf16_vec_kernel<2><<<(rows + 7) / 8, 256, 0, s>>>(x, o, rows, D, subtract_mean);
-    else if (ch <= 4) center_rows_bf16_vec_kernel<4><<<(rows + 7) / 8, 256, 0, s>>>(x, o, rows, D, subtract_mean);
-    else if (ch <= 6) center_rows_bf16_vec_kernel<6><<<(rows + 7) / 8, 256, 0, s>>>(x, o, rows, D, subtract_mean);
-    else center_rows_bf16_vec_kernel<8><<<(rows + 7) / 8, 256, 0, s>>>(x, o, rows, D, subtract_mean);
+    if (ch <= 2) center_rows_bf16_vec_kernel<2><<<(rows + 7) / 8, 256, 0, s>>>(x, o, rows, D);
+    else if (ch <= 4) center_rows_bf16_vec_kernel<4><<<(rows + 7) / 8, 256, 0, s>>>(x, o, rows, D);
+    else if (ch <= 6) center_rows_bf16_vec_kernel<6><<<(rows + 7) / 8, 256, 0, s>>>(x, o, rows, D);
+    else center_rows_bf16_vec_kernel<8><<<(rows + 7) / 8, 256, 0, s>>>(x, o, rows, D);
   } else {
-    if (!subtract_mean) return set_error(ODEVIT_ERR_UNSUPPORTED, "center_rows: the plain copy is built for the bf16 vector path only");
     center_rows_kernel<<<(rows + 7) / 8, 256, 0, s>>>(x, xc, xc_type, rstd_out, eps, rows, D);
   }
   ODV_LAUNCH_CHECK();
