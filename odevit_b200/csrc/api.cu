@@ -85,11 +85,6 @@ namespace {
 // ------------------------------------------------------------------------------------------------
 // Butcher tableaux of the fixed-grid methods (torchdiffeq _impl/fixed_grid.py, rk_common.py)
 // ------------------------------------------------------------------------------------------------
-struct Tableau {
-  int S;
-  float a[4][4];  // u_m = y + dt * sum_l a[m][l] * k_l   (m >= 1)
-  float b[4];     // y_next = y + dt * sum_l b[l] * k_l
-};
 const Tableau kEuler = {1, {{0}}, {1.f}};
 const Tableau kMidpoint = {2, {{0}, {0.5f}}, {0.f, 1.f}};
 const Tableau kRk38 = {4,
@@ -272,28 +267,29 @@ BwdBufs layout_bwd(const Plan& p, Arena& a, int S) {
 
 // The tape: one StageCtx per field evaluation e = step*S + stage, written by the forward solve and
 // read by the reverse sweep instead of recomputing the step (HBM is 180 GB: at the C100 bench shape
-// the tape is 3.3 GB).  Layout is a pure function of (plan, n_evals).
-StageCtx tape_ctx(const Plan& p, void* tape, long long e, size_t* total_bytes, long long n_evals) {
-  Arena a0(nullptr);
-  take_ctx(p, a0, true);
-  const size_t per = (a0.off + 1023) & ~size_t(1023);
-  if (total_bytes) {
-    Arena aw(nullptr);
-    take_weights(p, aw);                     // the folded weights of the forward, kept for the reverse sweep (tape_weights)
-    *total_bytes = per * (size_t)n_evals + ((aw.off + 1023) & ~size_t(1023));
-  }
-  if (!tape) return StageCtx{};
-  Arena a(reinterpret_cast<char*>(tape) + per * (size_t)e);
+// the tape is 3.3 GB).  Layout is a pure function of (plan, n_evals): n_evals slots of tape_slot_bytes,
+// then the folded weights of the forward (tape_weights).
+size_t tape_slot_bytes(const Plan& p) {
+  Arena a(nullptr);
+  take_ctx(p, a, true);
+  return (a.off + 1023) & ~size_t(1023);
+}
+
+size_t tape_bytes(const Plan& p, long long n_evals) {
+  Arena aw(nullptr);
+  take_weights(p, aw);
+  return tape_slot_bytes(p) * (size_t)n_evals + ((aw.off + 1023) & ~size_t(1023));
+}
+
+StageCtx tape_ctx(const Plan& p, const void* tape, long long e) {
+  Arena a(const_cast<char*>(reinterpret_cast<const char*>(tape)) + tape_slot_bytes(p) * (size_t)e);
   return take_ctx(p, a, true);
 }
 
 // The folded / transposed weights of the forward solve, stored behind the tape's evaluation slots: the reverse sweep of
 // the same step reads them instead of folding the (unchanged) parameters a second time.
-WeightBufs tape_weights(const Plan& p, void* tape, long long n_evals) {
-  Arena a0(nullptr);
-  take_ctx(p, a0, true);
-  const size_t per = (a0.off + 1023) & ~size_t(1023);
-  Arena a(reinterpret_cast<char*>(tape) + per * (size_t)n_evals);
+WeightBufs tape_weights(const Plan& p, const void* tape, long long n_evals) {
+  Arena a(const_cast<char*>(reinterpret_cast<const char*>(tape)) + tape_slot_bytes(p) * (size_t)n_evals);
   return take_weights(p, a);
 }
 
@@ -302,6 +298,11 @@ int check_ws(const void* ws, size_t have, size_t need) {
   if (reinterpret_cast<uintptr_t>(ws) & 1023) return set_error(ODEVIT_ERR_WORKSPACE, "workspace not 1024-byte aligned");
   if (have < need) return set_error(ODEVIT_ERR_WORKSPACE, "workspace too small: %zu < %zu bytes", have, need);
   return 0;
+}
+
+int check_tape(const Plan& p, const void* tape, size_t bytes, long long n_evals) {
+  ODV_TRY(check_device_ptr(tape, "tape"));
+  return check_ws(tape, bytes, tape_bytes(p, n_evals));
 }
 
 int check_device_ptr(const void* p, const char* what) {
@@ -677,9 +678,6 @@ int eval_forward(const Plan& p, const WeightBufs& wb, const StageCtx& c, const f
   return 0;
 }
 
-namespace {
-// Epilogue of stage `st` of a step starting at y with step dt: produces the next stage input
-// (or the step result when st == S-1) into `out`; stores k_st when a later stage needs it.
 Epi rk_epilogue(const Tableau& tb, int st, float dt, const float* y, float* const* k, float* out) {
   Epi e;
   e.out = out;
@@ -688,13 +686,41 @@ Epi rk_epilogue(const Tableau& tb, int st, float dt, const float* y, float* cons
   const bool last = (st == tb.S - 1);
   const float* row = last ? tb.b : tb.a[st + 1];
   e.c_new = dt * row[st];
-  for (int l = 0; l < st && l < 3; ++l) {
+  for (int l = 0; l < st; ++l) {
     if (row[l] != 0.f) { e.kin[l] = k[l]; e.c_k[l] = dt * row[l]; }
   }
-  e.k_store = (!last && st < 3) ? k[st] : nullptr;
+  e.k_store = last ? nullptr : k[st];
   return e;
 }
-}  // namespace
+
+// What one forward evaluation of a fixed-grid step keeps besides its stage combine: its intermediates (a tape slot or
+// the workspace's context) and, when wanted, its attention map and JaSMin statistic.
+struct EvalOut {
+  StageCtx ctx;
+  float* p_copy = nullptr;
+  float* jas_out = nullptr;
+  int jas_k = 0;
+};
+
+// The S stages of step j from row y with step dt: evaluation e = j*S + st (the dropout masks are keyed by it).  Stage 0
+// reads y, the later stages the stage buffer b.u; the epilogues (rk_epilogue) form each next stage input in b.u and the
+// step result in y_next.  out(e, st) gives each evaluation's EvalOut.  With fd_prev and fd_out, the last stage also folds
+// the finite-difference maxima of (fd_prev, y, y_next) into fd_out.  y_next == nullptr recomputes the intermediates
+// only: the last stage runs without its output GEMM.
+template <class Bufs, class Out>
+int rk_step(const Plan& p, const Bufs& b, const Tableau& tb, int j, float dt, const float* y, float* y_next,
+            const float* fd_prev, float* fd_out, Out out, cudaStream_t s) {
+  for (int st = 0; st < tb.S; ++st) {
+    const long long e = (long long)j * tb.S + st;
+    const bool last = (st == tb.S - 1);
+    const EvalOut o = out(e, st);
+    Epi rk = rk_epilogue(tb, st, dt, y, b.k, last ? y_next : b.u);
+    if (last && fd_prev && fd_out) { rk.fd_prev = fd_prev; rk.fd_out = fd_out; }
+    const Epi* epi = (last && !y_next) ? nullptr : &rk;
+    ODV_TRY(eval_forward(p, b.w, o.ctx, st == 0 ? y : b.u, b.P, o.p_copy, b.sq, b.tmp, e, epi, s, o.jas_out, o.jas_k));
+  }
+  return 0;
+}
 
 // VJP of one field evaluation: given dd = scaler * lambda (cotangent of the pre-scaler output, in
 // the activation type) and the stage intermediates `c`, accumulate G1, c1, G2, c2 and deliver
@@ -1012,9 +1038,7 @@ size_t odevit_tape_bytes(const odevit_desc* desc, int32_t method, int32_t n_grid
   if (make_plan(desc, &p)) return 0;
   const Tableau* tb = tableau_for(method);
   if (!tb || n_grid < 1) { set_error(ODEVIT_ERR_INVALID_ARG, "unknown method %d / empty grid", method); return 0; }
-  size_t need = 0;
-  tape_ctx(p, nullptr, 0, &need, (long long)(n_grid - 1) * tb->S);
-  return need;
+  return tape_bytes(p, (long long)(n_grid - 1) * tb->S);
 }
 
 int odevit_field_fwd(const odevit_desc* desc, const odevit_weights* w, const float* x, float* dx,
@@ -1049,6 +1073,9 @@ struct LeanOut {
   float* fd_max;
 };
 
+// The fixed-grid forward solve.  lean == nullptr: the trajectory into `states` and, when given, a tape for the reverse
+// sweep.  Otherwise trajectory-free: the rows live in a ring of three (the finite-difference window), in the caller's
+// slots of `rows_out` when they are control points, in `final_state` when last.
 int solve_fwd_impl(const odevit_desc* desc, const odevit_weights* w, int32_t method, const float* x0,
                    const float* t_grid_host, int32_t n_grid, float* states, float* final_state,
                    float* p_last, float* p_traj, int32_t p_traj_first_eval, float* jas_traj,
@@ -1066,12 +1093,8 @@ int solve_fwd_impl(const odevit_desc* desc, const odevit_weights* w, int32_t met
   const Tableau* tb = tableau_for(method);
   if (!tb) return set_error(ODEVIT_ERR_INVALID_ARG, "unknown method %d", method);
   if (!t_grid_host || n_grid < 1) return set_error(ODEVIT_ERR_INVALID_ARG, "t_grid must hold >= 1 point");
-  if (tape) {
-    size_t need = 0;
-    tape_ctx(p, nullptr, 0, &need, (long long)(n_grid - 1) * tb->S);
-    ODV_TRY(check_device_ptr(tape, "tape"));
-    ODV_TRY(check_ws(tape, tape_bytes, need));
-  }
+  const long long n_evals = (long long)(n_grid - 1) * tb->S;
+  if (tape) ODV_TRY(check_tape(p, tape, tape_bytes, n_evals));
   if (!states && !final_state) return set_error(ODEVIT_ERR_INVALID_ARG, "states and final_state both NULL");
   if (p.variant == ODEVIT_FIELD_MACARON && (p_last || p_traj))
     return set_error(ODEVIT_ERR_INVALID_ARG, "MACARON exposes no attention map (need_weights=False, macaron.py:60-65)");
@@ -1083,99 +1106,74 @@ int solve_fwd_impl(const odevit_desc* desc, const odevit_weights* w, int32_t met
   }
   if (n_grid == 2 && t_grid_host[1] == t_grid_host[0])
     return set_error(ODEVIT_ERR_INVALID_ARG, "t must be strictly increasing or decreasing");
+  if (lean && (states || tape)) return set_error(ODEVIT_ERR_INVALID_ARG, "the trajectory-free solve keeps neither states nor a tape");
+  const LeanOut lo = lean ? *lean : LeanOut{nullptr, nullptr, 0, nullptr};
+  for (int i = 0; i < lo.n_rows; ++i)
+    if (lo.row_index[i] < 0 || lo.row_index[i] >= n_grid)
+      return set_error(ODEVIT_ERR_INVALID_ARG, "row_index[%d]=%d outside [0,%d)", i, lo.row_index[i], n_grid);
   Arena a(workspace);
   FwdBufs f = layout_fwd(p, a, tb->S);
   ODV_TRY(check_ws(workspace, workspace_bytes, a.off));
   cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
   const size_t MD = (size_t)p.M * p.D;
-  ODV_TRY(prepare_drop_keys(p, f.drop_keys, (long long)(n_grid - 1) * tb->S, s));
-  if (tape) f.w = tape_weights(p, tape, (long long)(n_grid - 1) * tb->S);   // fold once per step: the reverse sweep reuses them
+  ODV_TRY(prepare_drop_keys(p, f.drop_keys, n_evals, s));
+  if (tape) f.w = tape_weights(p, tape, n_evals);   // fold once per step: the reverse sweep reuses them
   ODV_TRY(prepare_weights(p, w, f.w, s));
 
-  const float* y = x0;
+  const float* y = x0;   // row j
   if (states) {
     ODV_CUDA(cudaMemcpyAsync(states, x0, MD * 4, cudaMemcpyDeviceToDevice, s));
     y = states;
   }
-  if (lean) {
-    // ---- trajectory-free: rows live in a ring of three (the finite-difference window), in the caller's slots of
-    //      `rows_out` when they are control points, in `final_state` when last ----
-    if (states || tape) return set_error(ODEVIT_ERR_INVALID_ARG, "the trajectory-free solve keeps neither states nor a tape");
-    for (int i = 0; i < lean->n_rows; ++i)
-      if (lean->row_index[i] < 0 || lean->row_index[i] >= n_grid)
-        return set_error(ODEVIT_ERR_INVALID_ARG, "row_index[%d]=%d outside [0,%d)", i, lean->row_index[i], n_grid);
-    if (lean->fd_max) ODV_CUDA(cudaMemsetAsync(lean->fd_max, 0, (size_t)p.M * 4, s));
-    auto slot_of = [&](int j) -> float* {   // first caller slot that wants row j
-      for (int i = 0; i < lean->n_rows; ++i)
-        if (lean->row_index[i] == j) return lean->rows_out + (size_t)i * MD;
-      return nullptr;
-    };
-    auto fan_out = [&](int j, const float* src) -> int {   // row j into every further slot that names it
-      bool first = true;
-      for (int i = 0; i < lean->n_rows; ++i) {
-        if (lean->row_index[i] != j) continue;
-        float* dst = lean->rows_out + (size_t)i * MD;
-        if (first && dst == src) { first = false; continue; }
-        first = false;
-        ODV_CUDA(cudaMemcpyAsync(dst, src, MD * 4, cudaMemcpyDeviceToDevice, s));
-      }
-      return 0;
-    };
-    ODV_TRY(fan_out(0, x0));
-    const int S = tb->S;
-    const long long n_evals = (long long)(n_grid - 1) * S;
-    const float* row_prev = nullptr;   // row j - 1
-    const float* row_cur = x0;         // row j
-    for (int j = 0; j + 1 < n_grid; ++j) {
-      const float dt = t_grid_host[j + 1] - t_grid_host[j];
-      float* y_next = slot_of(j + 1);
-      if (!y_next) y_next = (j + 2 == n_grid && final_state) ? final_state : f.ytmp[(j + 1) % 3];
-      for (int st = 0; st < S; ++st) {
-        const long long e = (long long)j * S + st;
-        const float* u = (st == 0) ? row_cur : f.u;
-        float* out = (st == S - 1) ? y_next : f.u;
-        Epi rk = rk_epilogue(*tb, st, dt, row_cur, f.k, out);
-        if (st == S - 1 && row_prev && lean->fd_max) { rk.fd_prev = row_prev; rk.fd_out = lean->fd_max; }
-        float* p_copy = (p_last && e == n_evals - 1) ? p_last : nullptr;
-        float* jas_out = (jas_traj && e >= jas_first_eval) ? jas_traj + (size_t)(e - jas_first_eval) * p.B * p.H : nullptr;
-        ODV_TRY(eval_forward(p, f.w, f.ctx, u, f.P, p_copy, f.sq, f.tmp, e, &rk, s, jas_out, jas_k));
-      }
-      ODV_TRY(fan_out(j + 1, y_next));
-      row_prev = row_cur;
-      row_cur = y_next;
+  // small-token shapes: the whole solve of an image in one persistent CTA, state resident on the chip.  It writes
+  // neither rows_out nor fd_max, so the trajectory-free mode never takes it.
+  if (!lean && solve_resident_supports(p, n_grid, p_traj != nullptr || jas_traj != nullptr, tape != nullptr) &&
+      (tb->S == 1 || f.kbuf))
+    return solve_resident(p, f.w, *tb, x0, t_grid_host, n_grid, states, final_state, p_last, f.kbuf, s);
+
+  if (lo.fd_max) ODV_CUDA(cudaMemsetAsync(lo.fd_max, 0, (size_t)p.M * 4, s));
+  auto next_row = [&](int j) -> float* {   // where row j + 1 goes
+    if (states) return states + (size_t)(j + 1) * MD;
+    for (int i = 0; i < lo.n_rows; ++i)    // the first caller slot that names it
+      if (lo.row_index[i] == j + 1) return lo.rows_out + (size_t)i * MD;
+    if (j + 2 == n_grid && final_state) return final_state;
+    return f.ytmp[(j + 1) % 3];            // rows j - 1 and j stay readable
+  };
+  auto fan_out = [&](int j, const float* src) -> int {   // row j into every further slot that names it
+    bool first = true;
+    for (int i = 0; i < lo.n_rows; ++i) {
+      if (lo.row_index[i] != j) continue;
+      float* dst = lo.rows_out + (size_t)i * MD;
+      if (first && dst == src) { first = false; continue; }
+      first = false;
+      ODV_CUDA(cudaMemcpyAsync(dst, src, MD * 4, cudaMemcpyDeviceToDevice, s));
     }
-    if (final_state && row_cur != final_state) ODV_CUDA(cudaMemcpyAsync(final_state, row_cur, MD * 4, cudaMemcpyDeviceToDevice, s));
     return 0;
-  }
-  if (solve_resident_supports(p, n_grid, p_traj != nullptr || jas_traj != nullptr, tape != nullptr) && (tb->S == 1 || f.kbuf)) {
-    // small-token shapes: the whole solve of an image in one persistent CTA, state resident on the chip
-    return solve_resident(p, f.w, tb->S, tb->a, tb->b, x0, t_grid_host, n_grid, states, final_state, p_last, f.kbuf, s);
-  }
-  const int S = tb->S;
-  const long long n_evals = (long long)(n_grid - 1) * S;
+  };
+  auto p_slot = [&](long long e) -> float* {   // where the attention map of evaluation e goes
+    if (p_traj && e >= p_traj_first_eval) return p_traj + (size_t)(e - p_traj_first_eval) * p.BHNN;
+    return (p_last && e == n_evals - 1) ? p_last : nullptr;
+  };
+  auto out = [&](long long e, int) {
+    EvalOut o;
+    o.ctx = tape ? tape_ctx(p, tape, e) : f.ctx;
+    o.p_copy = p_slot(e);
+    if (jas_traj && e >= jas_first_eval) o.jas_out = jas_traj + (size_t)(e - jas_first_eval) * p.B * p.H;
+    o.jas_k = jas_k;
+    return o;
+  };
+  ODV_TRY(fan_out(0, x0));
+  const float* y_prev = nullptr;   // row j - 1
   for (int j = 0; j + 1 < n_grid; ++j) {
-    const float dt = t_grid_host[j + 1] - t_grid_host[j];
-    float* y_next = states ? states + (size_t)(j + 1) * MD
-                           : ((j + 2 == n_grid) ? final_state : f.ytmp[j & 1]);
-    for (int st = 0; st < S; ++st) {
-      const long long e = (long long)j * S + st;
-      const float* u = (st == 0) ? y : f.u;
-      float* out = (st == S - 1) ? y_next : f.u;
-      Epi rk = rk_epilogue(*tb, st, dt, y, f.k, out);
-      float* p_copy = nullptr;
-      if (p_traj && e >= p_traj_first_eval) p_copy = p_traj + (size_t)(e - p_traj_first_eval) * p.BHNN;
-      else if (p_last && e == n_evals - 1) p_copy = p_last;
-      const StageCtx ctx = tape ? tape_ctx(p, tape, e, nullptr, n_evals) : f.ctx;
-      float* jas_out = (jas_traj && e >= jas_first_eval) ? jas_traj + (size_t)(e - jas_first_eval) * p.B * p.H : nullptr;
-      ODV_TRY(eval_forward(p, f.w, ctx, u, f.P, p_copy, f.sq, f.tmp, e, &rk, s, jas_out, jas_k));
-      if (p_last && e == n_evals - 1 && p_copy != p_last)
-        ODV_CUDA(cudaMemcpyAsync(p_last, p_copy, (size_t)p.BHNN * 4, cudaMemcpyDeviceToDevice, s));
-    }
+    float* y_next = next_row(j);
+    ODV_TRY(rk_step(p, f, *tb, j, t_grid_host[j + 1] - t_grid_host[j], y, y_next, y_prev, lo.fd_max, out, s));
+    ODV_TRY(fan_out(j + 1, y_next));
+    y_prev = y;
     y = y_next;
   }
-  if (final_state && (states || n_grid == 1)) {
-    ODV_CUDA(cudaMemcpyAsync(final_state, y, MD * 4, cudaMemcpyDeviceToDevice, s));
-  }
+  if (p_last && n_evals > 0 && p_slot(n_evals - 1) != p_last)   // p_traj holds the last evaluation's map
+    ODV_CUDA(cudaMemcpyAsync(p_last, p_slot(n_evals - 1), (size_t)p.BHNN * 4, cudaMemcpyDeviceToDevice, s));
+  if (final_state && y != final_state) ODV_CUDA(cudaMemcpyAsync(final_state, y, MD * 4, cudaMemcpyDeviceToDevice, s));
   return 0;
 }
 }  // namespace
@@ -1231,12 +1229,7 @@ int odevit_solve_bwd(const odevit_desc* desc, const odevit_weights* w, int32_t m
   for (int i = 0; i < n_g_rows; ++i)
     if (g_row_index_host[i] < 0 || g_row_index_host[i] >= n_grid)
       return set_error(ODEVIT_ERR_INVALID_ARG, "g_row_index[%d]=%d outside [0,%d)", i, g_row_index_host[i], n_grid);
-  if (tape) {
-    size_t need = 0;
-    tape_ctx(p, nullptr, 0, &need, (long long)(n_grid - 1) * tb->S);
-    ODV_TRY(check_device_ptr(tape, "tape"));
-    ODV_TRY(check_ws(tape, tape_bytes, need));
-  }
+  if (tape) ODV_TRY(check_tape(p, tape, tape_bytes, (long long)(n_grid - 1) * tb->S));
   Arena a(workspace);
   BwdBufs b = layout_bwd(p, a, tb->S);
   ODV_TRY(check_ws(workspace, workspace_bytes, a.off));
@@ -1246,7 +1239,7 @@ int odevit_solve_bwd(const odevit_desc* desc, const odevit_weights* w, int32_t m
   const bool need_c2 = wants_c2(gw);
   ODV_TRY(prepare_drop_keys(p, b.drop_keys, (long long)(n_grid - 1) * S, s));
   if (tape) {   // the forward of this step left its folded weights behind the tape's slots
-    b.w = tape_weights(p, const_cast<void*>(tape), (long long)(n_grid - 1) * S);
+    b.w = tape_weights(p, tape, (long long)(n_grid - 1) * S);
     b.w.user = w;
   } else {
     ODV_TRY(prepare_weights(p, w, b.w, s));
@@ -1297,17 +1290,10 @@ int odevit_solve_bwd(const odevit_desc* desc, const odevit_weights* w, int32_t m
     //     else recomputed from the trajectory row (the last stage skips GEMM2)
     StageCtx ctx[4];
     for (int st = 0; st < S; ++st)
-      ctx[st] = tape ? tape_ctx(p, const_cast<void*>(tape), (long long)j * S + st, nullptr, 0) : b.ctx[st];
-    for (int st = 0; st < S && !tape; ++st) {
-      const float* u = (st == 0) ? y : b.u;
-      const long long e = (long long)j * S + st;
-      if (st < S - 1) {
-        Epi rk = rk_epilogue(*tb, st, dt, y, b.k, b.u);
-        ODV_TRY(eval_forward(p, b.w, b.ctx[st], u, b.P, nullptr, b.sq, b.tmp, e, &rk, s));
-      } else {
-        ODV_TRY(eval_forward(p, b.w, b.ctx[st], u, b.P, nullptr, b.sq, b.tmp, e, nullptr, s));
-      }
-    }
+      ctx[st] = tape ? tape_ctx(p, tape, (long long)j * S + st) : b.ctx[st];
+    if (!tape)
+      ODV_TRY(rk_step(p, b, *tb, j, dt, y, nullptr, nullptr, nullptr,
+                      [&](long long, int st) { return EvalOut{b.ctx[st]}; }, s));
     // (2) reverse through the stages
     //     lambda_st = dt*(b[st]*G + sum_{m>st} a[m][st]*mu_m),  mu_st = J(u_st)^T lambda_st,
     //     dL/dy = G + sum_st mu_st  (+ the cotangents injected at row j)

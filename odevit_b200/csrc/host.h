@@ -96,6 +96,17 @@ int check_device_ptr(const void* p, const char* what);
 int check_weights(const Plan& p, const odevit_weights* w);
 int prepare_weights(const Plan& p, const odevit_weights* w, WeightBufs& wb, cudaStream_t s);
 
+// Butcher tableau of an explicit Runge-Kutta method: the fixed-grid methods (api.cu, up to 4 stages) and Dormand-Prince
+// (solve_adaptive.cu, 6 stages)
+struct Tableau {
+  int S;
+  float a[6][6];  // u_m = y + dt * sum_l a[m][l] * k_l   (m >= 1)
+  float b[6];     // y_next = y + dt * sum_l b[l] * k_l
+};
+// Epilogue of stage `st` of a step starting at y with step dt (api.cu): produces the next stage input (or the step result
+// when st == S-1) into `out`; stores k_st into k[st] when a later stage needs it.  k[l] is null where no buffer exists.
+Epi rk_epilogue(const Tableau& tb, int st, float dt, const float* y, float* const* k, float* out);
+
 // One forward field evaluation at `u` (api.cu); `rk` (nullable) is the epilogue of its last GEMM.
 int eval_forward(const Plan& p, const WeightBufs& wb, const StageCtx& c, const float* u, float* P,
                  float* p_copy, float* sq, float* tmp, long long e, const Epi* rk, cudaStream_t s,
@@ -118,16 +129,18 @@ int attention_vjp(const Plan& p, const void* qkv, const void* oh, long long ld_o
 bool solve_resident_shape_ok(const Plan& p);
 bool solve_resident_supports(const Plan& p, int n_grid, bool wants_p_traj, bool has_tape);
 size_t solve_resident_scratch_floats(const Plan& p);
-int solve_resident(const Plan& p, const WeightBufs& wb, int S, const float (*ta)[4], const float* tbv, const float* x0,
-                   const float* t_host, int n_grid, float* states, float* final_state, float* p_last, float* kbuf,
-                   cudaStream_t s);
+int solve_resident(const Plan& p, const WeightBufs& wb, const Tableau& tb, const float* x0, const float* t_host,
+                   int n_grid, float* states, float* final_state, float* p_last, float* kbuf, cudaStream_t s);
 
 // Reverse-sweep pieces shared by odevit_solve_bwd and odevit_solve_adaptive_bwd (api.cu):
-//   layout_bwd: the fixed-grid workspace for S stages;  tape_ctx: slot e of a tape of n_evals evaluations (its byte count
-//   into *total_bytes when given);  eval_vjp: VJP of one field evaluation, mu delivered through `mu_epi` (the EPI_RK
-//   epilogue of its last GEMM);  finish_grads: the accumulators unfolded into the caller's gradients, once per call
+//   layout_bwd: the fixed-grid workspace for S stages;  tape_bytes / check_tape / tape_ctx: the size of a tape of n_evals
+//   evaluations, the check of a caller's tape against it, and the context of evaluation e in it;  eval_vjp: VJP of one
+//   field evaluation, mu delivered through `mu_epi` (the EPI_RK epilogue of its last GEMM);  finish_grads: the
+//   accumulators unfolded into the caller's gradients, once per call
 BwdBufs layout_bwd(const Plan& p, Arena& a, int S);
-StageCtx tape_ctx(const Plan& p, void* tape, long long e, size_t* total_bytes, long long n_evals);
+size_t tape_bytes(const Plan& p, long long n_evals);
+int check_tape(const Plan& p, const void* tape, size_t bytes, long long n_evals);
+StageCtx tape_ctx(const Plan& p, const void* tape, long long e);
 int eval_vjp(const Plan& p, const WeightBufs& wb, const StageCtx& c, BwdBufs& b, const float* g_p, bool need_c2,
              const odevit_weight_grads* gw, long long ev, const Epi& mu_epi, cudaStream_t s);
 int finish_grads(const Plan& p, const odevit_weights* w, const odevit_weight_grads* gw, const BwdBufs& b, cudaStream_t s);

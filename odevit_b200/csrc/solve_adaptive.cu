@@ -37,14 +37,17 @@
 namespace odevit {
 namespace {
 
-// Dormand-Prince tableau with Shampine's dense-output midpoint (torchdiffeq _impl/dopri5.py)
-constexpr double kBeta[6][6] = {
-    {1. / 5},
-    {3. / 40, 9. / 40},
-    {44. / 45, -56. / 15, 32. / 9},
-    {19372. / 6561, -25360. / 2187, 64448. / 6561, -212. / 729},
-    {9017. / 3168, -355. / 33, 46732. / 5247, 49. / 176, -5103. / 18656},
-    {35. / 384, 0, 500. / 1113, 125. / 192, -2187. / 6784, 11. / 84}};   // = c_sol[:6]
+// Dormand-Prince tableau with Shampine's dense-output midpoint (torchdiffeq _impl/dopri5.py): a[m] = beta[m - 1],
+// b = c_sol[:6]
+const Tableau kDopri5 = {
+    6,
+    {{0},
+     {(float)(1. / 5)},
+     {(float)(3. / 40), (float)(9. / 40)},
+     {(float)(44. / 45), (float)(-56. / 15), (float)(32. / 9)},
+     {(float)(19372. / 6561), (float)(-25360. / 2187), (float)(64448. / 6561), (float)(-212. / 729)},
+     {(float)(9017. / 3168), (float)(-355. / 33), (float)(46732. / 5247), (float)(49. / 176), (float)(-5103. / 18656)}},
+    {(float)(35. / 384), 0.f, (float)(500. / 1113), (float)(125. / 192), (float)(-2187. / 6784), (float)(11. / 84)}};
 __constant__ float kCErr[7] = {(float)(35. / 384 - 1951. / 21600), 0.f, (float)(500. / 1113 - 22642. / 50085),
                                (float)(125. / 192 - 451. / 720), (float)(-2187. / 6784 + 12231. / 42400),
                                (float)(11. / 84 - 649. / 6300), (float)(-1. / 60)};
@@ -384,6 +387,23 @@ int eval_plain(const Plan& p, AdBufs& f, const float* u, float* out, cudaStream_
   return eval_forward(p, f.w, f.ctx, u, f.P, nullptr, f.sq, nullptr, 0, &e, s);
 }
 
+// The stages k2..k6 of one step of every image from y0 and k[0] = k1 (FSAL): u2 by a row pass, then the evaluation of
+// u_{m+1} stores k_{m+1} and its epilogue forms u_{m+2} in u (y1 after k6).  ctx(m): the intermediates of that
+// evaluation.  y1 == nullptr recomputes the intermediates only: k6's output GEMM is skipped.
+template <class Ctx>
+int dp_stages(const Plan& p, const WeightBufs& w, Ctx ctx, float* P, float* sq, const float* y0, float* const* k,
+              const double* dt, float* u, float* y1, cudaStream_t s) {
+  ODV_TRY(row_axpy(p, y0, k[0], kDopri5.a[1][0], dt, u, s));
+  for (int m = 1; m <= 5; ++m) {
+    if (!y1 && m == 5) return eval_forward(p, w, ctx(m), u, P, nullptr, sq, nullptr, 0, nullptr, s);
+    Epi e = rk_epilogue(kDopri5, m, 1.f, y0, k, m == 5 ? y1 : u);   // dt_b is applied per image in the epilogue
+    e.row_dt = dt; e.rows_per_image = p.N;
+    e.k_store = k[m];
+    ODV_TRY(eval_forward(p, w, ctx(m), u, P, nullptr, sq, nullptr, 0, &e, s));
+  }
+  return 0;
+}
+
 struct Host {
   int* pinned = nullptr;             // [2][4] sync words of rounds with r & 1 == 0 / 1
   cudaEvent_t ev[2] = {nullptr, nullptr};
@@ -548,19 +568,7 @@ int solve_adaptive_impl(const odevit_desc* desc, const odevit_weights* w, const 
     const int c = (int)(r & 1), n = c ^ 1;
     const double* dt = f.dt + (size_t)c * B;
     ODV_CUDA(cudaMemsetAsync(f.sync + c, 0, sizeof(int), s));
-    ODV_TRY(row_axpy(p, f.y0, f.k[0], (float)kBeta[0][0], dt, f.u, s));   // u2
-    for (int m = 1; m <= 5; ++m) {   // evaluation of u_{m+1} gives k_{m+1} and forms u_{m+2} (y1 after k6)
-      Epi e;
-      e.y = f.y0; e.y_coef = 1.f;
-      e.row_dt = dt; e.rows_per_image = N;
-      e.k_store = f.k[m];
-      e.c_new = (float)kBeta[m][m];
-      for (int l = 0, slot = 0; l < m; ++l)
-        if (kBeta[m][l] != 0.0) { e.kin[slot] = f.k[l]; e.c_k[slot] = (float)kBeta[m][l]; ++slot; }
-      float* out = (m == 5) ? f.y1 : f.u;
-      e.out = out;
-      ODV_TRY(eval_forward(p, f.w, f.ctx, f.u, f.P, nullptr, f.sq, nullptr, 0, &e, s));
-    }
+    ODV_TRY(dp_stages(p, f.w, [&](int) { return f.ctx; }, f.P, f.sq, f.y0, f.k, dt, f.u, f.y1, s));
     ODV_TRY(eval_plain(p, f, f.y1, f.k[6], s));   // k7 = f(y1)
     ad_rowsq_kernel<RS_ERR><<<row_blocks, 256, 0, s>>>(f.y0, f.y1, f.k[0], nullptr, f.k[2], f.k[3], f.k[4], f.k[5],
                                                        f.k[6], dt, frtol, fatol, p.M, N, D, f.row0, nullptr);
@@ -639,9 +647,7 @@ extern "C" size_t odevit_adaptive_tape_bytes(const odevit_desc* desc, int32_t S)
   Plan p{};
   if (make_plan(desc, &p)) return 0;
   if (S < 1) { set_error(ODEVIT_ERR_INVALID_ARG, "S %d < 1", (int)S); return 0; }
-  size_t need = 0;
-  tape_ctx(p, nullptr, 0, &need, 6LL * S + 1);
-  return need;
+  return tape_bytes(p, 6LL * S + 1);
 }
 
 // Reverse sweep with the recorded steps frozen.  Evaluation e = 6 s + i of the replay is f(ckpt[s]) for i = 0 (k1 of step
@@ -683,12 +689,7 @@ extern "C" int odevit_solve_adaptive_bwd(const odevit_desc* desc, const odevit_w
     S = n > S ? n : S;
   }
   if (S < 1) return set_error(ODEVIT_ERR_INVALID_ARG, "no image has an accepted step");
-  if (tape) {
-    size_t need = 0;
-    tape_ctx(p, nullptr, 0, &need, 6LL * S + 1);
-    ODV_TRY(check_device_ptr(tape, "tape"));
-    ODV_TRY(check_ws(tape, tape_bytes, need));
-  }
+  if (tape) ODV_TRY(check_tape(p, tape, tape_bytes, 6LL * S + 1));
   Arena a(workspace);
   AdBwdBufs f = layout_adaptive_bwd(p, a);
   ODV_TRY(check_ws(workspace, workspace_bytes, a.off));
@@ -708,33 +709,18 @@ extern "C" int odevit_solve_adaptive_bwd(const odevit_desc* desc, const odevit_w
   // context of evaluation 6 st + i: its tape slot, else the recompute buffer (the replay's own evaluations all go to
   // ctx[0], which leaves f(ckpt[S]) there for reverse step S)
   auto ctx_of = [&](int st, int i) -> StageCtx {
-    return tape ? tape_ctx(p, tape, 6LL * st + i, nullptr, 0) : f.ctx[i];
+    return tape ? tape_ctx(p, tape, 6LL * st + i) : f.ctx[i];
   };
   auto eval_k1 = [&](int r, const StageCtx& c) -> int {   // k1 = f(ckpt[r])
     Epi e;
     e.out = f.k[0]; e.c_new = 1.f;
     return eval_forward(p, b.w, c, row(r), b.P, nullptr, b.sq, nullptr, 0, &e, s);
   };
-  // the stages k2..k6 of step st from ckpt[st] and k1 (as a round of the forward forms them).  replay: the k6
-  // evaluation's epilogue writes ckpt[st + 1]; recompute: only the contexts are needed, k6's output GEMM is skipped
+  // the stages k2..k6 of step st from ckpt[st] and k1.  replay: the k6 evaluation's epilogue writes ckpt[st + 1];
+  // recompute: only the contexts are needed
   auto stages = [&](int st, bool replay) -> int {
-    const double* dt = dt_of(st);
-    const float* y0 = row(st);
-    ODV_TRY(row_axpy(p, y0, f.k[0], (float)kBeta[0][0], dt, b.u, s));   // u2
-    for (int m = 1; m <= 5; ++m) {
-      const StageCtx c = tape ? ctx_of(st, m) : f.ctx[replay ? 0 : m];
-      if (!replay && m == 5) return eval_forward(p, b.w, c, b.u, b.P, nullptr, b.sq, nullptr, 0, nullptr, s);
-      Epi e;
-      e.y = y0; e.y_coef = 1.f;
-      e.row_dt = dt; e.rows_per_image = N;
-      e.k_store = f.k[m];
-      e.c_new = (float)kBeta[m][m];
-      for (int l = 0, slot = 0; l < m; ++l)
-        if (kBeta[m][l] != 0.0) { e.kin[slot] = f.k[l]; e.c_k[slot] = (float)kBeta[m][l]; ++slot; }
-      e.out = (m == 5) ? row(st + 1) : b.u;
-      ODV_TRY(eval_forward(p, b.w, c, b.u, b.P, nullptr, b.sq, nullptr, 0, &e, s));
-    }
-    return 0;
+    auto ctx = [&](int m) { return tape ? ctx_of(st, m) : f.ctx[replay ? 0 : m]; };
+    return dp_stages(p, b.w, ctx, b.P, b.sq, row(st), f.k, dt_of(st), b.u, replay ? row(st + 1) : nullptr, s);
   };
 
   // ---- replay: ckpt[1..S] (and the tape) ----
@@ -758,6 +744,7 @@ extern "C" int odevit_solve_adaptive_bwd(const odevit_desc* desc, const odevit_w
     e.out2 = b.dd; e.out2_scale = p.scaler; e.aux_type = p.dd_type;
     return rk_apply_rows(e, G, p.M, p.D, s);
   };
+  const Tableau& tb = kDopri5;
   auto stage_vjps = [&](int st) -> int {   // k6 .. k2 of step st; dd holds scaler * lambda_6
     const InterpCot& cot = f.cot[st & 1];
     for (int m = 5; m >= 1; --m) {
@@ -766,11 +753,11 @@ extern "C" int odevit_solve_adaptive_bwd(const odevit_desc* desc, const odevit_w
       e.aux_type = p.dd_type;
       e.row_dt = dt_of(st); e.rows_per_image = N;
       e.k_store = f.mu[m];
-      e.c_new = (float)kBeta[m - 1][t];
+      e.c_new = tb.a[m][t];
       int n = 0;
       for (int q = m + 1; q <= 5; ++q)
-        if (kBeta[q - 1][t] != 0.0) { e.kin[n] = f.mu[q]; e.c_k[n] = (float)kBeta[q - 1][t]; ++n; }
-      if (kBeta[5][t] != 0.0) { e.kin[n] = G; e.c_k[n] = (float)kBeta[5][t]; ++n; }
+        if (tb.a[q][t] != 0.f) { e.kin[n] = f.mu[q]; e.c_k[n] = tb.a[q][t]; ++n; }
+      if (tb.b[t] != 0.f) { e.kin[n] = G; e.c_k[n] = tb.b[t]; ++n; }
       // the dense output's cotangent of k[t] enters unscaled; k2 has no dense-output weight (c_mid[1] = 0)
       e.y = t == 0 ? cot.k17 : t == 1 ? G : cot.k[t - 2];
       e.y_coef = t == 1 ? 0.f : 1.f;
@@ -798,7 +785,7 @@ extern "C" int odevit_solve_adaptive_bwd(const odevit_desc* desc, const odevit_w
   ODV_TRY(seed(f.cot[S & 1].k17, 0.f, dt_of(S - 1)));   // G = 0: dd = scaler * g_k7 of step S - 1
   ODV_TRY(final_vjp(S));
   for (int st = S - 1; st >= 0; --st) {
-    ODV_TRY(seed(f.cot[st & 1].k[3], (float)kBeta[5][5], dt_of(st)));   // lambda_6
+    ODV_TRY(seed(f.cot[st & 1].k[3], tb.b[5], dt_of(st)));   // lambda_6
     if (!tape) {
       ODV_TRY(eval_k1(st, f.ctx[0]));
       ODV_TRY(stages(st, false));

@@ -759,19 +759,18 @@ bool solve_resident_supports(const Plan& p, int n_grid, bool wants_p_traj, bool 
   return solve_resident_shape_ok(p);
 }
 
-int solve_resident(const Plan& p, const WeightBufs& wb, int S, const float (*ta)[4], const float* tbv, const float* x0,
-                   const float* t_host, int n_grid, float* states, float* final_state, float* p_last, float* kbuf,
-                   cudaStream_t s) {
+int solve_resident(const Plan& p, const WeightBufs& wb, const Tableau& tb, const float* x0, const float* t_host,
+                   int n_grid, float* states, float* final_state, float* p_last, float* kbuf, cudaStream_t s) {
   ProfScope prof(KC_RESIDENT, s);
   ResArgs a;
   a.B = p.B; a.N = p.N; a.D = p.D; a.H = p.H; a.hid = p.hid;
   a.RA = (p.N + 15) / 16 * 16;
   a.NK = a.RA;
-  a.n_grid = n_grid; a.S = S; a.scaler = p.scaler;
+  a.n_grid = n_grid; a.S = tb.S; a.scaler = p.scaler;
   for (int j = 0; j + 1 < n_grid; ++j) a.dt[j] = t_host[j + 1] - t_host[j];
   for (int i = 0; i < 4; ++i) {
-    a.b[i] = tbv[i];
-    for (int j = 0; j < 4; ++j) a.a[i][j] = ta[i][j];
+    a.b[i] = tb.b[i];
+    for (int j = 0; j < 4; ++j) a.a[i][j] = tb.a[i][j];
   }
   a.x0 = x0; a.states = states; a.final_state = final_state; a.p_last = p_last;
   a.b1cat = wb.b1cat; a.b2 = wb.b2; a.kbuf = kbuf;

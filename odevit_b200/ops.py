@@ -297,6 +297,24 @@ def _row_index_tensor(row_index: Tuple[int, ...], device: torch.device) -> torch
     return t
 
 
+def _solve_grid_outputs(x0: torch.Tensor, t: torch.Tensor, spec: FieldSpec, method: str, want_p_last: bool,
+                        jas: Optional[Tuple[int, int]]):
+    """What both fixed-grid solves pass the same way: (T, the host grid as a C array, the evaluation count, p_last
+    [B,H,N,N] | None, (jas_traj [E,B,H] | None, its first evaluation, k))."""
+    B, N, _ = x0.shape
+    T = int(t.numel())
+    t_c = (ctypes.c_float * T)(*t.detach().to("cpu", torch.float32).contiguous().tolist())
+    n_evals = (T - 1) * _lib.STAGES[method]
+    p_last = (torch.empty(B, spec.heads, N, N, device=x0.device, dtype=torch.float32)
+              if (want_p_last and n_evals > 0) else None)
+    jas_traj, jas_first, jas_k = None, 0, 0
+    if jas is not None and n_evals > 0:
+        jas_first, jas_k = max(0, min(int(jas[0]), n_evals)), int(jas[1])
+        if n_evals - jas_first > 0:
+            jas_traj = torch.empty(n_evals - jas_first, B, spec.heads, device=x0.device, dtype=torch.float32)
+    return T, t_c, n_evals, p_last, (jas_traj, jas_first, jas_k)
+
+
 class _OdeSolve(torch.autograd.Function):
     """(states, final, rows, p_last, p_traj) = solve(x0).
 
@@ -314,28 +332,18 @@ class _OdeSolve(torch.autograd.Function):
                 names: Tuple[str, ...], track: bool, *weights):
         x0 = _require_cuda(x0, "x0")
         B, N, D = x0.shape
-        T = int(t_host.numel())
-        S = _lib.STAGES[method]
         desc = spec.desc(B, N)
         w, keep = _pack_weights(names, weights)
-        t_host = t_host.detach().to("cpu", torch.float32).contiguous()
-        t_c = (ctypes.c_float * T)(*t_host.tolist())
+        T, t_c, n_evals, p_last, (jas_traj, jas_first, jas_k) = _solve_grid_outputs(x0, t_host, spec, method,
+                                                                                   want_p_last, jas)
         states = torch.empty(T, B, N, D, device=x0.device, dtype=torch.float32)
         final = torch.empty(B, N, D, device=x0.device, dtype=torch.float32)
-        n_evals = (T - 1) * S
-        p_last = (torch.empty(B, spec.heads, N, N, device=x0.device, dtype=torch.float32)
-                  if (want_p_last and n_evals > 0) else None)
         p_traj = None
         first = 0
         if p_traj_first is not None and n_evals > 0:
             first = max(0, min(int(p_traj_first), n_evals))
             if n_evals - first > 0:
                 p_traj = torch.empty(n_evals - first, B, spec.heads, N, N, device=x0.device, dtype=torch.float32)
-        jas_traj, jas_first, jas_k = None, 0, 0
-        if jas is not None and n_evals > 0:
-            jas_first, jas_k = max(0, min(int(jas[0]), n_evals)), int(jas[1])
-            if n_evals - jas_first > 0:
-                jas_traj = torch.empty(n_evals - jas_first, B, spec.heads, device=x0.device, dtype=torch.float32)
         buf, ws, ws_bytes = _workspace(desc, _lib.WS_SOLVE_FWD, _lib.METHODS[method], x0.device)
         # `track`: a backward pass can follow (grad mode on and something requires grad); decided by the
         # caller, because inside forward() grad mode is always off and needs_input_grad ignores no_grad()
@@ -490,25 +498,14 @@ def ode_solve_lean(x0: torch.Tensor, t: torch.Tensor, spec: FieldSpec, method: s
     names = tuple(k for k, v in weights.items() if v is not None)
     x0 = _require_cuda(x0.detach(), "x0")
     B, N, D = x0.shape
-    T = int(t.numel())
-    S = _lib.STAGES[method]
     desc = spec.desc(B, N)
     w, keep = _pack_weights(names, [weights[k].detach() for k in names])
-    t_host = t.detach().to("cpu", torch.float32).contiguous()
-    t_c = (ctypes.c_float * T)(*t_host.tolist())
-    n_evals = (T - 1) * S
+    T, t_c, n_evals, p_last, (jas_traj, jas_first, jas_k) = _solve_grid_outputs(x0, t, spec, method, want_p_last, jasmin)
     final = torch.empty(B, N, D, device=x0.device, dtype=torch.float32)
     row_index = [int(i) for i in row_index]
     rows = torch.empty(len(row_index), B, N, D, device=x0.device, dtype=torch.float32) if row_index else None
     idx_c = (ctypes.c_int32 * max(1, len(row_index)))(*row_index)
     fd_max = torch.empty(B, N, device=x0.device, dtype=torch.float32)
-    p_last = (torch.empty(B, spec.heads, N, N, device=x0.device, dtype=torch.float32)
-              if (want_p_last and n_evals > 0) else None)
-    jas_traj, jas_first, jas_k = None, 0, 0
-    if jasmin is not None and n_evals > 0:
-        jas_first, jas_k = max(0, min(int(jasmin[0]), n_evals)), int(jasmin[1])
-        if n_evals - jas_first > 0:
-            jas_traj = torch.empty(n_evals - jas_first, B, spec.heads, device=x0.device, dtype=torch.float32)
     buf, ws, ws_bytes = _workspace(desc, _lib.WS_SOLVE_FWD, _lib.METHODS[method], x0.device)
     with torch.cuda.device(x0.device):
         st = _lib.lib().odevit_solve_fwd_lean(ctypes.byref(desc), ctypes.byref(w), _lib.METHODS[method], _ptr(x0), t_c, T,

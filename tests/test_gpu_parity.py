@@ -569,7 +569,7 @@ def test_jasmin_in_kernel_equals_exported_maps(N_img, R, B, k):
     assert torch.equal(a["states"][:2], b["states"][:2])
 
 
-@pytest.mark.parametrize("solver,prec", [("euler", "bf16"), ("rk4", "bf16"), ("euler", "fp32")])
+@pytest.mark.parametrize("solver,prec", [("euler", "bf16"), ("midpoint", "bf16"), ("rk4", "bf16"), ("euler", "fp32")])
 def test_trajectory_free_inference_equals_materialised(solver, prec):
     """Inference without `output_hidden_states` keeps no [T,B,N,D] tensor (odevit_solve_fwd_lean: ring of three states,
     finite-difference bound folded into the epilogue of each step's last GEMM, control-point rows written directly):
