@@ -693,6 +693,39 @@ Epi rk_epilogue(const Tableau& tb, int st, float dt, const float* y, float* cons
   return e;
 }
 
+Epi rk_vjp_epilogue(const Tableau& tb, int m, float dt, const double* row_dt, int rows_per_image, const float* G,
+                    float* const* mu, const float* g_t) {
+  const int t = m - 1;
+  const float h = row_dt ? 1.f : dt;
+  Epi e;
+  e.k_store = mu[m];
+  e.c_new = h * tb.a[m][t];
+  int n = 0;
+  for (int l = m + 1; l < tb.S; ++l)
+    if (tb.a[l][t] != 0.f) { e.kin[n] = mu[l]; e.c_k[n] = h * tb.a[l][t]; ++n; }
+  // The branch follows the epilogue's arithmetic, not the caller: EPI_ROWDT scales every term by the image's step
+  // except y, so y carries the unscaled g_t (or G with coefficient 0 where there is none) and G joins the kin terms.
+  // A scalar dt is folded into the coefficients and G takes the y slot.
+  if (row_dt) {
+    e.row_dt = row_dt; e.rows_per_image = rows_per_image;
+    if (tb.b[t] != 0.f) { e.kin[n] = G; e.c_k[n] = tb.b[t]; }
+    e.y = g_t ? g_t : G; e.y_coef = g_t ? 1.f : 0.f;
+  } else {
+    e.y = G; e.y_coef = dt * tb.b[t];
+  }
+  return e;
+}
+
+Epi rk_vjp_row_epilogue(const float* G, float* const* mu, int n_mu, const float* const* rows, int n_rows, float* out) {
+  Epi e;
+  e.y = G; e.y_coef = 1.f; e.c_new = 1.f;
+  int n = 0;
+  for (int m = 1; m <= n_mu; ++m) { e.kin[n] = mu[m]; e.c_k[n] = 1.f; ++n; }
+  for (int i = 0; i < n_rows; ++i) { e.kin[n] = rows[i]; e.c_k[n] = 1.f; ++n; }
+  e.out = out;
+  return e;
+}
+
 // What one forward evaluation of a fixed-grid step keeps besides its stage combine: its intermediates (a tape slot or
 // the workspace's context) and, when wanted, its attention map and JaSMin statistic.
 struct EvalOut {
@@ -856,6 +889,19 @@ int eval_vjp(const Plan& p, const WeightBufs& wb, const StageCtx& c, BwdBufs& b,
   if (!fused_colsum) ODV_TRY(colsum_accum(b.dz, p.act, R, p.M, R, b.c1, s));
   else if (!dq_colsum_done) ODV_TRY(colsum_accum(b.dz, p.act, R, p.M, D, b.c1, s));     // the dq block only
   return 0;
+}
+
+int rk_step_vjp(const Plan& p, BwdBufs& b, const Tableau& tb, float dt, const double* row_dt, const float* const* g,
+                float* const* mu, const StageCtx* ctx, long long e0, const float* g_p, bool need_c2,
+                const odevit_weight_grads* gw, Epi row_epi, cudaStream_t s) {
+  for (int m = tb.S - 1; m >= 1; --m) {
+    Epi e = rk_vjp_epilogue(tb, m, dt, row_dt, p.N, b.gy, mu, g ? g[m - 1] : nullptr);
+    e.aux_type = p.dd_type;
+    e.out2 = b.dd; e.out2_scale = p.scaler;
+    ODV_TRY(eval_vjp(p, b.w, ctx[m], b, m == tb.S - 1 ? g_p : nullptr, need_c2, gw, e0 + m, e, s));
+  }
+  row_epi.aux_type = p.dd_type;
+  return eval_vjp(p, b.w, ctx[0], b, tb.S == 1 ? g_p : nullptr, need_c2, gw, e0, row_epi, s);
 }
 
 int finish_grads(const Plan& p, const odevit_weights* w, const odevit_weight_grads* gw, const BwdBufs& b,
@@ -1294,50 +1340,20 @@ int odevit_solve_bwd(const odevit_desc* desc, const odevit_weights* w, int32_t m
     if (!tape)
       ODV_TRY(rk_step(p, b, *tb, j, dt, y, nullptr, nullptr, nullptr,
                       [&](long long, int st) { return EvalOut{b.ctx[st]}; }, s));
-    // (2) reverse through the stages
-    //     lambda_st = dt*(b[st]*G + sum_{m>st} a[m][st]*mu_m),  mu_st = J(u_st)^T lambda_st,
-    //     dL/dy = G + sum_st mu_st  (+ the cotangents injected at row j)
-    bool dd_seeded = true;
-    for (int st = S - 1; st >= 0; --st) {
-      const bool last_eval = (j == n_grid - 2 && st == S - 1);
-      Epi e;  // epilogue of the mu GEMM: v = mu_st
-      e.aux_type = p.dd_type;
-      if (st > 0) {
-        // keep mu_st; dd <- scaler * lambda_{st-1}
-        e.k_store = b.mu[st];
-        const int t = st - 1;
-        e.c_new = dt * tb->a[st][t];
-        e.y = b.gy; e.y_coef = dt * tb->b[t];
-        int n = 0;
-        for (int m = st + 1; m < S; ++m)
-          if (tb->a[m][t] != 0.f) { e.kin[n] = b.mu[m]; e.c_k[n] = dt * tb->a[m][t]; ++n; }
-        e.out = nullptr;
-        e.out2 = b.dd; e.out2_scale = p.scaler;
-      } else {
-        // G <- G + mu_0 + sum_{m>=1} mu_m + injected(j);  dd <- seed of step j-1
-        e.c_new = 1.f;
-        e.y = b.gy; e.y_coef = 1.f;
-        int n = 0;
-        for (int m = 1; m < S; ++m) { e.kin[n] = b.mu[m]; e.c_k[n] = 1.f; ++n; }
-        const float* inj[Epi::kMaxTerms];
-        const int n_inj = injected_terms(j, inj, Epi::kMaxTerms);
-        const bool fits = (n + n_inj <= Epi::kMaxTerms);
-        if (fits) for (int i = 0; i < n_inj; ++i) { e.kin[n] = inj[i]; e.c_k[n] = 1.f; ++n; }
-        e.out = b.gy;
-        if (fits && j > 0) {
-          const float dt_prev = t_grid_host[j] - t_grid_host[j - 1];
-          e.out2 = b.dd; e.out2_scale = p.scaler * dt_prev * tb->b[S - 1];
-        } else {
-          e.out2 = nullptr;
-          dd_seeded = false;
-        }
-        ODV_TRY(eval_vjp(p, b.w, ctx[st], b, last_eval ? g_p_last : nullptr, need_c2, gw, (long long)j * S + st, e, s));
-        if (!fits) ODV_TRY(inject(j));
-        if (!dd_seeded && j > 0) ODV_TRY(seed_dd(t_grid_host[j] - t_grid_host[j - 1]));
-        continue;
-      }
-      ODV_TRY(eval_vjp(p, b.w, ctx[st], b, last_eval ? g_p_last : nullptr, need_c2, gw, (long long)j * S + st, e, s));
+    // (2) reverse through the stages: G <- G + sum_st mu_st + the cotangents injected at row j, and the row epilogue
+    //     seeds dd for step j-1 -- unless the terms overflow it: then the injection and the seed follow as passes
+    const float* inj[Epi::kMaxTerms];
+    const int n_inj = injected_terms(j, inj, Epi::kMaxTerms);
+    const bool fits = (S - 1 + n_inj <= Epi::kMaxTerms);
+    Epi row = rk_vjp_row_epilogue(b.gy, b.mu, S - 1, inj, fits ? n_inj : 0, b.gy);
+    if (fits && j > 0) {
+      row.out2 = b.dd;
+      row.out2_scale = p.scaler * (t_grid_host[j] - t_grid_host[j - 1]) * tb->b[S - 1];
     }
+    ODV_TRY(rk_step_vjp(p, b, *tb, dt, nullptr, nullptr, b.mu, ctx, (long long)j * S,
+                        j == n_grid - 2 ? g_p_last : nullptr, need_c2, gw, row, s));
+    if (!fits) ODV_TRY(inject(j));
+    if (!fits && j > 0) ODV_TRY(seed_dd(t_grid_host[j] - t_grid_host[j - 1]));
   }
   ODV_CUDA(cudaMemcpyAsync(g_x0, b.gy, MD * 4, cudaMemcpyDeviceToDevice, s));
   return finish_grads(p, w, gw, b, s);

@@ -106,6 +106,14 @@ struct Tableau {
 // Epilogue of stage `st` of a step starting at y with step dt (api.cu): produces the next stage input (or the step result
 // when st == S-1) into `out`; stores k_st into k[st] when a later stage needs it.  k[l] is null where no buffer exists.
 Epi rk_epilogue(const Tableau& tb, int st, float dt, const float* y, float* const* k, float* out);
+// Its reverse (api.cu): the epilogue of stage m's mu GEMM (m >= 1) with t = m - 1,
+//   lambda_t = g_t + h (a[m][t] mu_m + sum_{l>m} a[l][t] mu_l + b[t] G),
+// keeping mu_m in mu[m]; the caller routes lambda_t (to dd).  h is the scalar dt, or with row_dt (non-null: dt unused)
+// each image's step (EPI_ROWDT).  g_t (nullable, row_dt only) is the dense output's cotangent of stage t.
+Epi rk_vjp_epilogue(const Tableau& tb, int m, float dt, const double* row_dt, int rows_per_image, const float* G,
+                    float* const* mu, const float* g_t);
+// The epilogue of stage 0's mu GEMM: out = G + mu_0 + mu_1 + ... + mu_{n_mu} + rows[0] + ... + rows[n_rows - 1].
+Epi rk_vjp_row_epilogue(const float* G, float* const* mu, int n_mu, const float* const* rows, int n_rows, float* out);
 
 // One forward field evaluation at `u` (api.cu); `rk` (nullable) is the epilogue of its last GEMM.
 int eval_forward(const Plan& p, const WeightBufs& wb, const StageCtx& c, const float* u, float* P,
@@ -135,14 +143,21 @@ int solve_resident(const Plan& p, const WeightBufs& wb, const Tableau& tb, const
 // Reverse-sweep pieces shared by odevit_solve_bwd and odevit_solve_adaptive_bwd (api.cu):
 //   layout_bwd: the fixed-grid workspace for S stages;  tape_bytes / check_tape / tape_ctx: the size of a tape of n_evals
 //   evaluations, the check of a caller's tape against it, and the context of evaluation e in it;  eval_vjp: VJP of one
-//   field evaluation, mu delivered through `mu_epi` (the EPI_RK epilogue of its last GEMM);  finish_grads: the
-//   accumulators unfolded into the caller's gradients, once per call
+//   field evaluation, mu delivered through `mu_epi` (the EPI_RK epilogue of its last GEMM);  rk_step_vjp: the reverse
+//   of one step;  finish_grads: the accumulators unfolded into the caller's gradients, once per call
 BwdBufs layout_bwd(const Plan& p, Arena& a, int S);
 size_t tape_bytes(const Plan& p, long long n_evals);
 int check_tape(const Plan& p, const void* tape, size_t bytes, long long n_evals);
 StageCtx tape_ctx(const Plan& p, const void* tape, long long e);
 int eval_vjp(const Plan& p, const WeightBufs& wb, const StageCtx& c, BwdBufs& b, const float* g_p, bool need_c2,
              const odevit_weight_grads* gw, long long ev, const Epi& mu_epi, cudaStream_t s);
+// The stage VJPs of one step, S-1 down to 0, G in b.gy: evaluation e0 + st with the intermediates ctx[st].  On entry dd
+// holds scaler * lambda_{S-1}.  Stages S-1 .. 1 combine with rk_vjp_epilogue (dt / row_dt, g[t] of g (nullable)) and
+// leave scaler * lambda_{st-1} in dd; stage 0 runs the caller's `row_epi` (rk_vjp_row_epilogue and any dd seed it
+// adds).  g_p (nullable): the attention-map cotangent of stage S-1.
+int rk_step_vjp(const Plan& p, BwdBufs& b, const Tableau& tb, float dt, const double* row_dt, const float* const* g,
+                float* const* mu, const StageCtx* ctx, long long e0, const float* g_p, bool need_c2,
+                const odevit_weight_grads* gw, Epi row_epi, cudaStream_t s);
 int finish_grads(const Plan& p, const odevit_weights* w, const odevit_weight_grads* gw, const BwdBufs& b, cudaStream_t s);
 bool wants_c2(const odevit_weight_grads* gw);
 

@@ -58,7 +58,7 @@ enum KClass : int {
   KC_BWD_GEMM_G2,  // G2 += dd^T [O|h]
   KC_BWD_ATTN,     // attention VJP products (dP, dq, dk, dv)
   KC_BWD_SOFTMAX,  // softmax VJP rows
-  KC_BWD_GEMM_DX,  // zsum = dz @ W1cat
+  KC_BWD_GEMM_DX,  // mu = dz @ centred(W1cat) (+ RK stage-combine epilogue)
   KC_BWD_GEMM_G1,  // G1 += dz^T xc
   KC_BWD_COLSUM,   // bias-gradient column sums
   KC_COMBINE,      // reverse-mode stage combine / axpy
@@ -229,12 +229,9 @@ int softmax_bwd_rows(const float* p, float* dp, const float* dpx, long long rows
 int colsum_accum(const void* X, int x_type, long long ld, int rows, int cols, float* acc,
                  cudaStream_t s);
 
-// Reverse-mode stage combine (see odevit_api.cu):  optional mu = center(zsum) stored to mu_out,
-// then  v = sum_i coef[i]*term[i]  (+ coef_mu*mu) ; writes out_f32 = v and/or out_dd = cast(dd_scale*v)
+// Reverse-mode stage combine (the seed and overflow passes of the reverse sweeps, the MACARON VJP):
+// v = sum_i coef[i]*term[i] ; writes out_f32 = v and/or out_dd = cast(dd_scale*v)
 struct CombineArgs {
-  const float* zsum = nullptr;  // raw d/d(xc) from GEMM5 (nullable)
-  float* mu_out = nullptr;      // centered zsum (nullable)
-  float coef_mu = 0.f;
   int n_terms = 0;
   const float* term[6] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
   float coef[6] = {0, 0, 0, 0, 0, 0};

@@ -5,7 +5,7 @@
 //   softmax_rows       softmax over key positions        nn.MultiheadAttention explicit path (:228)
 //   softmax_bwd_rows   its VJP (+ injected dP for the `attentions` output)
 //   colsum_accum       bias-gradient column sums
-//   vjp_combine        CenterNorm VJP + reverse-mode Runge-Kutta stage combination
+//   vjp_combine        reverse-mode Runge-Kutta stage combination
 //   fold / unfold      CenterNorm affine folded into the GEMM weights, and the chain rule back
 #include "epilogue.cuh"
 #include "internal.h"
@@ -226,31 +226,11 @@ __global__ void __launch_bounds__(256) vjp_combine_kernel(CombineArgs a, int row
   const int lane = threadIdx.x & 31;
   if (row >= rows) return;
   const long long base = (long long)row * D;
-  float mu[MAX_PER_LANE];
-  if (a.zsum) {
-    float s = 0.f;
-#pragma unroll
-    for (int i = 0; i < MAX_PER_LANE; ++i) {
-      const int c = lane + i * 32;
-      mu[i] = (c < D) ? a.zsum[base + c] : 0.f;
-      s += mu[i];
-    }
-    const float mean = warp_sum(s) / (float)D;
-#pragma unroll
-    for (int i = 0; i < MAX_PER_LANE; ++i) {
-      const int c = lane + i * 32;
-      mu[i] -= mean;
-      if (a.mu_out && c < D) a.mu_out[base + c] = mu[i];
-    }
-  } else {
-#pragma unroll
-    for (int i = 0; i < MAX_PER_LANE; ++i) mu[i] = 0.f;
-  }
 #pragma unroll
   for (int i = 0; i < MAX_PER_LANE; ++i) {
     const int c = lane + i * 32;
     if (c >= D) continue;
-    float v = a.coef_mu * mu[i];
+    float v = 0.f;
     for (int t = 0; t < a.n_terms; ++t) v = fmaf(a.coef[t], a.term[t][base + c], v);
     if (a.out_f32) a.out_f32[base + c] = v;
     if (a.out_dd) store_elem(a.out_dd, base + c, a.dd_type, a.dd_scale * v);

@@ -654,7 +654,7 @@ extern "C" size_t odevit_adaptive_tape_bytes(const odevit_desc* desc, int32_t S)
 // s, k7 of step s - 1) and k_{i+1} of step s for i = 1..5.  With G the cotangent of ckpt[s + 1] (everything downstream of
 // it), reverse step s runs
 //   lambda_6 = g_k6 + dt_b c_sol[5] G                                   (a row pass: rk_apply_rows with EPI_ROWDT)
-//   VJP of k6 .. k2: mu_m, and in the mu GEMM's EPI_RK | EPI_ROWDT epilogue
+//   VJP of k6 .. k2 (rk_step_vjp with row_dt): mu_m, and in the mu GEMM's EPI_RK | EPI_ROWDT epilogue
 //     lambda_{m-1} = g_k{m-1} + dt_b (beta[m-1][m-1] mu_m + sum_{l>m} beta[l-1][m-1] mu_l + c_sol[m-1] G)
 //   VJP of f(ckpt[s]) with lambda_1 + g_k7 of step s - 1 (the same evaluation):  G <- G + sum mu + g of row s
 // where the g_* are the dense output's cotangents (ad_interp_vjp_kernel).  Reverse step S is that last VJP alone, at each
@@ -745,45 +745,17 @@ extern "C" int odevit_solve_adaptive_bwd(const odevit_desc* desc, const odevit_w
     return rk_apply_rows(e, G, p.M, p.D, s);
   };
   const Tableau& tb = kDopri5;
-  auto stage_vjps = [&](int st) -> int {   // k6 .. k2 of step st; dd holds scaler * lambda_6
-    const InterpCot& cot = f.cot[st & 1];
-    for (int m = 5; m >= 1; --m) {
-      const int t = m - 1;   // the epilogue forms lambda of k[t]
-      Epi e;
-      e.aux_type = p.dd_type;
-      e.row_dt = dt_of(st); e.rows_per_image = N;
-      e.k_store = f.mu[m];
-      e.c_new = tb.a[m][t];
-      int n = 0;
-      for (int q = m + 1; q <= 5; ++q)
-        if (tb.a[q][t] != 0.f) { e.kin[n] = f.mu[q]; e.c_k[n] = tb.a[q][t]; ++n; }
-      if (tb.b[t] != 0.f) { e.kin[n] = G; e.c_k[n] = tb.b[t]; ++n; }
-      // the dense output's cotangent of k[t] enters unscaled; k2 has no dense-output weight (c_mid[1] = 0)
-      e.y = t == 0 ? cot.k17 : t == 1 ? G : cot.k[t - 2];
-      e.y_coef = t == 1 ? 0.f : 1.f;
-      e.out2 = b.dd; e.out2_scale = p.scaler;
-      ODV_TRY(eval_vjp(p, b.w, ctx_of(st, m), b, nullptr, need_c2, gw, 6LL * st + m, e, s));
-    }
-    return 0;
-  };
-  auto final_vjp = [&](int st) -> int {   // f(ckpt[st]): G <- G + its mu + the stage mus of step st + g of row st
-    Epi e;
-    e.aux_type = p.dd_type;
-    e.y = G; e.y_coef = 1.f; e.c_new = 1.f;
-    int n = 0;
-    if (st < S)
-      for (int m = 1; m <= 5; ++m) { e.kin[n] = f.mu[m]; e.c_k[n] = 1.f; ++n; }
-    e.kin[n] = f.cot[st & 1].y; e.c_k[n] = 1.f;
-    e.out = st == 0 ? g_x0 : G;
-    return eval_vjp(p, b.w, ctx_of(st, 0), b, nullptr, need_c2, gw, 6LL * st, e, s);
-  };
 
   ODV_CUDA(cudaMemsetAsync(G, 0, (size_t)MD * 4, s));
   ODV_CUDA(cudaMemsetAsync(f.cot[S & 1].y, 0, (size_t)MD * 4, s));
   ODV_CUDA(cudaMemsetAsync(f.cot[S & 1].k17, 0, (size_t)MD * 4, s));
   ODV_TRY(interp_vjp(S - 1));
   ODV_TRY(seed(f.cot[S & 1].k17, 0.f, dt_of(S - 1)));   // G = 0: dd = scaler * g_k7 of step S - 1
-  ODV_TRY(final_vjp(S));
+  {   // reverse step S: f(ckpt[S]) alone, G <- G + its mu + g of row S
+    Epi e = rk_vjp_row_epilogue(G, f.mu, 0, &f.cot[S & 1].y, 1, G);
+    e.aux_type = p.dd_type;
+    ODV_TRY(eval_vjp(p, b.w, ctx_of(S, 0), b, nullptr, need_c2, gw, 6LL * S, e, s));
+  }
   for (int st = S - 1; st >= 0; --st) {
     ODV_TRY(seed(f.cot[st & 1].k[3], tb.b[5], dt_of(st)));   // lambda_6
     if (!tape) {
@@ -791,8 +763,13 @@ extern "C" int odevit_solve_adaptive_bwd(const odevit_desc* desc, const odevit_w
       ODV_TRY(stages(st, false));
     }
     if (st > 0) ODV_TRY(interp_vjp(st - 1));
-    ODV_TRY(stage_vjps(st));
-    ODV_TRY(final_vjp(st));
+    // the dense output's cotangents of k1 .. k5 (k2 has no dense-output weight: c_mid[1] = 0) and of row st
+    const InterpCot& cot = f.cot[st & 1];
+    const float* g[5] = {cot.k17, nullptr, cot.k[0], cot.k[1], cot.k[2]};
+    StageCtx ctx[6];
+    for (int i = 0; i < 6; ++i) ctx[i] = ctx_of(st, i);
+    ODV_TRY(rk_step_vjp(p, b, tb, 1.f, dt_of(st), g, f.mu, ctx, 6LL * st, nullptr, need_c2, gw,
+                        rk_vjp_row_epilogue(G, f.mu, 5, &cot.y, 1, st == 0 ? g_x0 : G), s));
   }
   return finish_grads(p, w, gw, b, s);
 }
