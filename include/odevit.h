@@ -24,7 +24,8 @@
  * Conventions (SURVEY.md section 8b):
  *   - plain pointers and sizes only; no torch types; every device buffer, including the workspace,
  *     is owned by the caller; the library never allocates device memory and never synchronises
- *     (except odevit_solve_adaptive[_record], which cannot know its number of rounds in advance);
+ *     (except odevit_solve_adaptive[_record], which cannot know its number of rounds in advance;
+ *     odevit_solve_adaptive_resident decides them on the device and does not synchronise);
  *   - all work is enqueued on `stream` and is asynchronous with respect to the host;
  *   - `t_grid` is a HOST pointer (the per-step dt = t[i+1]-t[i] is formed on the host in fp32,
  *     exactly as torchdiffeq forms it);
@@ -152,7 +153,8 @@ typedef enum {
   ODEVIT_WS_SOLVE_BWD = 2, /* odevit_solve_bwd                                                 */
   ODEVIT_WS_ENCODER_FWD = 3, /* odevit_encoder_fwd (method ignored)                            */
   ODEVIT_WS_SOLVE_ADAPTIVE = 4, /* odevit_solve_adaptive[_record] (method ignored)              */
-  ODEVIT_WS_SOLVE_ADAPTIVE_BWD = 5 /* odevit_solve_adaptive_bwd (method ignored)                */
+  ODEVIT_WS_SOLVE_ADAPTIVE_BWD = 5, /* odevit_solve_adaptive_bwd (method ignored)               */
+  ODEVIT_WS_SOLVE_ADAPTIVE_RESIDENT = 6 /* odevit_solve_adaptive_resident (method ignored)      */
 } odevit_ws_kind;
 
 /* ABI / build identification. */
@@ -344,6 +346,26 @@ int odevit_solve_adaptive_bwd(const odevit_desc* desc, const odevit_weights* w, 
                               const float* g_states, float* g_x0, const odevit_weight_grads* gw, float* ckpt,
                               void* tape, size_t tape_bytes, void* workspace, size_t workspace_bytes,
                               odevit_stream_t stream);
+
+/* The per-image Dormand-Prince solve of odevit_solve_adaptive run inside the on-chip-state kernel: ONE launch, one
+ * persistent CTA per image at a time (images dealt to CTAs as they become free), the state in shared memory, the stage
+ * vectors k1..k7 in a per-CTA L2-resident scratch, every accept / reject decision taken on the chip.  Same algorithm,
+ * arguments and outputs as odevit_solve_adaptive, with a different contract:
+ *   - it never synchronises and may be captured into a CUDA graph (the step sequence is decided on the device at every
+ *     replay);
+ *   - failures are reported PER IMAGE in status [B] (device int32, required): 0 ok, 1 max_num_steps exceeded, 2
+ *     non-finite error ratio, 3 t + dt == t.  A failed image stops; its rows of `states` from the first output time it
+ *     had not passed are NaN; the other images finish normally.  Returns 0 once enqueued.
+ *   - the error ratio is summed in a different (fixed) order than odevit_solve_adaptive's, so results are not bitwise
+ *     those of the multi-kernel solve (the same bf16 tolerance applies).
+ * Envelope (ODEVIT_ERR_UNSUPPORTED outside it, no fallback): PARALLEL field, bf16, head dim 64, dim a multiple of 64 up
+ * to 192, 1..128 tokens, hidden a multiple of 128; dropout 0 (ODEVIT_ERR_INVALID_ARG); 2 <= n_out <= 129.  Row 0 of
+ * states is x0.  Workspace kind ODEVIT_WS_SOLVE_ADAPTIVE_RESIDENT. */
+int odevit_solve_adaptive_resident(const odevit_desc* desc, const odevit_weights* w, const float* x0,
+                                   const float* t_out_host, int32_t n_out, double rtol, double atol, double first_step,
+                                   int32_t max_num_steps, float* states, int32_t* nfe, int32_t* accepted,
+                                   int32_t* rejected, int32_t* status, void* workspace, size_t workspace_bytes,
+                                   odevit_stream_t stream);
 
 /* 1 when odevit_solve_fwd runs this inference solve in the on-chip-state kernel (one persistent CTA per image,
  * trajectory rows written from shared memory): the caller then has no reason to prefer the trajectory-free form. */

@@ -1069,6 +1069,8 @@ size_t odevit_workspace_bytes(const odevit_desc* desc, int32_t ws_kind, int32_t 
     a.off = solve_adaptive_workspace_bytes(p);
   } else if (ws_kind == ODEVIT_WS_SOLVE_ADAPTIVE_BWD) {
     a.off = solve_adaptive_bwd_workspace_bytes(p);
+  } else if (ws_kind == ODEVIT_WS_SOLVE_ADAPTIVE_RESIDENT) {
+    a.off = solve_adaptive_resident_workspace_bytes(p);
   } else {
     const Tableau* tb = tableau_for(method);
     if (!tb) { set_error(ODEVIT_ERR_INVALID_ARG, "unknown method %d", method); return 0; }

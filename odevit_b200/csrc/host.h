@@ -132,6 +132,8 @@ int attention_vjp(const Plan& p, const void* qkv, const void* oh, long long ld_o
                   const float* g_p, void* dz, int R, Drop drop, cudaStream_t s, float* dq_colsum = nullptr,
                   bool* colsum_done = nullptr);
 
+constexpr int kResidentMaxGrid = 129;   // grid points / output times the on-chip-state kernel carries in its arguments
+
 // On-chip-state solver for small-token shapes (solve_resident.cu): one persistent CTA per image runs
 // every step of the solve with the ODE state in shared memory.  Inference, PARALLEL field, bf16 mode.
 bool solve_resident_shape_ok(const Plan& p);
@@ -139,6 +141,14 @@ bool solve_resident_supports(const Plan& p, int n_grid, bool wants_p_traj, bool 
 size_t solve_resident_scratch_floats(const Plan& p);
 int solve_resident(const Plan& p, const WeightBufs& wb, const Tableau& tb, const float* x0, const float* t_host,
                    int n_grid, float* states, float* final_state, float* p_last, float* kbuf, cudaStream_t s);
+// Its adaptive mode (odevit_solve_adaptive_resident): per-image Dormand-Prince, one launch, no host round trip.
+// envelope: null when the shape is covered, else what is out of range.  t_out [n_out] fp64 host, 2 <= n_out <= 129;
+// next_image: one device int (the image dealer); status [B] device, never null.
+const char* solve_resident_adaptive_envelope(const Plan& p);
+size_t solve_resident_adaptive_scratch_floats(const Plan& p);
+int solve_resident_adaptive(const Plan& p, const WeightBufs& wb, const float* x0, const double* t_out, int n_out,
+                            double rtol, double atol, double first_step, int max_steps, float* states, int* nfe,
+                            int* accepted, int* rejected, int* status, float* kbuf, int* next_image, cudaStream_t s);
 
 // Reverse-sweep pieces shared by odevit_solve_bwd and odevit_solve_adaptive_bwd (api.cu):
 //   layout_bwd: the fixed-grid workspace for S stages;  tape_bytes / check_tape / tape_ctx: the size of a tape of n_evals
@@ -165,6 +175,7 @@ bool wants_c2(const odevit_weight_grads* gw);
 // ODEVIT_WS_SOLVE_ADAPTIVE_BWD)
 size_t solve_adaptive_workspace_bytes(const Plan& p);
 size_t solve_adaptive_bwd_workspace_bytes(const Plan& p);
+size_t solve_adaptive_resident_workspace_bytes(const Plan& p);   // ODEVIT_WS_SOLVE_ADAPTIVE_RESIDENT
 
 // MACARON field (field_macaron.cu)
 int macaron_forward(const Plan& p, const WeightBufs& wb, const StageCtx& c, const float* u, float* P,

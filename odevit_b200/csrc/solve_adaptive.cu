@@ -30,6 +30,7 @@
 #include <cmath>
 #include <vector>
 
+#include "dopri5.cuh"
 #include "epilogue.cuh"
 #include "host.h"
 #include "internal.h"
@@ -37,27 +38,14 @@
 namespace odevit {
 namespace {
 
-// Dormand-Prince tableau with Shampine's dense-output midpoint (torchdiffeq _impl/dopri5.py): a[m] = beta[m - 1],
-// b = c_sol[:6]
-const Tableau kDopri5 = {
-    6,
-    {{0},
-     {(float)(1. / 5)},
-     {(float)(3. / 40), (float)(9. / 40)},
-     {(float)(44. / 45), (float)(-56. / 15), (float)(32. / 9)},
-     {(float)(19372. / 6561), (float)(-25360. / 2187), (float)(64448. / 6561), (float)(-212. / 729)},
-     {(float)(9017. / 3168), (float)(-355. / 33), (float)(46732. / 5247), (float)(49. / 176), (float)(-5103. / 18656)}},
-    {(float)(35. / 384), 0.f, (float)(500. / 1113), (float)(125. / 192), (float)(-2187. / 6784), (float)(11. / 84)}};
-__constant__ float kCErr[7] = {(float)(35. / 384 - 1951. / 21600), 0.f, (float)(500. / 1113 - 22642. / 50085),
-                               (float)(125. / 192 - 451. / 720), (float)(-2187. / 6784 + 12231. / 42400),
-                               (float)(11. / 84 - 649. / 6300), (float)(-1. / 60)};
-__constant__ float kCMid[7] = {(float)(6025192743. / 30085553152. / 2), 0.f, (float)(51252292925. / 65400821598. / 2),
-                               (float)(-2691868925. / 45128329728. / 2), (float)(187940372067. / 1594534317056. / 2),
-                               (float)(-1776094331. / 19743644256. / 2), (float)(11237099. / 235043384. / 2)};
+__constant__ float kCErr[7] = {kDopri5Err[0], kDopri5Err[1], kDopri5Err[2], kDopri5Err[3],
+                               kDopri5Err[4], kDopri5Err[5], kDopri5Err[6]};
+__constant__ float kCMid[7] = {kDopri5Mid[0], kDopri5Mid[1], kDopri5Mid[2], kDopri5Mid[3],
+                               kDopri5Mid[4], kDopri5Mid[5], kDopri5Mid[6]};
 
 constexpr int kMaxOut = 4096;        // output times a workspace holds (32 KB of fp64)
 constexpr int kRedThreads = 256;     // per-image reductions: one block per image
-constexpr int kErrMax = 0, kErrNonFinite = 1, kErrUnderflow = 2, kErrRecord = 3;
+constexpr int kErrRecord = 3;
 constexpr int kNoError = 0x7fffffff;
 
 // sync words: [0], [1] active-image count of rounds with r & 1 == 0 / 1; [2] min(b * 4 + kind) over failed images
@@ -197,16 +185,9 @@ __global__ void __launch_bounds__(kRedThreads) ad_init_step_kernel(int phase, co
   if (phase == 0) {
     __syncthreads();
     const double s1 = block_sum_fixed(row1 + (long long)b * N, N, red);
-    if (threadIdx.x == 0) {
-      const double d0 = sqrt(s0 / nel), d1 = sqrt(s1 / nel);
-      h0[b] = (d0 < 1e-5 || d1 < 1e-5) ? 1e-6 : 0.01 * d0 / d1;
-      d1v[b] = d1;
-    }
+    if (threadIdx.x == 0) dp5_probe_step(s0, s1, nel, h0[b], d1v[b]);
   } else if (threadIdx.x == 0) {
-    const double hh = h0[b], d1 = d1v[b];
-    const double d2 = sqrt(s0 / nel) / hh;
-    const double h1 = (d1 <= 1e-15 && d2 <= 1e-15) ? fmax(1e-6, hh * 1e-3) : pow(0.01 / fmax(d1, d2), 1.0 / 5.0);
-    dt[b] = fmin(100.0 * hh, h1);
+    dt[b] = dp5_first_step(s0, nel, h0[b], d1v[b]);
   }
 }
 
@@ -256,8 +237,7 @@ __global__ void __launch_bounds__(kRedThreads) ad_control_kernel(
       n_rej[b] += 1;
     }
     // _optimal_step_size(dt, ratio, safety 0.9, ifactor 10, dfactor 0.2, order 5)
-    if (ratio == 0.0) dt_new = dt * 10.0;
-    else dt_new = dt * fmin(10.0, fmax(0.9 * pow(ratio, -1.0 / 5.0), ratio < 1.0 ? 1.0 : 0.2));
+    dt_new = dp5_next_step(dt, ratio);
     if (fail < 0 && on < n_out) {
       if (att >= max_steps) fail = kErrMax;
       else if (t1 + dt_new == t1) fail = kErrUnderflow;
@@ -298,16 +278,8 @@ __global__ void __launch_bounds__(256) ad_commit_kernel(float* y0, const float* 
       m = fmaf(kCMid[4], k5[i], m);
       m = fmaf(kCMid[5], k6[i], m);
       m = fmaf(kCMid[6], f1, m);
-      const float ym = fmaf(dt, m, a0);
-      const float ca = 2.f * dt * (f1 - f0) - 8.f * (a1 + a0) + 16.f * ym;
-      const float cb = dt * (5.f * f0 - 3.f * f1) + 18.f * a0 + 14.f * a1 - 32.f * ym;
-      const float cc = dt * (f1 - 4.f * f0) - 11.f * a0 - 5.f * a1 + 16.f * ym;
-      const float cd = dt * f0;
-      for (int j = lo; j < hi; ++j) {
-        const float x = (float)((t_out[j] - t0) / dtd);
-        const float x2 = x * x, x3 = x2 * x, x4 = x3 * x;
-        states[(long long)j * MD + i] = a0 + x * cd + x2 * cc + x3 * cb + x4 * ca;
-      }
+      const Dp5Quartic qa(a0, a1, f0, f1, m, dt);
+      for (int j = lo; j < hi; ++j) states[(long long)j * MD + i] = qa.at((float)((t_out[j] - t0) / dtd));
     }
     y0[i] = a1;
     k1[i] = f1;
@@ -641,6 +613,64 @@ extern "C" int odevit_solve_adaptive_record(const odevit_desc* desc, const odevi
   rec.t0 = step_t0; rec.dt = step_dt; rec.out = step_out; rec.cap = step_cap;
   return solve_adaptive_impl(desc, w, x0, t_out_host, n_out, rtol, atol, first_step, max_num_steps, states, nfe,
                              accepted, rejected, rec, workspace, workspace_bytes, stream);
+}
+
+namespace {
+struct AdResBufs {
+  WeightBufs w;
+  float* kbuf;
+  int* next_image;
+};
+AdResBufs layout_adaptive_resident(const Plan& p, Arena& a) {
+  AdResBufs f;
+  f.w = take_weights(p, a);
+  f.kbuf = a.f32(solve_resident_adaptive_scratch_floats(p));
+  f.next_image = reinterpret_cast<int*>(a.take(16));
+  return f;
+}
+}  // namespace
+
+size_t odevit::solve_adaptive_resident_workspace_bytes(const Plan& p) {
+  Arena a(nullptr);
+  layout_adaptive_resident(p, a);
+  return a.off;
+}
+
+extern "C" int odevit_solve_adaptive_resident(const odevit_desc* desc, const odevit_weights* w, const float* x0,
+                                              const float* t_out_host, int32_t n_out, double rtol, double atol,
+                                              double first_step, int32_t max_num_steps, float* states, int32_t* nfe,
+                                              int32_t* accepted, int32_t* rejected, int32_t* status, void* workspace,
+                                              size_t workspace_bytes, odevit_stream_t stream) {
+  Plan p{};
+  ODV_TRY(make_plan(desc, &p));
+  ODV_TRY(check_weights(p, w));
+  if (p.any_drop) return set_error(ODEVIT_ERR_INVALID_ARG, "the adaptive solve is inference-only: dropout must be 0");
+  if (const char* why = solve_resident_adaptive_envelope(p))
+    return set_error(ODEVIT_ERR_UNSUPPORTED, "the on-chip adaptive solve covers this shape only with %s", why);
+  ODV_TRY(check_device_ptr(x0, "x0"));
+  ODV_TRY(check_device_ptr(states, "states"));
+  if (!status) return set_error(ODEVIT_ERR_INVALID_ARG, "status is NULL");
+  ODV_TRY(check_device_ptr(status, "status"));
+  if (nfe) ODV_TRY(check_device_ptr(nfe, "nfe"));
+  if (accepted) ODV_TRY(check_device_ptr(accepted, "accepted"));
+  if (rejected) ODV_TRY(check_device_ptr(rejected, "rejected"));
+  std::vector<double> t_out;
+  if (n_out > kResidentMaxGrid)
+    return set_error(ODEVIT_ERR_INVALID_ARG, "t_out must hold 2..%d host values on the chip, got %d", kResidentMaxGrid,
+                     (int)n_out);
+  ODV_TRY(read_t_out(t_out_host, n_out, t_out));
+  if (!(rtol >= 0.0 && atol >= 0.0 && rtol + atol > 0.0 && std::isfinite(rtol) && std::isfinite(atol)))
+    return set_error(ODEVIT_ERR_INVALID_ARG, "rtol %g / atol %g: both >= 0, finite, not both 0", rtol, atol);
+  if (!std::isfinite(first_step)) return set_error(ODEVIT_ERR_INVALID_ARG, "first_step is not finite");
+  if (max_num_steps < 1) return set_error(ODEVIT_ERR_INVALID_ARG, "max_num_steps %d < 1", (int)max_num_steps);
+  Arena a(workspace);
+  AdResBufs f = layout_adaptive_resident(p, a);
+  ODV_TRY(check_ws(workspace, workspace_bytes, a.off));
+  cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
+  ODV_TRY(prepare_weights(p, w, f.w, s));
+  ODV_CUDA(cudaMemcpyAsync(states, x0, (size_t)p.M * p.D * 4, cudaMemcpyDeviceToDevice, s));
+  return solve_resident_adaptive(p, f.w, x0, t_out.data(), n_out, rtol, atol, first_step > 0 ? first_step : 0.0,
+                                 max_num_steps, states, nfe, accepted, rejected, status, f.kbuf, f.next_image, s);
 }
 
 extern "C" size_t odevit_adaptive_tape_bytes(const odevit_desc* desc, int32_t S) {

@@ -35,8 +35,11 @@
 #include <cuda.h>
 #include <cuda_fp16.h>
 
+#include <cstddef>
 #include <cstdlib>
+#include <type_traits>
 
+#include "dopri5.cuh"
 #include "epilogue.cuh"
 #include "host.h"
 #include "ptx.cuh"
@@ -66,7 +69,7 @@ __host__ __device__ constexpr int res_producer(bool full) { return full ? 16 : 3
 __host__ __device__ constexpr int res_loader(bool full) { return full ? 17 : 7; }
 constexpr int NU = 10;                               // weight-ring slots of 8 KB
 constexpr int T_R0 = 0, T_O = 128, T_R1 = 192;
-constexpr int kMaxGrid = 129;                        // grid points carried in the kernel parameters
+constexpr int kMaxGrid = kResidentMaxGrid;           // grid points carried in the kernel parameters
 constexpr int kMaxJobs = 64, kMaxAllocs = 112;
 constexpr int NB = 8;                                // barrier pairs of the weight ring (>= allocations in flight)
 
@@ -110,11 +113,42 @@ struct ResArgs {
   Sched sc;
 };
 
+// The adaptive mode's arguments (odevit_solve_adaptive_resident): the output times and the Dormand-Prince tableau take
+// the place of the fixed grid's step sizes and Butcher tableau.
+struct ResArgsAd {
+  int B, N, RA, NK, D, H, hid;
+  int n_out, max_steps;
+  float scaler, rtol, atol;
+  double first_step;     // <= 0: selected per image (one probe evaluation)
+  float a[6][6], b[6], c_err[7], c_mid[7];
+  const float* x0;       // [B, N, D]
+  float* states;         // [n_out, B, N, D] (row 0 written by the host wrapper)
+  const float* b1cat;
+  const float* b2;
+  float* kbuf;           // [grid][8][D][RA] fp32 scratch: k1..k7 (k1 and k7 swap slots 0 and 6) and y1 (slot 7)
+  int* next_image;       // the image dealer (zeroed by the host wrapper)
+  int *nfe, *accepted, *rejected, *status;   // [B] or null (status: never null)
+  Sched sc;
+  // Last, and not copied to shared memory (1 KB the C10 shape does not have there): read from the parameter space,
+  // only when a step is accepted
+  double t_out[kMaxGrid];
+};
+// bytes of the arguments the kernel copies to shared memory
+template <class Args> __host__ __device__ constexpr int res_smem_args() { return (int)sizeof(Args); }
+template <> __host__ __device__ constexpr int res_smem_args<ResArgsAd>() { return (int)offsetof(ResArgsAd, t_out); }
+__device__ __forceinline__ int res_stages(const ResArgs& a) { return a.S; }
+__device__ __forceinline__ int res_stages(const ResArgsAd&) { return 1; }
+__device__ __forceinline__ int res_evals(const ResArgs& a) { return (a.n_grid - 1) * a.S; }
+__device__ __forceinline__ int res_evals(const ResArgsAd&) { return 0; }
+// What the compute warps announce with the last compute phase of an evaluation (adaptive mode): the image steps on, its
+// solve is over and the next image's initial phase follows, or the CTA has no image left
+enum : int { CTL_RUN = 0, CTL_NEXT = 1, CTL_DONE = 2 };
+
 struct Smem {
   int xc_atom;           // bytes of one 64-column atom of RA rows
   int off_xc, off_q, off_k, off_v, off_g, off_ring, off_y, off_b1, off_b2, off_ex, off_args, off_bars, total;
 };
-__host__ __device__ inline Smem smem_layout(int RA, int N, int D, int hid) {
+__host__ __device__ inline Smem smem_layout(int RA, int N, int D, int hid, int args_bytes = (int)sizeof(ResArgs)) {
   Smem s;
   s.xc_atom = RA * 128;
   int o = 0;
@@ -130,7 +164,7 @@ __host__ __device__ inline Smem smem_layout(int RA, int N, int D, int hid) {
   s.off_b1 = o; o += (3 * D + hid) * 4;
   s.off_b2 = o; o += D * 4;
   s.off_ex = o; o += 2 * 4 * 128 * 4;   // row-reduction exchange: [max or mean | sum][column share][row]
-  s.off_args = o; o += (int)((sizeof(ResArgs) + 15) / 16 * 16);   // the kernel arguments (see the kernel's first lines)
+  s.off_args = o; o += (args_bytes + 15) / 16 * 16;   // the kernel arguments (see the kernel's first lines)
   s.off_bars = o; o += 256;
   s.total = o;
   return s;
@@ -223,16 +257,17 @@ __device__ int rtr_n[2];
 #define RTR(cls, slot) do { } while (0)
 #endif
 
-template <bool FULL>
+template <bool FULL, bool ADAPTIVE>
 __global__ void __launch_bounds__(res_threads(FULL), 1)
 solve_resident_kernel(const __grid_constant__ CUtensorMap tmW1, const __grid_constant__ CUtensorMap tmW2,
-                      const __grid_constant__ ResArgs a_param) {
+                      const __grid_constant__ std::conditional_t<ADAPTIVE, ResArgsAd, ResArgs> a_param) {
+  using Args = std::conditional_t<ADAPTIVE, ResArgsAd, ResArgs>;
   extern __shared__ __align__(1024) uint8_t smem[];
-  const Smem L = smem_layout(a_param.RA, a_param.N, a_param.D, a_param.hid);
+  const Smem L = smem_layout(a_param.RA, a_param.N, a_param.D, a_param.hid, res_smem_args<Args>());
   // The arguments are read from a shared-memory copy: the job list, step sizes and tableau are indexed
   // dynamically all through the solve, and the constant cache does not hold them next to the instruction
   // stream's own constants (measured: ~2000 cycles per 150-instruction loop iteration with LDC in it).
-  const ResArgs& a = *reinterpret_cast<const ResArgs*>(smem + L.off_args);
+  const Args& a = *reinterpret_cast<const Args*>(smem + L.off_args);
   uint8_t* sXC = smem + L.off_xc;
   uint8_t* sQ = smem + L.off_q;
   uint8_t* sK = smem + L.off_k;
@@ -249,6 +284,9 @@ solve_resident_kernel(const __grid_constant__ CUtensorMap tmW1, const __grid_con
   uint64_t* bar_mma = bars + 2 * NB;      // [2] the MMA group of job (parity of the job counter) has retired
   uint64_t* bar_cmp = bars + 2 * NB + 2;  // [2] the compute phase (parity of the phase counter) is finished
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 2 * NB + 4);
+  // adaptive mode: [0] CTL_* of the last compute phase, [1] the image just dealt, [2] 1 once the CTA has no image left
+  // (the loader stops), [3] weight allocations the producer consumed (teardown)
+  volatile int* ctl = reinterpret_cast<volatile int*>(bars + 2 * NB + 6);
 
   constexpr int RES_THREADS = res_threads(FULL), PRODUCER = res_producer(FULL), LOADER = res_loader(FULL);
   const int warp = threadIdx.x >> 5;
@@ -260,7 +298,7 @@ solve_resident_kernel(const __grid_constant__ CUtensorMap tmW1, const __grid_con
   const int D = a_param.D, H = a_param.H, N = a_param.N, NK = a_param.NK;
   const int T_HB = T_R1 + D;
   const int nJ = a_param.sc.n_jobs;
-  const int n_evals = (a_param.n_grid - 1) * a_param.S;
+  const int n_evals = res_evals(a_param);
   const int n_mine = (a_param.B - (int)blockIdx.x + (int)gridDim.x - 1) / (int)gridDim.x;
   const int n_quads = (N + 31) >> 5;           // token-row quadrants that hold rows
 
@@ -268,12 +306,13 @@ solve_resident_kernel(const __grid_constant__ CUtensorMap tmW1, const __grid_con
     for (int i = 0; i < NB; ++i) { ptx::mbar_init(bar_full + i, 1); ptx::mbar_init(bar_free + i, 1); }
     for (int i = 0; i < 2; ++i) { ptx::mbar_init(bar_mma + i, 1); ptx::mbar_init(bar_cmp + i, n_quads * 128); }
     ptx::fence_barrier_init();
+    if constexpr (ADAPTIVE) ctl[2] = 0;
   }
   if (warp == PRODUCER) ptx::tmem_alloc(tmem_slot, 512);
   // biases -> shared memory; operand tiles zeroed once (rows [N, RA) stay zero: a thread only writes its own row)
   for (int i = threadIdx.x; i < 3 * D + a_param.hid; i += RES_THREADS) sB1[i] = a_param.b1cat[i];
   for (int i = threadIdx.x; i < D; i += RES_THREADS) sB2[i] = a_param.b2[i];
-  for (int i = threadIdx.x; i < (int)(sizeof(ResArgs) / 4); i += RES_THREADS)
+  for (int i = threadIdx.x; i < res_smem_args<Args>() / 4; i += RES_THREADS)
     reinterpret_cast<uint32_t*>(smem + L.off_args)[i] = reinterpret_cast<const uint32_t*>(&a_param)[i];
   for (int i = threadIdx.x; i < L.off_ring / 16; i += RES_THREADS) reinterpret_cast<uint4*>(smem)[i] = make_uint4(0u, 0u, 0u, 0u);
   ptx::fence_async_shared();
@@ -282,6 +321,7 @@ solve_resident_kernel(const __grid_constant__ CUtensorMap tmW1, const __grid_con
   ptx::tc_fence_after();
   const uint32_t tmem = *tmem_slot;
 
+  uint32_t ld_issued = 0;                   // adaptive mode: weight allocations the loader issued
   if (warp == PRODUCER) {
     // ======================= producer: weight units + every MMA =======================
     // The ring moves UNITS: one [64 x 64] bf16 box (8 KB).  A tile of the job list is D/64 consecutive units
@@ -342,7 +382,56 @@ solve_resident_kernel(const __grid_constant__ CUtensorMap tmW1, const __grid_con
       r1_acc = 1u;
     };
 
-    for (int idx = 0; idx < n_mine; ++idx) {
+    // the MMA group of one job, committed to bar_mma
+    auto issue = [&](int kind, int arg) {
+      if (kind == JOB_QKV) {
+        if (arg > 0) mma_into_out(q_lo);                         // O of the previous head (in the q tile)
+        mma_xc(tmem + T_R0, id_qkv);
+      } else if (kind == JOB_S) {
+        const uint64_t da = DESC0 + q_lo, db = DESC0 + k_lo;
+#pragma unroll
+        for (int kk = 0; kk < 4; ++kk) ptx::mma_ss_pred(tmem + T_R0, da + 2 * kk, db + 2 * kk, id_s, kk > 0 ? 1u : 0u, lead);
+      } else if (kind == JOB_PV) {
+        for (int ks = 0; ks < NK / 16; ++ks)
+          ptx::mma_ts_pred(tmem + T_O, tmem + T_R0 + ks * 8, ptx::smem_desc_sw128(v_addr + ks * 2048, 8192, 1024), id_pv,
+                      ks > 0 ? 1u : 0u, lead);
+      } else if (kind == JOB_FC) {
+        if (arg > 0)
+          for (int m = 0; m < 2; ++m) mma_into_out(g_lo + m * atom_lo);      // fc2 of the previous chunk
+        mma_xc(tmem + T_HB, id_fc1);
+      } else {  // JOB_F
+        mma_into_out(q_lo);                                      // O of the last head
+        for (int m = 0; m < 2; ++m) mma_into_out(g_lo + m * atom_lo);
+      }
+      ptx::commit_pred(ptx::smem_u32(bar_mma + (int)(gm & 1)), lead);
+      ++gm;
+    };
+
+    if constexpr (ADAPTIVE) {
+      // The number of evaluations is decided on the chip: the compute warps announce with each F phase whether the
+      // image steps on, the next image's initial phase follows, or the CTA is done (ctl[0]).  The next evaluation's
+      // first job waits for that phase anyway (dep < 0), so reading the word there costs nothing.
+      uint32_t P = 0;                         // phase that formed the current evaluation's stage input
+      need(P);
+      if (ctl[0] != CTL_DONE) {
+        for (;;) {
+          r1_acc = 0u;
+#pragma unroll 1
+          for (int j = 0; j < nJ; ++j) {
+            const int dep = a.sc.dep[j];
+            need(dep < 0 ? P : P + 1 + (uint32_t)dep);
+            issue(a.sc.kind[j], a.sc.arg[j]);
+          }
+          P += nJ;
+          need(P);
+          const int f = ctl[0];
+          if (f == CTL_DONE) break;
+          if (f == CTL_NEXT) ++P;             // the next image's initial phase
+        }
+      }
+      ctl[3] = (int)cg;
+    }
+    for (int idx = 0; idx < n_mine && !ADAPTIVE; ++idx) {
       const uint32_t base = (uint32_t)idx * (1u + (uint32_t)n_evals * nJ);   // phase of the image's initial xc
       for (int ev = 0; ev < n_evals; ++ev) {
         r1_acc = 0u;
@@ -355,27 +444,7 @@ solve_resident_kernel(const __grid_constant__ CUtensorMap tmW1, const __grid_con
           RTR(1, j * 4 + 0);
           need(dep < 0 ? base + (uint32_t)ev * nJ : base + 1 + (uint32_t)ev * nJ + dep);
           RTR(1, j * 4 + 1);
-          if (kind == JOB_QKV) {
-            if (arg > 0) mma_into_out(q_lo);                         // O of the previous head (in the q tile)
-            mma_xc(tmem + T_R0, id_qkv);
-          } else if (kind == JOB_S) {
-            const uint64_t da = DESC0 + q_lo, db = DESC0 + k_lo;
-#pragma unroll
-            for (int kk = 0; kk < 4; ++kk) ptx::mma_ss_pred(tmem + T_R0, da + 2 * kk, db + 2 * kk, id_s, kk > 0 ? 1u : 0u, lead);
-          } else if (kind == JOB_PV) {
-            for (int ks = 0; ks < NK / 16; ++ks)
-              ptx::mma_ts_pred(tmem + T_O, tmem + T_R0 + ks * 8, ptx::smem_desc_sw128(v_addr + ks * 2048, 8192, 1024), id_pv,
-                          ks > 0 ? 1u : 0u, lead);
-          } else if (kind == JOB_FC) {
-            if (arg > 0)
-              for (int m = 0; m < 2; ++m) mma_into_out(g_lo + m * atom_lo);      // fc2 of the previous chunk
-            mma_xc(tmem + T_HB, id_fc1);
-          } else {  // JOB_F
-            mma_into_out(q_lo);                                      // O of the last head
-            for (int m = 0; m < 2; ++m) mma_into_out(g_lo + m * atom_lo);
-          }
-          ptx::commit_pred(ptx::smem_u32(bar_mma + (int)(gm & 1)), lead);
-          ++gm;
+          issue(kind, arg);
           RTR(1, j * 4 + 2);
         }
       }
@@ -387,13 +456,28 @@ solve_resident_kernel(const __grid_constant__ CUtensorMap tmW1, const __grid_con
     const bool leader = ptx::elect_one();
     if (leader) { ptx::prefetch_tensormap(&tmW1); ptx::prefetch_tensormap(&tmW2); }
     const int n_allocs = a.sc.n_allocs;
-    const uint32_t total = (uint32_t)n_mine * n_evals * n_allocs;
+    const uint32_t total = ADAPTIVE ? 0xffffffffu : (uint32_t)n_mine * n_evals * n_allocs;
     int li = 0;
-    for (uint32_t g = 0; g < total; ++g) {
+    uint32_t g = 0;
+    // adaptive mode: the allocation cycle is the same whatever the evaluation boundaries are, so the loader streams it
+    // until the CTA has no image left; the waits of the allocations nobody will consume end on that flag
+    int lead_lane = 0;
+    if constexpr (ADAPTIVE) lead_lane = __ffs(__ballot_sync(0xffffffffu, leader)) - 1;
+    for (; g < total; ++g) {
       const Alloc al = a.sc.alloc[li];
       if (g >= al.back) {   // the allocation whose slots / barrier pair this one reuses has been released
         const uint32_t w = g - al.back;
-        ptx::mbar_wait(bar_free + (w & (NB - 1)), (w / NB) & 1);
+        if constexpr (ADAPTIVE) {
+          int st = 0;   // the leader's view, for the whole warp: 1 released, 2 the CTA is done
+          for (uint32_t spins = 0; st == 0;) {
+            st = ptx::mbar_try_wait(bar_free + (w & (NB - 1)), (w / NB) & 1) ? 1 : (ctl[2] ? 2 : 0);
+            st = __shfl_sync(0xffffffffu, st, lead_lane);
+            if (++spins > (1u << 24)) __trap();
+          }
+          if (st == 2) break;
+        } else {
+          ptx::mbar_wait(bar_free + (w & (NB - 1)), (w / NB) & 1);
+        }
       }
       if (leader) {
         uint64_t* fb = bar_full + (g & (NB - 1));
@@ -410,6 +494,7 @@ solve_resident_kernel(const __grid_constant__ CUtensorMap tmW1, const __grid_con
       __syncwarp();
       if (++li == n_allocs) li = 0;
     }
+    ld_issued = g;
   } else if (warp < 16 && (warp & 3) < n_quads) {
     // ======================= compute warps: thread = (token row, column quarter) =======================
     const int q = warp & 3, cw = warp >> 2;
@@ -429,7 +514,7 @@ solve_resident_kernel(const __grid_constant__ CUtensorMap tmW1, const __grid_con
       ++gc;
     };
     float* yrow = sY + (size_t)(row_ok ? r : 0) * (D + 4);   // row stride D+4 floats: conflict-free 16-byte accesses
-    float* kb = a_param.kbuf + (size_t)blockIdx.x * 3 * D * 128;
+    float* kb = a_param.kbuf + (size_t)blockIdx.x * (ADAPTIVE ? 8 * D * a_param.RA : 3 * D * 128);
     float* ex_max = sEx;          // softmax row max; between evaluations the CenterNorm row sums
     float* ex_sum = sEx + 512;
     float* ex_mean = sEx;
@@ -459,8 +544,76 @@ solve_resident_kernel(const __grid_constant__ CUtensorMap tmW1, const __grid_con
       }
     };
 
-    for (int idx = 0; idx < n_mine; ++idx) {
-      const int img = (int)blockIdx.x + idx * (int)gridDim.x;
+    // ---- adaptive mode ----
+    // CTA-wide sums over the compute warps in a fixed order (rows, then warps): accept / reject never varies between runs
+    auto cta_sum = [&](double& s0, double& s1) {
+#pragma unroll
+      for (int o = 16; o > 0; o >>= 1) {
+        s0 += __shfl_xor_sync(0xffffffffu, s0, o);
+        s1 += __shfl_xor_sync(0xffffffffu, s1, o);
+      }
+      double* red = reinterpret_cast<double*>(ex_sum);   // the softmax sums are dead until the next S phase
+      if ((threadIdx.x & 31) == 0) { red[2 * warp] = s0; red[2 * warp + 1] = s1; }
+      asm volatile("bar.sync 5, %0;" ::"r"(n_quads * 128) : "memory");
+      s0 = 0.0; s1 = 0.0;
+      for (int w = 0; w < 16; ++w)
+        if ((w & 3) < n_quads) { s0 += red[2 * w]; s1 += red[2 * w + 1]; }
+    };
+    // the next image for this CTA (>= B: none left): images cost different numbers of steps, so they are dealt as CTAs
+    // become free, and an image's result does not depend on which CTA runs it
+    auto fetch = [&](const auto& ap) -> int {
+      if (threadIdx.x == 0) ctl[1] = atomicAdd(ap.next_image, 1);
+      asm volatile("bar.sync 5, %0;" ::"r"(n_quads * 128) : "memory");
+      return ctl[1];
+    };
+    int img = 0;
+    // the image's controller, the same in every compute thread (each forms it from the same CTA-wide sums).  stage s
+    // evaluates k_{s+1} (s = 0..6) or the initial-step probe (kProbe); k1 and k7 swap slots 0 and 6 on accept (FSAL)
+    constexpr int kProbe = 7;
+    double t = 0.0, dt = 0.0, h0 = 0.0, d1 = 0.0;
+    int on = 1, att = 0, n_acc = 0, n_rej = 0, stage = 0, k1s = 0, nfe_base = 1;
+    bool stepping = false;
+    auto kslot = [&](int l) { return l == 0 ? k1s : (l == 6 ? 6 - k1s : l); };
+    auto kld = [&](int l, int col) { return kb[((size_t)kslot(l) * D + col) * a_param.RA + r]; };
+    // u2 = y0 + dt a21 k1 -> R1: the first stage input of an attempt; returns the partial row sum
+    auto form_u2 = [&]() -> float {
+      float part = 0.f;
+#pragma unroll 1
+      for (int g = 0; g < ngq; ++g) {
+        const int col0 = cw * DQ + g * 16;
+        float v[16];
+        lds16(yrow + col0, v);
+        const float dtf = (float)dt;
+#pragma unroll
+        for (int jj = 0; jj < 16; ++jj) {
+          const float k1 = row_ok ? kld(0, col0 + jj) : 0.f;
+          v[jj] = fmaf(dtf, a.a[1][0] * k1, v[jj]);
+          part += v[jj];
+        }
+        tmem_st16f(t_lane + T_R1 + col0, v);
+      }
+      return part;
+    };
+    if constexpr (ADAPTIVE) {
+      img = fetch(a_param);
+      if (img >= a_param.B) {   // nothing for this CTA: release the producer and the loader
+        if (threadIdx.x == 0) { ctl[0] = CTL_DONE; ctl[2] = 1; }
+        done();
+      } else if (threadIdx.x == 0) {
+        ctl[0] = CTL_RUN;
+      }
+    }
+
+    for (int idx = 0; ADAPTIVE ? img < a_param.B : idx < n_mine; ++idx) {
+      if constexpr (ADAPTIVE) {
+        t = a_param.t_out[0];
+        dt = a.first_step > 0 ? a.first_step : 0.0;
+        nfe_base = a.first_step > 0 ? 1 : 2;
+        on = 1; att = 0; n_acc = 0; n_rej = 0; stage = 0; k1s = 0;
+        stepping = true;
+      } else {
+        img = (int)blockIdx.x + idx * (int)gridDim.x;
+      }
       // ---- x0 -> resident state, first xc ----
       {
         if (cw == 0) bulk_wait_read();   // the previous image's last row stores have read the state
@@ -487,8 +640,8 @@ solve_resident_kernel(const __grid_constant__ CUtensorMap tmW1, const __grid_con
         centre_from_r1(part);
         done();
       }
-      for (int ev = 0; ev < n_evals; ++ev) {
-        const int step = ev / a.S, st = ev - step * a.S;
+      for (int ev = 0; ADAPTIVE ? stepping : ev < n_evals; ++ev) {
+        const int step = ev / res_stages(a), st = ev - step * res_stages(a);
         const bool last_eval = (ev == n_evals - 1);
 #ifdef RES_TRACE
         rtr_on = (blockIdx.x == 0 && idx == 0 && ev == 1 && threadIdx.x == 0);
@@ -578,17 +731,19 @@ solve_resident_kernel(const __grid_constant__ CUtensorMap tmW1, const __grid_con
             ex_sum[cw * 128 + r] = sum;
             quad_sync(q);
             inv_sum = 1.f / ((ex_sum[r] + ex_sum[128 + r]) + (ex_sum[256 + r] + ex_sum[384 + r]));
-            if (last_eval && a_param.p_last && row_ok) {
-              float* p_row = a_param.p_last + (((size_t)img * H + arg) * N + r) * N;
+            if constexpr (!ADAPTIVE) {
+              if (last_eval && a_param.p_last && row_ok) {
+                float* p_row = a_param.p_last + (((size_t)img * H + arg) * N + r) * N;
 #pragma unroll
-              for (int i = 0; i < 4; ++i)
-                if (cw + 4 * i < ng) {
+                for (int i = 0; i < 4; ++i)
+                  if (cw + 4 * i < ng) {
 #pragma unroll
-                  for (int jj = 0; jj < 8; ++jj) {
-                    const int col = (cw + 4 * i) * 8 + jj;
-                    if (col < N) p_row[col] = v[i][jj] * inv_sum;
+                    for (int jj = 0; jj < 8; ++jj) {
+                      const int col = (cw + 4 * i) * 8 + jj;
+                      if (col < N) p_row[col] = v[i][jj] * inv_sum;
+                    }
                   }
-                }
+              }
             }
             ptx::tmem_st_wait();
           } else if (kind == JOB_PV) {
@@ -601,6 +756,188 @@ solve_resident_kernel(const __grid_constant__ CUtensorMap tmW1, const __grid_con
             if (row_ok) {
               st_tile8(sQ, L.xc_atom, r, cw * 16, v);
               st_tile8(sQ, L.xc_atom, r, cw * 16 + 8, v + 8);
+            }
+          } else if constexpr (ADAPTIVE) {
+            // ---- k = scaler (OUT + b2) kept in the scratch; a stage combine, or norm partials -> the step decision ----
+            const double nel = (double)N * D;
+            const bool combine = (stage >= 1 && stage <= 5) || (stage == 0 && a.first_step > 0);
+            const float* coef = stage == 5 ? a.b : a.a[stage + 1 < 6 ? stage + 1 : 0];
+            const float dtf = (float)dt;
+            float part = 0.f;
+            double s0 = 0.0, s1 = 0.0;
+#pragma unroll 1
+            for (int g = 0; g < ngq; ++g) {
+              const int col0 = cw * DQ + g * 16;
+              float v[16];
+              ptx::tmem_ld16(t_lane + T_R1 + col0, v);
+              float bv[16];
+              lds16(sB2 + col0, bv);
+              float yv[16];
+              lds16(yrow + col0, yv);
+              ptx::tmem_ld_wait();
+#pragma unroll
+              for (int jj = 0; jj < 16; ++jj) v[jj] = a.scaler * (v[jj] + bv[jj]);
+              if (stage != kProbe && row_ok) {
+#pragma unroll
+                for (int jj = 0; jj < 16; ++jj) kb[((size_t)kslot(stage) * D + col0 + jj) * a_param.RA + r] = v[jj];
+              }
+              if (combine) {   // u_{s+2} = y0 + dt sum_l a[s+1][l] k_l  (after k6: y1 with b = c_sol, kept in slot 7)
+                float acc[16];
+#pragma unroll
+                for (int jj = 0; jj < 16; ++jj) acc[jj] = coef[stage] * v[jj];
+#pragma unroll 1
+                for (int l = 0; l < stage; ++l) {
+                  const float cl = coef[l];
+                  if (cl != 0.f && row_ok) {
+#pragma unroll
+                    for (int jj = 0; jj < 16; ++jj) acc[jj] = fmaf(cl, kld(l, col0 + jj), acc[jj]);
+                  }
+                }
+#pragma unroll
+                for (int jj = 0; jj < 16; ++jj) {
+                  v[jj] = fmaf(dtf, acc[jj], yv[jj]);
+                  part += v[jj];
+                }
+                if (stage == 5 && row_ok) {
+#pragma unroll
+                  for (int jj = 0; jj < 16; ++jj) kb[((size_t)7 * D + col0 + jj) * a_param.RA + r] = v[jj];
+                }
+                tmem_st16f(t_lane + T_R1 + col0, v);
+              } else if (row_ok) {
+#pragma unroll
+                for (int jj = 0; jj < 16; ++jj) {
+                  const float sc = a.atol + fabsf(yv[jj]) * a.rtol;
+                  if (stage == 0) {            // initial-step selection: |y0 / sc|^2, |f0 / sc|^2
+                    const float q0 = yv[jj] / sc, q1 = v[jj] / sc;
+                    s0 += (double)(q0 * q0);
+                    s1 += (double)(q1 * q1);
+                  } else if (stage == kProbe) {   // |(f1 - f0) / sc|^2
+                    const float q = (v[jj] - kld(0, col0 + jj)) / sc;
+                    s0 += (double)(q * q);
+                  } else {                     // |err / tol|^2, err = dt sum_l c_err[l] k_l, k7 = v
+                    float e = a.c_err[0] * kld(0, col0 + jj);
+                    e = fmaf(a.c_err[2], kld(2, col0 + jj), e);
+                    e = fmaf(a.c_err[3], kld(3, col0 + jj), e);
+                    e = fmaf(a.c_err[4], kld(4, col0 + jj), e);
+                    e = fmaf(a.c_err[5], kld(5, col0 + jj), e);
+                    e = fmaf(a.c_err[6], v[jj], e);
+                    e *= dtf;
+                    const float tol = a.atol + a.rtol * fmaxf(fabsf(yv[jj]), fabsf(kld(7, col0 + jj)));
+                    const float q = e / tol;
+                    s0 += (double)(q * q);
+                  }
+                }
+              }
+            }
+            bool finished = false;
+            if (combine) {
+              ++stage;
+            } else if (stage == 0) {
+              cta_sum(s0, s1);
+              dp5_probe_step(s0, s1, nel, h0, d1);
+              const float hf = (float)h0;
+              part = 0.f;
+#pragma unroll 1
+              for (int g = 0; g < ngq; ++g) {   // the probe y0 + h0 f0
+                const int col0 = cw * DQ + g * 16;
+                float v[16];
+                lds16(yrow + col0, v);
+#pragma unroll
+                for (int jj = 0; jj < 16; ++jj) {
+                  v[jj] = fmaf(hf, 1.f * (row_ok ? kld(0, col0 + jj) : 0.f), v[jj]);
+                  part += v[jj];
+                }
+                tmem_st16f(t_lane + T_R1 + col0, v);
+              }
+              stage = kProbe;
+            } else if (stage == kProbe) {
+              cta_sum(s0, s1);
+              dt = dp5_first_step(s0, nel, h0, d1);
+              part = form_u2();
+              stage = 1;
+            } else {
+              // ---- the step decision (ad_control_kernel's arithmetic) ----
+              cta_sum(s0, s1);
+              const double ratio = sqrt(s0 / nel);
+              ++att;
+              int fail = -1, on1 = on;
+              const bool ok = ratio <= 1.0;
+              double t1 = t, dt_new = 0.0;
+              if (!isfinite(ratio)) {
+                fail = kErrNonFinite;
+              } else {
+                if (ok) {
+                  t1 = t + dt;
+                  while (on1 < a.n_out && a_param.t_out[on1] <= t1) ++on1;
+                  ++n_acc;
+                } else {
+                  ++n_rej;
+                }
+                dt_new = dp5_next_step(dt, ratio);
+                if (on1 < a.n_out) {
+                  if (att >= a.max_steps) fail = kErrMax;
+                  else if (t1 + dt_new == t1) fail = kErrUnderflow;
+                }
+              }
+              const size_t MD = (size_t)a.B * N * D;
+              float* srow = a_param.states + ((size_t)img * N + r) * D;
+              if (fail < 0 && ok) {
+                // dense output for every output time in (t, t1] (ad_commit_kernel's arithmetic), then y0 <- y1
+                if (row_ok) {
+#pragma unroll 1
+                  for (int c4 = 0; c4 < DQ / 4; ++c4) {
+                    const int col = cw * DQ + c4 * 4;
+                    Dp5Quartic qa[4];
+#pragma unroll
+                    for (int i = 0; i < 4; ++i) {
+                      const float f0 = kld(0, col + i), f1 = kld(6, col + i), y1 = kld(7, col + i);
+                      float m = a.c_mid[0] * f0;
+                      m = fmaf(a.c_mid[2], kld(2, col + i), m);
+                      m = fmaf(a.c_mid[3], kld(3, col + i), m);
+                      m = fmaf(a.c_mid[4], kld(4, col + i), m);
+                      m = fmaf(a.c_mid[5], kld(5, col + i), m);
+                      m = fmaf(a.c_mid[6], f1, m);
+                      qa[i] = Dp5Quartic(yrow[col + i], y1, f0, f1, m, dtf);
+                      yrow[col + i] = y1;
+                    }
+                    for (int jo = on; jo < on1; ++jo) {
+                      const float x = (float)((a_param.t_out[jo] - t) / dt);
+                      *reinterpret_cast<float4*>(srow + (size_t)jo * MD + col) = make_float4(qa[0].at(x), qa[1].at(x), qa[2].at(x), qa[3].at(x));
+                    }
+                  }
+                }
+                k1s = 6 - k1s;
+                t = t1;
+                on = on1;
+              }
+              if (fail >= 0 && row_ok) {   // a failed image stops: the rows it has not reached are NaN
+                for (int jo = on; jo < a.n_out; ++jo)
+                  for (int c = 0; c < DQ; c += 4)
+                    *reinterpret_cast<float4*>(srow + (size_t)jo * MD + cw * DQ + c) = make_float4(NAN, NAN, NAN, NAN);
+              }
+              dt = dt_new;
+              finished = fail >= 0 || on >= a.n_out;
+              if (finished) {
+                if (threadIdx.x == 0) {
+                  if (a_param.nfe) a_param.nfe[img] = nfe_base + 6 * att;
+                  if (a_param.accepted) a_param.accepted[img] = n_acc;
+                  if (a_param.rejected) a_param.rejected[img] = n_rej;
+                  a_param.status[img] = fail + 1;
+                }
+                img = fetch(a_param);
+                if (threadIdx.x == 0) {
+                  ctl[0] = img < a_param.B ? CTL_NEXT : CTL_DONE;
+                  if (img >= a_param.B) ctl[2] = 1;
+                }
+                stepping = false;
+              } else {
+                part = form_u2();
+                stage = 1;
+              }
+            }
+            if (!finished) {
+              if (threadIdx.x == 0) ctl[0] = CTL_RUN;
+              centre_from_r1(part);
             }
           } else {
             // ---- k = scaler (OUT + b2); stage combine on the resident state; next stage input -> xc ----
@@ -670,6 +1007,11 @@ solve_resident_kernel(const __grid_constant__ CUtensorMap tmW1, const __grid_con
   }
   ptx::tc_fence_before();
   __syncthreads();
+  if constexpr (ADAPTIVE) {
+    // no TMA write may land after the CTA exits: wait for the allocations issued past the last one consumed
+    if (warp == LOADER)
+      for (uint32_t g = (uint32_t)ctl[3]; g < ld_issued; ++g) ptx::mbar_wait(bar_full + (g & (NB - 1)), (g / NB) & 1);
+  }
 #ifdef RES_TRACE
   if (blockIdx.x == 0 && threadIdx.x == 0)
     for (int w = 0; w < 2; ++w)
@@ -735,6 +1077,41 @@ bool build_sched(int D, int H, int C, Sched& sc) {
   return true;
 }
 
+// null when the kernel covers the shape with `args_bytes` of arguments in shared memory, else what is out of range
+const char* resident_envelope(const Plan& p, int args_bytes) {
+  if (p.variant != ODEVIT_FIELD_PARALLEL) return "the PARALLEL field only";
+  if (p.precision != ODEVIT_BF16) return "bf16 precision only";
+  if (p.d != 64) return "head dim 64 only";
+  if (p.D % 64 || p.D > 192) return "dim a multiple of 64, <= 192";
+  if (p.hid % 128 || p.hid < 128) return "hidden a multiple of 128";
+  if (p.N > 128 || p.N < 1) return "1..128 tokens";
+  if (3 * p.H + p.hid / 128 + 1 > kMaxJobs || 4 * p.H + 5 * (p.hid / 128) > kMaxAllocs || 3 * p.D + p.hid > 0x7fff)
+    return "the job list of one evaluation is too long";
+  const int RA = (p.N + 15) / 16 * 16;
+  if (smem_layout(RA, p.N, p.D, p.hid, args_bytes).total > 227 * 1024) return "the state does not fit in shared memory";
+  return nullptr;
+}
+
+template <bool FULL, bool ADAPTIVE, class Args>
+int launch_resident(const Args& a, const CUtensorMap& t1, const CUtensorMap& t2, int grid, cudaStream_t s) {
+  const int bytes = smem_layout(a.RA, a.N, a.D, a.hid, res_smem_args<Args>()).total;
+  static int configured_bytes = 0;
+  if (bytes > configured_bytes) {
+    ODV_CUDA(cudaFuncSetAttribute(solve_resident_kernel<FULL, ADAPTIVE>, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes));
+    configured_bytes = bytes;
+  }
+  solve_resident_kernel<FULL, ADAPTIVE><<<grid, res_threads(FULL), bytes, s>>>(t1, t2, a);
+  ODV_LAUNCH_CHECK();
+  return 0;
+}
+
+int resident_tmaps(const Plan& p, const WeightBufs& wb, CUtensorMap* t1, CUtensorMap* t2) {
+  const int R = 3 * p.D + p.hid, K2 = p.D + p.hid;
+  ODV_TRY(make_tmap_2d_bf16(t1, wb.w1cat, p.D, R, p.D, 64, 64));
+  ODV_TRY(make_tmap_2d_bf16(t2, wb.w2cat, K2, p.D, K2, 64, 64));
+  return 0;
+}
+
 }  // namespace
 
 size_t solve_resident_scratch_floats(const Plan& p) {
@@ -743,12 +1120,42 @@ size_t solve_resident_scratch_floats(const Plan& p) {
   return (size_t)grid * 3 * p.D * 128;
 }
 
-bool solve_resident_shape_ok(const Plan& p) {
-  if (p.variant != ODEVIT_FIELD_PARALLEL || p.precision != ODEVIT_BF16) return false;
-  if (p.d != 64 || p.D % 64 || p.D > 192 || p.hid % 128 || p.hid < 128 || p.N > 128 || p.N < 1) return false;
-  if (3 * p.H + p.hid / 128 + 1 > kMaxJobs || 4 * p.H + 5 * (p.hid / 128) > kMaxAllocs || 3 * p.D + p.hid > 0x7fff) return false;
-  const int RA = (p.N + 15) / 16 * 16;
-  return smem_layout(RA, p.N, p.D, p.hid).total <= 227 * 1024;
+bool solve_resident_shape_ok(const Plan& p) { return resident_envelope(p, res_smem_args<ResArgs>()) == nullptr; }
+
+const char* solve_resident_adaptive_envelope(const Plan& p) { return resident_envelope(p, res_smem_args<ResArgsAd>()); }
+
+size_t solve_resident_adaptive_scratch_floats(const Plan& p) {
+  const int sms = num_sms();
+  const int grid = p.B < sms ? p.B : sms;
+  return (size_t)grid * 8 * p.D * ((p.N + 15) / 16 * 16);
+}
+
+int solve_resident_adaptive(const Plan& p, const WeightBufs& wb, const float* x0, const double* t_out, int n_out,
+                            double rtol, double atol, double first_step, int max_steps, float* states, int* nfe,
+                            int* accepted, int* rejected, int* status, float* kbuf, int* next_image, cudaStream_t s) {
+  ProfScope prof(KC_RESIDENT, s);
+  ResArgsAd a;
+  a.B = p.B; a.N = p.N; a.D = p.D; a.H = p.H; a.hid = p.hid;
+  a.RA = (p.N + 15) / 16 * 16;
+  a.NK = a.RA;
+  a.n_out = n_out; a.max_steps = max_steps;
+  a.scaler = p.scaler; a.rtol = (float)rtol; a.atol = (float)atol;
+  a.first_step = first_step;
+  for (int i = 0; i < 6; ++i) {
+    a.b[i] = kDopri5.b[i];
+    for (int j = 0; j < 6; ++j) a.a[i][j] = kDopri5.a[i][j];
+  }
+  for (int i = 0; i < 7; ++i) { a.c_err[i] = kDopri5Err[i]; a.c_mid[i] = kDopri5Mid[i]; }
+  for (int i = 0; i < kMaxGrid; ++i) a.t_out[i] = i < n_out ? t_out[i] : 0.0;
+  a.x0 = x0; a.states = states; a.b1cat = wb.b1cat; a.b2 = wb.b2; a.kbuf = kbuf; a.next_image = next_image;
+  a.nfe = nfe; a.accepted = accepted; a.rejected = rejected; a.status = status;
+  if (!build_sched(p.D, p.H, p.hid / 128, a.sc)) return set_error(ODEVIT_ERR_INVALID_ARG, "resident solver: allocation list too long");
+  CUtensorMap t1, t2;
+  ODV_TRY(resident_tmaps(p, wb, &t1, &t2));
+  const int sms = num_sms();
+  const int grid = p.B < sms ? p.B : sms;
+  ODV_CUDA(cudaMemsetAsync(next_image, 0, sizeof(int), s));
+  return p.N > 96 ? launch_resident<true, true>(a, t1, t2, grid, s) : launch_resident<false, true>(a, t1, t2, grid, s);
 }
 
 bool solve_resident_supports(const Plan& p, int n_grid, bool wants_p_traj, bool has_tape) {
@@ -775,24 +1182,11 @@ int solve_resident(const Plan& p, const WeightBufs& wb, const Tableau& tb, const
   a.x0 = x0; a.states = states; a.final_state = final_state; a.p_last = p_last;
   a.b1cat = wb.b1cat; a.b2 = wb.b2; a.kbuf = kbuf;
   if (!build_sched(p.D, p.H, p.hid / 128, a.sc)) return set_error(ODEVIT_ERR_INVALID_ARG, "resident solver: allocation list too long");
-  const int R = 3 * p.D + p.hid, K2 = p.D + p.hid;
   CUtensorMap t1, t2;
-  ODV_TRY(make_tmap_2d_bf16(&t1, wb.w1cat, p.D, R, p.D, 64, 64));
-  ODV_TRY(make_tmap_2d_bf16(&t2, wb.w2cat, K2, p.D, K2, 64, 64));
-  const Smem L = smem_layout(a.RA, a.N, a.D, a.hid);
-  const bool full = p.N > 96;
-  static int configured_bytes[2] = {0, 0};
-  if (L.total > configured_bytes[full]) {
-    if (full) ODV_CUDA(cudaFuncSetAttribute(solve_resident_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, L.total));
-    else ODV_CUDA(cudaFuncSetAttribute(solve_resident_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, L.total));
-    configured_bytes[full] = L.total;
-  }
+  ODV_TRY(resident_tmaps(p, wb, &t1, &t2));
   const int sms = num_sms();
   const int grid = p.B < sms ? p.B : sms;
-  if (full) solve_resident_kernel<true><<<grid, res_threads(true), L.total, s>>>(t1, t2, a);
-  else solve_resident_kernel<false><<<grid, res_threads(false), L.total, s>>>(t1, t2, a);
-  ODV_LAUNCH_CHECK();
-  return 0;
+  return p.N > 96 ? launch_resident<true, false>(a, t1, t2, grid, s) : launch_resident<false, false>(a, t1, t2, grid, s);
 }
 
 }  // namespace odevit

@@ -261,7 +261,8 @@ class ViTMacaron(nn.Module):
             res = ops.ode_solve_adaptive(tokens, t, block.field_spec(self.odefunc.scaler), block.field_weights(),
                                          cfg["rtol"], cfg["atol"], first_step=cfg.get("first_step"),
                                          max_num_steps=cfg.get("max_num_steps", ops.DOPRI5_MAX_NUM_STEPS),
-                                         differentiable=cfg.get("differentiable", False))
+                                         differentiable=cfg.get("differentiable", False),
+                                         capturable=cfg.get("capturable", False))
             if idx is not None:
                 res["rows"] = res["states"][idx]
         else:

@@ -552,6 +552,29 @@ def _adaptive_call(x0, t_c, T: int, spec: FieldSpec, names, weights, rtol: float
     return st, states, counts
 
 
+_ADAPTIVE_STATUS = {1: "max_num_steps ({max_steps}) exceeded before t_out[-1]", 2: "non-finite error ratio",
+                    3: "underflow in dt (t + dt == t)"}
+
+
+def _adaptive_resident_call(x0, t_c, T: int, spec: FieldSpec, names, weights, rtol: float, atol: float, fs: float,
+                            max_num_steps: int):
+    """One odevit_solve_adaptive_resident call (enqueued only: no synchronisation).
+    Returns (states [T,B,N,D], counts [4,B] int32 = nfe, accepted, rejected, status)."""
+    B, N, D = x0.shape
+    desc = spec.desc(B, N)
+    w, keep = _pack_weights(names, weights)
+    states = torch.empty(T, B, N, D, device=x0.device, dtype=torch.float32)
+    counts = torch.empty(4, B, device=x0.device, dtype=torch.int32)
+    buf, ws, ws_bytes = _workspace(desc, _lib.WS_SOLVE_ADAPTIVE_RESIDENT, 0, x0.device)
+    with torch.cuda.device(x0.device):
+        st = _lib.lib().odevit_solve_adaptive_resident(ctypes.byref(desc), ctypes.byref(w), _ptr(x0), t_c, T,
+                                                       float(rtol), float(atol), fs, int(max_num_steps), _ptr(states),
+                                                       _ptr(counts[0]), _ptr(counts[1]), _ptr(counts[2]),
+                                                       _ptr(counts[3]), ws, ws_bytes, _stream())
+    _lib.check(st, "odevit_solve_adaptive_resident")
+    return states, counts
+
+
 def _adaptive_check(st: int, what: str) -> None:
     if st == _lib.ERR_NOT_CONVERGED:
         raise NotConvergedError(_lib.lib().odevit_last_error_string().decode("utf-8", "replace"))
@@ -616,7 +639,8 @@ class _AdaptiveSolve(torch.autograd.Function):
 
 def ode_solve_adaptive(x0: torch.Tensor, t: torch.Tensor, spec: FieldSpec, weights: Dict[str, Optional[torch.Tensor]],
                        rtol: float, atol: float, first_step: Optional[float] = None,
-                       max_num_steps: int = DOPRI5_MAX_NUM_STEPS, differentiable: bool = False):
+                       max_num_steps: int = DOPRI5_MAX_NUM_STEPS, differentiable: bool = False,
+                       capturable: bool = False):
     """Adaptive Dormand-Prince 5(4) solve with per-image step control (odevit_solve_adaptive).
 
     torchdiffeq's dopri5 run on every image on its own: the error norm, the accept / reject decisions, the step sizes
@@ -629,9 +653,22 @@ def ode_solve_adaptive(x0: torch.Tensor, t: torch.Tensor, spec: FieldSpec, weigh
     (discretise-then-optimise: odevit_solve_adaptive_record / odevit_solve_adaptive_bwd).  Gradients with respect to
     `t` are not built.
 
+    capturable=True: the same algorithm inside the on-chip-state kernel (odevit_solve_adaptive_resident): one launch, no
+    synchronisation, so the call can be captured into a CUDA graph; a replay decides the step sequence on the device
+    again.  Failures are reported per image in `status` [B] (0 ok, 1 max_num_steps, 2 non-finite error ratio, 3 dt
+    underflow; a failed image's rows from the first output it did not reach are NaN).  Outside a capture `status` is
+    read once after the launch and the lowest failed image raises NotConvergedError; inside a capture nothing is checked.
+    Covers the PARALLEL field in bf16 at on-chip shapes (head dim 64, dim <= 192, <= 128 tokens, len(t) <= 129), inference
+    only: anything else raises, it never falls back to the synchronising solve.  This is a different contract, not a
+    faster setting: the default path is the forward of the differentiable solve and raises at the first failure.
+
     Returns dict(states [len(t),B,N,D] (row i = solution at t[i]), final [B,N,D], nfe [B], accepted [B], rejected [B]
-    (int32, device), rounds (int: rounds with at least one image still stepping = max_b accepted + rejected))."""
+    (int32, device), rounds (int: rounds with at least one image still stepping = max_b accepted + rejected; with
+    capturable=True a 0-d device tensor) and, with capturable=True, status [B] (int32, device))."""
     names = tuple(k for k, v in weights.items() if v is not None)
+    if capturable:
+        return _ode_solve_adaptive_capturable(x0, t, spec, weights, names, rtol, atol, first_step, max_num_steps,
+                                              differentiable)
     track = torch.is_grad_enabled() and (x0.requires_grad or any(weights[k].requires_grad for k in names))
     if track and not differentiable:
         raise OdevitError("the adaptive solve is inference-only (no backward is built): run it under torch.no_grad() "
@@ -658,6 +695,35 @@ def ode_solve_adaptive(x0: torch.Tensor, t: torch.Tensor, spec: FieldSpec, weigh
     rounds = int((counts[1] + counts[2]).max().item())
     return {"states": states, "final": states[-1], "nfe": counts[0], "accepted": counts[1], "rejected": counts[2],
             "rounds": rounds}
+
+
+def _ode_solve_adaptive_capturable(x0, t, spec: FieldSpec, weights, names, rtol, atol, first_step, max_num_steps,
+                                   differentiable):
+    if differentiable:
+        raise OdevitError("capturable=True is inference-only: it cannot be combined with differentiable=True")
+    if torch.is_grad_enabled() and (x0.requires_grad or any(weights[k].requires_grad for k in names)):
+        raise OdevitError("the capturable adaptive solve is inference-only: run it under torch.no_grad() or detach x0 "
+                          "and the weights")
+    if spec.has_dropout:
+        raise OdevitError("the capturable adaptive solve is inference-only: the field's dropout must be 0 (call .eval())")
+    t_host = t.detach().to("cpu", torch.float32).contiguous()
+    T = int(t_host.numel())
+    t_c = (ctypes.c_float * max(1, T))(*t_host.tolist())
+    fs = 0.0 if first_step is None else float(first_step)
+    if first_step is not None and not fs > 0:
+        raise ValueError(f"first_step must be > 0, got {first_step}")
+    x0 = _require_cuda(x0.detach(), "x0")
+    states, counts = _adaptive_resident_call(x0, t_c, T, spec, names, [weights[k].detach() for k in names], rtol,
+                                             atol, fs, max_num_steps)
+    if not torch.cuda.is_current_stream_capturing():
+        status = counts[3].cpu()
+        bad = torch.nonzero(status).flatten()
+        if bad.numel():
+            b = int(bad[0])
+            raise NotConvergedError(f"image {b}: " + _ADAPTIVE_STATUS.get(int(status[b]), "status %d" % int(status[b]))
+                                    .format(max_steps=int(max_num_steps)))
+    return {"states": states, "final": states[-1], "nfe": counts[0], "accepted": counts[1], "rejected": counts[2],
+            "status": counts[3], "rounds": (counts[1] + counts[2]).max()}
 
 
 def fd_curvature(states: torch.Tensor, delta_t: float) -> torch.Tensor:

@@ -235,15 +235,18 @@ def _check_field_module(func, who: str) -> None:
 
 
 def odeint_adaptive(func, y0: torch.Tensor, t: torch.Tensor, *, rtol: float = 1e-7, atol: float = 1e-9,
-                    options: Optional[dict] = None, return_stats: bool = False, differentiable: bool = False):
+                    options: Optional[dict] = None, return_stats: bool = False, differentiable: bool = False,
+                    capturable: bool = False):
     """`torchdiffeq.odeint(func, y0, t, method="dopri5", rtol, atol, options)` for the fused vector field, with the
     step size controlled PER IMAGE (ops.ode_solve_adaptive): image b's error norm, steps and dense output depend on
     image b alone, where torchdiffeq takes one norm over the batch.  `t` strictly increasing; options: `first_step`,
     `max_num_steps` (attempted steps per image over the whole solve, not per output interval).  Exports no attention
     maps.  Inference only unless `differentiable`: then the trajectory is differentiable with respect to y0 and the
     field's weights, with each image's accepted steps frozen (not the continuous adjoint, and not autograd through an
-    unrolled torchdiffeq solve).  Returns the trajectory [len(t), *y0.shape], or (trajectory, stats) with stats =
-    dict(nfe, accepted, rejected: int32 [B] device tensors, rounds: int) when `return_stats`."""
+    unrolled torchdiffeq solve).  `capturable`: the on-chip, non-synchronising form that a CUDA graph can capture
+    (ops.ode_solve_adaptive; stats then also hold `status` and `rounds` is a 0-d device tensor).  Returns the trajectory
+    [len(t), *y0.shape], or (trajectory, stats) with stats = dict(nfe, accepted, rejected: int32 [B] device tensors,
+    rounds: int) when `return_stats`."""
     _check_field_module(func, "odeint_adaptive")
     options = dict(options or {})
     unknown = set(options) - {"first_step", "max_num_steps"}
@@ -252,19 +255,19 @@ def odeint_adaptive(func, y0: torch.Tensor, t: torch.Tensor, *, rtol: float = 1e
     res = ops.ode_solve_adaptive(y0, t, func.block.field_spec(func.scaler), func.block.field_weights(), rtol, atol,
                                  first_step=options.get("first_step"),
                                  max_num_steps=options.get("max_num_steps", ops.DOPRI5_MAX_NUM_STEPS),
-                                 differentiable=differentiable)
+                                 differentiable=differentiable, capturable=capturable)
     if return_stats:
-        return res["states"], {k: res[k] for k in ("nfe", "accepted", "rejected", "rounds")}
+        return res["states"], {k: res[k] for k in ("nfe", "accepted", "rejected", "rounds", "status") if k in res}
     return res["states"]
 
 
 def adaptive_solve_args(model: nn.Module, output_flags: Dict[str, bool]) -> dict:
     """Checks a model's `adaptive_solve` request (a dict with rtol, atol and optionally first_step, max_num_steps,
-    differentiable) and the forward's arguments against what the adaptive solve can give."""
+    differentiable, capturable) and the forward's arguments against what the adaptive solve can give."""
     cfg = dict(model.adaptive_solve)
-    unknown = set(cfg) - {"rtol", "atol", "first_step", "max_num_steps", "differentiable"}
+    unknown = set(cfg) - {"rtol", "atol", "first_step", "max_num_steps", "differentiable", "capturable"}
     if unknown or "rtol" not in cfg or "atol" not in cfg:
-        raise ValueError(f"adaptive_solve takes rtol, atol [, first_step, max_num_steps, differentiable], "
+        raise ValueError(f"adaptive_solve takes rtol, atol [, first_step, max_num_steps, differentiable, capturable], "
                          f"got {sorted(model.adaptive_solve)}")
     for name, on in output_flags.items():
         if on:
@@ -599,7 +602,8 @@ class ViTNeuralODE(nn.Module):
                                      self.odefunc.block.field_weights(), cfg["rtol"], cfg["atol"],
                                      first_step=cfg.get("first_step"),
                                      max_num_steps=cfg.get("max_num_steps", ops.DOPRI5_MAX_NUM_STEPS),
-                                     differentiable=cfg.get("differentiable", False))
+                                     differentiable=cfg.get("differentiable", False),
+                                     capturable=cfg.get("capturable", False))
         states, final = res["states"], res["final"]
         logits = self.head(final[:, 0])
         out = {
