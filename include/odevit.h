@@ -435,6 +435,18 @@ int odevit_drop_state_advance(uint64_t* state, odevit_stream_t stream);
 int64_t odevit_launch_count(void);
 void odevit_reset_launch_count(void);
 
+/* Deterministic mode (torch.use_deterministic_algorithms(True) in the Python layer).  While on, every floating-point
+ * reduction of the backward paths -- the split-K weight-gradient GEMMs, the bias-gradient column sums, the norm and
+ * res_scale gradient unfold, the extract_mass blur transpose -- sums in a fixed order (partials in workspace scratch,
+ * then one ordered pass) instead of through atomics: identical inputs give bitwise-identical outputs on the same build,
+ * GPU model and SM count.  Off (the default) runs the atomic kernels, unchanged.  odevit_workspace_bytes returns what
+ * the CURRENT mode needs (the backward layouts grow by the partial-slab scratch), so query it after setting the mode.
+ * odevit_gemm_bf16 in this mode does not split K.
+ * Scope is process-wide, not per thread: PyTorch's switch is process-wide and the backward runs on PyTorch's autograd
+ * thread, not on the thread that set it.  Change it only between calls, not while another thread is inside one. */
+int odevit_set_deterministic(int32_t on);
+int32_t odevit_deterministic(void);
+
 /* Diagnostic entry (no reference counterpart): the GEMM kernel on its own, for unit parity tests.
  *   C[M,N] (fp32, row-major) = or += sum_k A(m,k) * B(n,k), bf16 operands.
  *   mn_major == 0: A is [M,K], B is [N,K] row-major (K contiguous);

@@ -77,6 +77,9 @@ def lib() -> ctypes.CDLL:
     L.odevit_last_error_string.restype = ctypes.c_char_p
     L.odevit_launch_count.restype = ctypes.c_int64
     L.odevit_reset_launch_count.restype = None
+    L.odevit_set_deterministic.restype = ctypes.c_int
+    L.odevit_set_deterministic.argtypes = [ctypes.c_int32]
+    L.odevit_deterministic.restype = ctypes.c_int32
     L.odevit_workspace_bytes.restype = ctypes.c_size_t
     L.odevit_workspace_bytes.argtypes = [ctypes.POINTER(Desc), ctypes.c_int32, ctypes.c_int32]
     L.odevit_field_fwd.restype = ctypes.c_int
@@ -216,4 +219,4 @@ DECLARED_SYMBOLS = ("odevit_abi_version", "odevit_build_info", "odevit_last_erro
                     "odevit_workspace_bytes", "odevit_field_fwd", "odevit_solve_fwd", "odevit_solve_bwd",
                     "odevit_field_bwd", "odevit_tape_bytes", "odevit_fd_curvature", "odevit_jasmin_rowmax", "odevit_encoder_cache_bytes", "odevit_encoder_fwd", "odevit_launch_count", "odevit_reset_launch_count", "odevit_drop_state_advance", "odevit_solve_fwd_lean", "odevit_solve_adaptive", "odevit_solve_adaptive_record", "odevit_solve_adaptive_resident", "odevit_adaptive_tape_bytes", "odevit_solve_adaptive_bwd", "odevit_solve_uses_resident", "odevit_tokens_fwd", "odevit_head_ce_fwd", "odevit_head_ce_bwd", "odevit_extract_mass_fwd", "odevit_extract_mass_bwd", "odevit_pil_bilinear_ksize", "odevit_pil_bilinear_tables", "odevit_preprocess_u8",
                     "odevit_gemm_bf16", "odevit_profile_enable", "odevit_profile_reserve", "odevit_profile_num_classes", "odevit_profile_class_name",
-                    "odevit_profile_read")
+                    "odevit_profile_read", "odevit_set_deterministic", "odevit_deterministic")

@@ -35,6 +35,11 @@ namespace odevit {
 // (PyTorch runs the backward on its own autograd thread, which must be counted too).
 static thread_local char g_err[512] = "ok";
 static std::atomic<int64_t> g_launches{0};
+// Process-wide like torch.use_deterministic_algorithms, which the Python layer mirrors into it (and like the counter:
+// the backward runs on PyTorch's autograd thread)
+static std::atomic<int> g_deterministic{0};
+
+bool deterministic() { return g_deterministic.load(std::memory_order_relaxed) != 0; }
 
 int set_error(int code, const char* fmt, ...) {
   va_list ap;
@@ -60,7 +65,7 @@ ProfState g_prof;
 const char* const kClassNames[KC_COUNT] = {
     "center_rows", "gemm_in_qkv_fc1", "attn_qk", "softmax", "attn_pv", "gemm_out_rk",
     "bwd_gemm_doh", "bwd_gemm_g2", "bwd_attn", "bwd_softmax", "bwd_gemm_dx", "bwd_gemm_g1",
-    "bwd_colsum", "combine", "weights", "fused_attn", "fused_attn_bwd", "fd_curvature", "fused_attn_export", "resident_solve", "other"};
+    "bwd_colsum", "combine", "weights", "fused_attn", "fused_attn_bwd", "fd_curvature", "fused_attn_export", "resident_solve", "det_sum", "other"};
 }  // namespace
 
 ProfScope::ProfScope(int c, cudaStream_t st) : cls(c), s(st), slot(-1) {
@@ -182,6 +187,22 @@ StageCtx take_ctx(const Plan& p, Arena& a, bool with_hpre) {
   return c;
 }
 
+// deterministic mode: one scratch region for the partial slabs of whichever reduction runs (they run one after another
+// on the call's stream, each finished by its det_sum before the next starts)
+void det_scratch(const Plan& p, Arena& a) {
+  p.det_ws = nullptr;
+  p.det_ws_bytes = 0;
+  if (!deterministic()) return;
+  const int R = 3 * p.D + p.hid;
+  size_t f = gemm_tc_det_bytes() / 4;
+  auto at_least = [&f](size_t n) { if (n > f) f = n; };
+  at_least(colsum_part_floats(p.M, R));
+  at_least(ln_bwd_part_floats(p.M, p.D));
+  at_least(unfold_part_floats(p.D, p.hid));
+  p.det_ws_bytes = f * 4;
+  p.det_ws = a.f32(f);
+}
+
 void split_scratch(const Plan& p, Arena& a) {
   p.split_a = p.split_b = nullptr;
   p.split_a_bytes = p.split_b_bytes = 0;
@@ -262,6 +283,7 @@ BwdBufs layout_bwd(const Plan& p, Arena& a, int S) {
   b.dd1 = p.split_out ? a.take(MD * e) : nullptr;
   b.dd2 = p.split_out ? a.take(MD * e) : nullptr;
   split_scratch(p, a);
+  det_scratch(p, a);
   return b;
 }
 
@@ -436,7 +458,10 @@ static int gemm_split3(const Plan& p, const GemmArgs& g, cudaStream_t s, bool* t
   return gemm_tc(t, s);
 }
 
-int gemm(const Plan& p, const GemmArgs& g, cudaStream_t s) {
+int gemm(const Plan& p, const GemmArgs& g_in, cudaStream_t s) {
+  GemmArgs g = g_in;
+  g.det_ws = p.det_ws;
+  g.det_ws_bytes = p.det_ws_bytes;
   if (p.precision == ODEVIT_BF16 && gemm_tc_supports(g)) return gemm_tc(g, s);
   if (p.precision == ODEVIT_FP32) {
     bool taken = false;
@@ -770,7 +795,8 @@ int eval_vjp(const Plan& p, const WeightBufs& wb, const StageCtx& c, BwdBufs& b,
   const size_t e = dtype_size(p.act);
   char* dz = reinterpret_cast<char*>(b.dz);
   // (softmax attention, no attention-map dropout, the single-GEMM form of d[O|h]: see below)
-  bool fused_colsum = p.variant == ODEVIT_FIELD_PARALLEL && p.p_attn == 0.f && !p.split_out;
+  // (the deterministic mode sums every bias-gradient block in colsum_accum, which adds its partials in a fixed order)
+  bool fused_colsum = p.variant == ODEVIT_FIELD_PARALLEL && p.p_attn == 0.f && !p.split_out && !deterministic();
   if (p.split_out) {
     // the cotangent enters the out-proj branch under the proj mask and the fc2 branch under the mlp-output mask
     if (gw->fc2_b) return set_error(ODEVIT_ERR_UNSUPPORTED, "dropout with an fc2 bias is not built (the reference has none)");
@@ -820,7 +846,7 @@ int eval_vjp(const Plan& p, const WeightBufs& wb, const StageCtx& c, BwdBufs& b,
       g.kclass = KC_BWD_GEMM_G2;
       ODV_TRY(gemm(p, g, s));
     }
-    if (need_c2) ODV_TRY(colsum_accum(b.dd2, p.act, D, p.M, D, b.c2, s));
+    if (need_c2) ODV_TRY(colsum_accum(b.dd2, p.act, D, p.M, D, b.c2, s, p.det_ws));
   } else {
   {  // d[O|h] = dd @ [Wo|W2];  GELU' on the h half
     GemmArgs g;
@@ -855,7 +881,7 @@ int eval_vjp(const Plan& p, const WeightBufs& wb, const StageCtx& c, BwdBufs& b,
     g.kclass = KC_BWD_GEMM_G2;
     ODV_TRY(gemm(p, g, s));
   }
-  if (need_c2) ODV_TRY(colsum_accum(b.dd, p.act, D, p.M, D, b.c2, s));
+  if (need_c2) ODV_TRY(colsum_accum(b.dd, p.act, D, p.M, D, b.c2, s, p.det_ws));
   }
 
   // ---- attention VJP per (image, head) ----------------------------------------------------------
@@ -886,8 +912,8 @@ int eval_vjp(const Plan& p, const WeightBufs& wb, const StageCtx& c, BwdBufs& b,
     g.kclass = KC_BWD_GEMM_G1;
     ODV_TRY(gemm(p, g, s));
   }
-  if (!fused_colsum) ODV_TRY(colsum_accum(b.dz, p.act, R, p.M, R, b.c1, s));
-  else if (!dq_colsum_done) ODV_TRY(colsum_accum(b.dz, p.act, R, p.M, D, b.c1, s));     // the dq block only
+  if (!fused_colsum) ODV_TRY(colsum_accum(b.dz, p.act, R, p.M, R, b.c1, s, p.det_ws));
+  else if (!dq_colsum_done) ODV_TRY(colsum_accum(b.dz, p.act, R, p.M, D, b.c1, s, p.det_ws));     // the dq block only
   return 0;
 }
 
@@ -910,6 +936,7 @@ int finish_grads(const Plan& p, const odevit_weights* w, const odevit_weight_gra
   u.D = p.D; u.hid = p.hid; u.heads = p.H; u.w = w; u.gw = gw;
   u.G1 = b.G1; u.c1 = b.c1; u.G2 = b.G2; u.c2 = b.c2;
   u.q_scale = q_scale_of(p);
+  u.part = p.det_ws;
   if (p.variant == ODEVIT_FIELD_MACARON) {
     u.c3 = b.c3;
     return unfold_grads_macaron(u, s);
@@ -942,6 +969,12 @@ int odevit_drop_state_advance(uint64_t* state, odevit_stream_t stream) {
 }
 
 int64_t odevit_launch_count(void) { return g_launches.load(); }
+
+int odevit_set_deterministic(int32_t on) {
+  g_deterministic.store(on ? 1 : 0);
+  return 0;
+}
+int32_t odevit_deterministic(void) { return g_deterministic.load(); }
 void odevit_reset_launch_count(void) { g_launches.store(0); }
 
 int odevit_gemm_bf16(int32_t M, int32_t N, int32_t K, int32_t mn_major, const void* A, const void* B, float* C,

@@ -203,7 +203,7 @@ int ffn_vjp(const Plan& p, const WeightBufs& wb, BwdBufs& b, const void* n, cons
     g.kclass = KC_BWD_GEMM_G2;
     ODV_TRY(gemm(p, g, s));
   }
-  ODV_TRY(colsum_accum(b.ddc, p.act, D, p.M, D, b.c3, s));
+  ODV_TRY(colsum_accum(b.ddc, p.act, D, p.M, D, b.c3, s, p.det_ws));
   {  // dn = dh @ W1
     GemmArgs g;
     g.M = p.M; g.N = D; g.K = hid;
@@ -224,7 +224,7 @@ int ffn_vjp(const Plan& p, const WeightBufs& wb, BwdBufs& b, const void* n, cons
     g.kclass = KC_BWD_GEMM_G1;
     ODV_TRY(gemm(p, g, s));
   }
-  return colsum_accum(dh, p.act, hid, p.M, hid, b.c1 + 3 * D, s);
+  return colsum_accum(dh, p.act, hid, p.M, hid, b.c1 + 3 * D, s, p.det_ws);
 }
 
 }  // namespace
@@ -249,6 +249,7 @@ int macaron_vjp(const Plan& p, const WeightBufs& wb, const StageCtx& c, BwdBufs&
     a.x = c.x2; a.dn = b.dn; a.w = w->norm_c_w; a.g_in = g; a.g_out = g;
     a.dd_out = b.ddc; a.dd_type = p.act; a.dd_coef = 1.f;  // attention branch coefficient
     a.dw = gw->norm_c_w; a.db = gw->norm_c_b; a.eps = kLnEps;
+    a.part = p.det_ws;
     ODV_TRY(ln_bwd_rows(a, p.M, D, s));
   }
   // ---- attention:  g1 = g2 + LN2'(x1)^T dn2 ----
@@ -277,7 +278,7 @@ int macaron_vjp(const Plan& p, const WeightBufs& wb, const StageCtx& c, BwdBufs&
     gm.kclass = KC_BWD_GEMM_G2;
     ODV_TRY(gemm(p, gm, s));
   }
-  ODV_TRY(colsum_accum(b.ddc, p.act, D, p.M, D, b.c2, s));
+  ODV_TRY(colsum_accum(b.ddc, p.act, D, p.M, D, b.c2, s, p.det_ws));
   ODV_TRY(attention_vjp(p, c.qkv, c.oh, K2, c.lse, b, nullptr, b.dz, R, make_drop(p, DS_ATTN, ev), s));  // dq|dk|dv -> dz[:, :3D] (ld R)
   {  // dn2 = dz[:, :3D] @ W_in (q rows scaled)
     GemmArgs gm;
@@ -299,12 +300,13 @@ int macaron_vjp(const Plan& p, const WeightBufs& wb, const StageCtx& c, BwdBufs&
     gm.kclass = KC_BWD_GEMM_G1;
     ODV_TRY(gemm(p, gm, s));
   }
-  ODV_TRY(colsum_accum(b.dz, p.act, R, p.M, 3 * D, b.c1, s));
+  ODV_TRY(colsum_accum(b.dz, p.act, R, p.M, 3 * D, b.c1, s, p.det_ws));
   {
     LnBwdArgs a;
     a.x = c.x1; a.dn = b.dn; a.w = w->norm_b_w; a.g_in = g; a.g_out = g;
     a.dd_out = b.ddc; a.dd_type = p.act; a.dd_coef = 0.5f;  // first half-FFN coefficient
     a.dw = gw->norm_b_w; a.db = gw->norm_b_b; a.eps = kLnEps;
+    a.part = p.det_ws;
     ODV_TRY(ln_bwd_rows(a, p.M, D, s));
   }
   // ---- first half-FFN:  g0 = g1 + LN1'(x0)^T dn1 ----
@@ -313,6 +315,7 @@ int macaron_vjp(const Plan& p, const WeightBufs& wb, const StageCtx& c, BwdBufs&
     LnBwdArgs a;
     a.x = c.x0; a.dn = b.dn; a.w = w->norm_a_w; a.g_in = g; a.g_out = g;
     a.dw = gw->norm_a_w; a.db = gw->norm_a_b; a.eps = kLnEps;
+    a.part = p.det_ws;
     ODV_TRY(ln_bwd_rows(a, p.M, D, s));
   }
   // mu = g0; the reverse-mode stage combine (may rewrite b.dd in place: element-wise, read before write)

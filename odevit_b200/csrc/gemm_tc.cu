@@ -91,6 +91,8 @@ struct DevArgs {
   // through all N tiles, the expensive ones spread out); the set of tiles in flight per wave is unchanged.
   int tile_skew;
   Epi epi;
+  // EPI_DET: split-K partial slabs [split_k][M][N] (fp32, row stride N)
+  float* part;
 };
 
 // the tile of `unit` in wave w_ (see DevArgs::tile_skew); a unit without a tile in the last wave is done
@@ -182,7 +184,17 @@ __device__ __forceinline__ void epilogue_role(const DevArgs& g, float* scratch, 
 #pragma unroll
           for (int i = 0; i < 8; ++i) w[i] = ptx::lds_f32x4(((i & 1) ? ld_base1 : ld_base0) + (uint32_t)(512 * i));
           __syncwarp();
-          if (live) epi8_finish<EPI, ATOMIC, FULL>(g.epi, m0, g.M, n, w, pre);
+          if constexpr ((EPI & EPI_DET) != 0 && ATOMIC) {
+            // split-K in the deterministic mode: plain stores into this split's slab; det_sum adds the slabs in order
+            if (live) {
+              float* pp = g.part + ((long long)(tile / (g.tiles_n * g.tiles_m)) * g.M + m0) * g.N + n;
+#pragma unroll
+              for (int i = 0; i < 8; ++i)
+                if (row_in<FULL>(m0, i, g.M)) stg_f32x4(pp + (long long)i * 4 * g.N, scale4(g.epi.alpha, w[i]));
+            }
+          } else {
+            if (live) epi8_finish<EPI, ATOMIC, FULL>(g.epi, m0, g.M, n, w, pre);
+          }
           GT_ADD(2);
         }
       };
@@ -420,7 +432,7 @@ int launch(const CUtensorMap& ta, const CUtensorMap& tb, const DevArgs& d, int u
 template <int CG, int BN, int EPI>
 int launch_major(bool mn, const CUtensorMap& ta, const CUtensorMap& tb, const DevArgs& d, int units, cudaStream_t s) {
   if (!mn) return launch<CG, BN, EPI, false, false>(ta, tb, d, units, s);
-  if constexpr ((EPI == EPI_STORE || EPI == EPI_ACCUM) && BN != 192) {
+  if constexpr ((EPI == EPI_STORE || EPI == EPI_ACCUM || EPI == (EPI_ACCUM | EPI_DET)) && BN != 192) {
     return launch<CG, BN, EPI, true, true>(ta, tb, d, units, s);
   } else {
     return set_error(ODEVIT_ERR_UNSUPPORTED, "gemm_tc: MN-major operands are built for the store / accumulate epilogues");
@@ -453,7 +465,9 @@ int launch_epi(int epi_mode, bool mn, const CUtensorMap& ta, const CUtensorMap& 
       if (d.epi.exact_gelu) return launch_major<CG, BN, EPI_BWD3 | EPI_EXACT>(mn, ta, tb, d, units, s);
       if (d.epi.drop.thresh) return launch_major<CG, BN, EPI_BWD3 | EPI_DROP>(mn, ta, tb, d, units, s);
       return launch_major<CG, BN, EPI_BWD3>(mn, ta, tb, d, units, s);
-    case EPI_ACCUM: return launch_major<CG, BN, EPI_ACCUM>(mn, ta, tb, d, units, s);
+    case EPI_ACCUM:
+      if (d.part) return launch_major<CG, BN, EPI_ACCUM | EPI_DET>(mn, ta, tb, d, units, s);
+      return launch_major<CG, BN, EPI_ACCUM>(mn, ta, tb, d, units, s);
     case EPI_TOKENS: return launch_major<CG, BN, EPI_TOKENS>(mn, ta, tb, d, units, s);
     default: return set_error(ODEVIT_ERR_INVALID_ARG, "gemm_tc: bad epilogue %d", epi_mode);
   }
@@ -466,7 +480,8 @@ struct TileChoice {
   int cg, bn, split_k;
 };
 
-TileChoice choose_tile(const GemmArgs& g, bool mn, int sms) {
+// no_split: the deterministic mode without partial-slab scratch keeps K whole
+TileChoice choose_tile(const GemmArgs& g, bool mn, int sms, bool no_split) {
   const char* env = getenv("ODEVIT_GEMM_TILE");  // "<cg>x<bn>", experiments only
   if (env && !env[0]) env = nullptr;
   const int num_kb = (g.K + BK - 1) / BK;
@@ -480,7 +495,7 @@ TileChoice choose_tile(const GemmArgs& g, bool mn, int sms) {
       const int units = sms / cg;
       const long long tiles = (long long)((g.M + BM * cg - 1) / (BM * cg)) * ((g.N + bn - 1) / bn);
       int sk = 1;
-      if (g.epi_mode == EPI_ACCUM) {
+      if (g.epi_mode == EPI_ACCUM && !no_split) {
         // weight-gradient shapes: few output tiles, very long K -> split K across the idle SMs
         sk = (int)(units / tiles);
         if (sk > num_kb / 8) sk = num_kb / 8;
@@ -570,7 +585,12 @@ int gemm_tc(const GemmArgs& g, cudaStream_t s) {
   ProfScope prof(g.kclass, s);
   const bool mn = (g.a_cs != 1);
   const int sms = num_sms();
-  const TileChoice tc = choose_tile(g, mn, sms);
+  // deterministic mode: a split-K accumulation goes through partial slabs and det_sum (or, without scratch for them,
+  // does not split K); every other GEMM has one writer per output element already
+  const bool det = deterministic() && g.epi_mode == EPI_ACCUM;
+  TileChoice tc = choose_tile(g, mn, sms, false);
+  if (det && tc.split_k > 1 && (!g.det_ws || (size_t)tc.split_k * g.M * g.N * 4 > g.det_ws_bytes))
+    tc = choose_tile(g, mn, sms, true);
   const int cg = tc.cg, bn = tc.bn;
   DevArgs d;
   d.M = g.M; d.N = g.N; d.K = g.K;
@@ -582,6 +602,7 @@ int gemm_tc(const GemmArgs& g, cudaStream_t s) {
   d.split_k = (d.num_kb + d.kb_per_split - 1) / d.kb_per_split;
   d.epi = g.epi;
   d.tile_skew = 0;
+  d.part = (det && d.split_k > 1) ? g.det_ws : nullptr;
   CUtensorMap ta, tb;
   const int brows = bn / cg;
   if (!mn) {
@@ -602,10 +623,20 @@ int gemm_tc(const GemmArgs& g, cudaStream_t s) {
       if (gcd(stride, d.tiles_n) == 1 && stride != 1 && stride != d.tiles_n - 1) { d.tile_skew = sk; break; }
     }
   }
-  if (cg == 1) return launch_epi<1, 128>(g.epi_mode, mn, ta, tb, d, units, s);
-  if (bn == 128) return launch_epi<2, 128>(g.epi_mode, mn, ta, tb, d, units, s);
-  if (bn == 192) return launch_epi<2, 192>(g.epi_mode, mn, ta, tb, d, units, s);
-  return launch_epi<2, 256>(g.epi_mode, mn, ta, tb, d, units, s);
+  if (!d.part) {
+    if (cg == 1) return launch_epi<1, 128>(g.epi_mode, mn, ta, tb, d, units, s);
+    if (bn == 128) return launch_epi<2, 128>(g.epi_mode, mn, ta, tb, d, units, s);
+    if (bn == 192) return launch_epi<2, 192>(g.epi_mode, mn, ta, tb, d, units, s);
+    return launch_epi<2, 256>(g.epi_mode, mn, ta, tb, d, units, s);
+  }
+  if (cg == 1) ODV_TRY((launch_epi<1, 128>(g.epi_mode, mn, ta, tb, d, units, s)));
+  else if (bn == 128) ODV_TRY((launch_epi<2, 128>(g.epi_mode, mn, ta, tb, d, units, s)));
+  else if (bn == 192) ODV_TRY((launch_epi<2, 192>(g.epi_mode, mn, ta, tb, d, units, s)));
+  else ODV_TRY((launch_epi<2, 256>(g.epi_mode, mn, ta, tb, d, units, s)));
+  return det_sum(reinterpret_cast<float*>(g.epi.out), g.epi.ld_out, d.part, d.split_k, (long long)g.M * g.N, g.M, g.N, s, false);
 }
+
+// split_k * tiles never exceeds the units of one wave (choose_tile), and a tile covers at most 128 * cg x 256 outputs
+size_t gemm_tc_det_bytes() { return (size_t)num_sms() * BM * 256 * 4; }
 
 }  // namespace odevit

@@ -23,6 +23,9 @@ struct Plan {
   mutable void* split_a = nullptr;
   mutable void* split_b = nullptr;
   mutable size_t split_a_bytes = 0, split_b_bytes = 0;
+  // deterministic mode: scratch for the partial slabs of the fixed-order reductions; set by layout_bwd (null otherwise)
+  mutable float* det_ws = nullptr;
+  mutable size_t det_ws_bytes = 0;
 };
 // mask of dropout site `site` in field evaluation `e` (e = step * stages + stage)
 Drop make_drop(const Plan& p, int site, long long e);

@@ -19,6 +19,10 @@ namespace odevit {
 int set_error(int code, const char* fmt, ...);
 void count_launch(int n = 1);
 
+// odevit_set_deterministic: every floating-point reduction of the backward paths sums in a fixed order (partials in
+// workspace scratch + det_sum) instead of through atomics
+bool deterministic();
+
 #define ODV_CUDA(call)                                                                   \
   do {                                                                                   \
     cudaError_t _e = (call);                                                             \
@@ -68,6 +72,7 @@ enum KClass : int {
   KC_FD_BOUND,        // finite-difference curvature of the trajectory (single pass)
   KC_FUSED_ATTN_EXPORT,  // fused attention forward that also writes the fp32 attention map
   KC_RESIDENT,        // on-chip-state solver: the whole solve of an image in one persistent CTA
+  KC_DET_SUM,         // deterministic mode: fixed-order sums of the reductions' partial slabs (det_sum)
   KC_OTHER,
   KC_COUNT
 };
@@ -110,7 +115,10 @@ enum EpiMode : int {
   EPI_EXACT = 32,
   // template-only flag (EPI_RK): per-image step size, r = y_coef*y + dt_b*(c_new*v + sum_i c_k[i]*kin[i]) with
   // dt_b = (float)Epi::row_dt[m / rows_per_image] (the adaptive solve: the host passes the tableau without dt)
-  EPI_ROWDT = 64
+  EPI_ROWDT = 64,
+  // template-only flag (EPI_ACCUM, tcgen05 kernel, split-K): each split stores alpha*acc to its own slab of
+  // DevArgs::part with plain stores; det_sum then adds the slabs in split order (the deterministic mode)
+  EPI_DET = 128
 };
 
 // One dropout site of one field evaluation: element (r, c) is kept iff hash(key, r, c) >= thresh and then
@@ -191,7 +199,18 @@ struct GemmArgs {
   int epi_mode = EPI_STORE;
   Epi epi;
   int kclass = KC_OTHER;
+  // deterministic mode: scratch for the split-K partial slabs (EPI_ACCUM); without it (or too small) K is not split
+  float* det_ws = nullptr;
+  size_t det_ws_bytes = 0;
 };
+// bytes of split-K partials any tcgen05 GEMM of the deterministic mode can need (split_k * tiles <= units)
+size_t gemm_tc_det_bytes();
+
+// dst[r * ld_dst + c] += part[0][r, c] + part[1][r, c] + ... (n_slab slabs of [rows, cols], slab_stride floats apart),
+// summed in slab order: the fixed-order second pass of every deterministic reduction.  Timed as KC_DET_SUM, or with
+// own_class false inside the caller's class (the weight-gradient GEMMs: their class time is what the mode costs them)
+int det_sum(float* dst, long long ld_dst, const float* part, int n_slab, long long slab_stride, int rows, int cols,
+            cudaStream_t s, bool own_class = true);
 
 // CUDA-core (FFMA) GEMM: any strides, any M/N/K, fp32 or bf16 operands, fp32 accumulate.
 int gemm_simt(const GemmArgs& g, cudaStream_t s);
@@ -225,9 +244,10 @@ int softmax_rows(float* p, float* copy_to, long long rows, int n, cudaStream_t s
 // ds = p * (dp + dpx - sum_j p*(dp+dpx)), written over dp.  dpx nullable.
 int softmax_bwd_rows(const float* p, float* dp, const float* dpx, long long rows, int n,
                      cudaStream_t s);
-// acc[j] += sum_r X[r, j]
+// acc[j] += sum_r X[r, j].  part: deterministic mode's scratch (colsum_part_floats), required there
 int colsum_accum(const void* X, int x_type, long long ld, int rows, int cols, float* acc,
-                 cudaStream_t s);
+                 cudaStream_t s, float* part = nullptr);
+size_t colsum_part_floats(int rows, int cols);
 
 // Reverse-mode stage combine (the seed and overflow passes of the reverse sweeps, the MACARON VJP):
 // v = sum_i coef[i]*term[i] ; writes out_f32 = v and/or out_dd = cast(dd_scale*v)
@@ -321,7 +341,9 @@ struct UnfoldArgs {
   const float* c1;  // [3D+hid]      = colsum dz
   const float* G2;  // [D, D+hid]    = sum dd^T [O|h]
   const float* c2;  // [D]           = colsum dd
+  float* part = nullptr;   // deterministic mode: partials of the norm and res_scale gradients (unfold_part_floats)
 };
+size_t unfold_part_floats(int D, int hid);
 int unfold_grads_parallel(const UnfoldArgs& a, cudaStream_t s);
 // MACARON (no folded norms; G2/c2/c3 were accumulated WITHOUT res_scale, macaron.py:104):
 //   dW_in += q_scale_row*G1[:3D], dW_fc1 += G1[3D:], dWo += rs*G2[:, :D], dW_fc2 += rs*G2[:, D:],
@@ -345,7 +367,9 @@ struct LnBwdArgs {
   float* dw = nullptr;
   float* db = nullptr;
   float eps = 1e-5f;
+  float* part = nullptr;   // deterministic mode: [blocks, 2, D] per-block partials of dw / db (ln_bwd_part_floats)
 };
+size_t ln_bwd_part_floats(int rows, int D);
 int ln_bwd_rows(const LnBwdArgs& a, int rows, int D, cudaStream_t s);
 // EPI_RK applied to a plain [rows, D] fp32 array v (alpha/bias ignored): the stage combine when the
 // producer of v is not a GEMM.

@@ -143,7 +143,9 @@ __global__ void mass_fwd_kernel(MassArgs g, float* __restrict__ out_mean, float*
   }
 }
 
-// g_mean [B, n] and/or g_heads [B, H, n] -> g_a [B, H, n]
+// g_mean [B, n] and/or g_heads [B, H, n] -> g_a [B, H, n].  DET (deterministic mode): blur^T as a gather with a fixed
+// tap order instead of a scatter through shared-memory atomics
+template <bool DET>
 __global__ void mass_bwd_kernel(MassArgs g, const float* __restrict__ g_mean, const float* __restrict__ g_heads,
                                 float* __restrict__ g_a) {
   __shared__ MassSmem sm;
@@ -158,6 +160,35 @@ __global__ void mass_bwd_kernel(MassArgs g, const float* __restrict__ g_mean, co
     float gf = gm;
     if (g_heads && t < g.n) gf += g_heads[base + t];
     // ---- blur^T: scatter the output gradient through the taps ----
+    if constexpr (DET) {
+      // gather: pixel t collects from the 3 x 3 neighbours whose (reflected) taps land on it.  A neighbour sy reaches y
+      // only from {y-1, y, y+1} (reflect(-1) = 1, reflect(side) = side - 2), with weight the sum of its taps that do.
+      // (sm.tile, the masked tile, is not read again by the backward: it stages the output gradient)
+      if (t < g.n) sm.tile[t] = gf;
+      __syncthreads();
+      if (t < g.n) {
+        if (g.smooth) {
+          const float kw[3] = {g.k1, g.k0, g.k1};
+          float acc = 0.f;
+          for (int sy = y - 1; sy <= y + 1; ++sy) {
+            if (sy < 0 || sy >= g.side) continue;
+            float wy = 0.f;
+#pragma unroll
+            for (int i = 0; i < 3; ++i) if (reflect(sy + i - 1, g.side) == y) wy += kw[i];
+            for (int sx = x - 1; sx <= x + 1; ++sx) {
+              if (sx < 0 || sx >= g.side) continue;
+              float wx = 0.f;
+#pragma unroll
+              for (int j = 0; j < 3; ++j) if (reflect(sx + j - 1, g.side) == x) wx += kw[j];
+              acc = fmaf(wy * wx, sm.tile[sy * g.side + sx], acc);
+            }
+          }
+          gt[t] = acc;
+        } else {
+          gt[t] = gf;
+        }
+      }
+    } else {
     gt[t] = 0.f;
     __syncthreads();
     if (t < g.n) {
@@ -172,6 +203,7 @@ __global__ void mass_bwd_kernel(MassArgs g, const float* __restrict__ g_mean, co
       } else {
         gt[t] = gf;
       }
+    }
     }
     __syncthreads();
     // ---- f = a o keep ----
@@ -241,7 +273,8 @@ int extract_mass_bwd(const float* a, int B, int H, int n, float threshold, int s
   MassArgs g;
   ODV_TRY(mass_args(&g, a, B, H, n, threshold, smooth, scale));
   ProfScope prof(KC_OTHER, s);
-  mass_bwd_kernel<<<B, mass_threads(n), 0, s>>>(g, g_mean, g_heads, g_a);
+  if (deterministic()) mass_bwd_kernel<true><<<B, mass_threads(n), 0, s>>>(g, g_mean, g_heads, g_a);
+  else mass_bwd_kernel<false><<<B, mass_threads(n), 0, s>>>(g, g_mean, g_heads, g_a);
   ODV_LAUNCH_CHECK();
   return 0;
 }

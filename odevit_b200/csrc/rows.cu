@@ -157,6 +157,8 @@ __global__ void __launch_bounds__(256) softmax_bwd_rows_kernel(const float* __re
   }
 }
 
+// DET (deterministic mode): the block's sums go to row blockIdx.y of the partial array `acc` [gridDim.y, cols] instead
+template <bool DET>
 __global__ void __launch_bounds__(128) colsum_kernel(const void* X, int x_type, long long ld, int rows,
                                                      int cols, int rows_per_block, float* acc) {
   const int c = blockIdx.x * 128 + threadIdx.x;
@@ -165,13 +167,15 @@ __global__ void __launch_bounds__(128) colsum_kernel(const void* X, int x_type, 
   const int r1 = min(rows, r0 + rows_per_block);
   float s = 0.f;
   for (int r = r0; r < r1; ++r) s += load_elem_rw(X, (long long)r * ld + c, x_type);
-  atomicAdd(acc + c, s);
+  if constexpr (DET) acc[(long long)blockIdx.y * cols + c] = s;
+  else atomicAdd(acc + c, s);
 }
 
 // bf16 fast path: a warp covers 256 columns with one 16-byte load per lane; the 8 warps of a block take interleaved
 // rows of an `rpb`-row panel (8 independent loads in flight per lane) and meet in shared memory; one atomic per column
 // and block (cols % 8 == 0, ld % 8 == 0).  Same-address atomics serialise in L2 (~27 cycles each): panels are kept
 // tall (few blocks per column) and the memory-level parallelism comes from the unrolled loads instead.
+template <bool DET>
 __global__ void __launch_bounds__(256) colsum_bf16_kernel(const __nv_bfloat16* __restrict__ X, long long ld,
                                                           int rows, int cols, int rpb, float* acc) {
   __shared__ float part[8][256];
@@ -216,7 +220,8 @@ __global__ void __launch_bounds__(256) colsum_bf16_kernel(const __nv_bfloat16* _
       float t = 0.f;
 #pragma unroll
       for (int w = 0; w < 8; ++w) t += part[w][c];
-      atomicAdd(acc + col, t);
+      if constexpr (DET) acc[(long long)blockIdx.y * cols + col] = t;
+      else atomicAdd(acc + col, t);
     }
   }
 }
@@ -475,7 +480,9 @@ __global__ void __launch_bounds__(256) ln_rows_kernel(const float* __restrict__ 
 }
 
 // One warp walks rows row0, row0+stride, ...; the per-column sums for dw / db stay in registers and
-// meet the other warps of the block in shared memory, then one atomic per column and block.
+// meet the other warps of the block in shared memory, then one atomic per column and block (DET: one store into
+// the block's row of a.part [gridDim.x, 2, D]).
+template <bool DET>
 __global__ void __launch_bounds__(256) ln_bwd_rows_kernel(LnBwdArgs a, int rows, int D) {
   __shared__ float red[8][32 * MAX_PER_LANE];  // 32 KB: per-warp column partials
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -540,7 +547,8 @@ __global__ void __launch_bounds__(256) ln_bwd_rows_kernel(LnBwdArgs a, int rows,
       float t = 0.f;
 #pragma unroll
       for (int k = 0; k < 8; ++k) t += red[k][c];
-      atomicAdd(dst + c, t);
+      if constexpr (DET) a.part[((long long)blockIdx.x * 2 + which) * D + c] = t;
+      else atomicAdd(dst + c, t);
     }
   }
 }
@@ -644,7 +652,8 @@ __global__ void __launch_bounds__(256) l2_vjp_fix_kernel(const float* __restrict
 
 // ---- MACARON gradient assembly ------------------------------------------------------------------
 // block = one row i of G2 [D, D+hid]: dWo[i,:] += rs*G2[i,:D], dW2[i,:] += rs*G2[i,D:], biases, and the
-// res_scale gradient <Wo,G2a> + <W2,G2b> + <bo,c2> + <b2,c3> (block partial -> one atomic)
+// res_scale gradient <Wo,G2a> + <W2,G2b> + <bo,c2> + <b2,c3> (block partial -> one atomic; DET: a.part[block])
+template <bool DET>
 __global__ void __launch_bounds__(128) unfold_w2_macaron_kernel(UnfoldArgs a, odevit_weights w, odevit_weight_grads g) {
   const int D = a.D, hid = a.hid, K2 = D + hid;
   const int i = blockIdx.x;
@@ -670,7 +679,10 @@ __global__ void __launch_bounds__(128) unfold_w2_macaron_kernel(UnfoldArgs a, od
   dot = warp_sum(dot);
   if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = dot;
   __syncthreads();
-  if (threadIdx.x == 0 && g.res_scale) atomicAdd(g.res_scale, red[0] + red[1] + red[2] + red[3]);
+  if (threadIdx.x == 0 && g.res_scale) {
+    if constexpr (DET) a.part[i] = red[0] + red[1] + red[2] + red[3];
+    else atomicAdd(g.res_scale, red[0] + red[1] + red[2] + red[3]);
+  }
 }
 
 // ---- weight folding (PARALLEL variant) -------------------------------------------------------
@@ -846,8 +858,10 @@ __global__ void __launch_bounds__(128) unfold_w1_kernel(UnfoldArgs a, odevit_wei
   (void)hid;
 }
 
-// one block = 128 columns i x a slice of kUnfoldRows rows j of G1; partial sums meet through atomics
+// one block = 128 columns i x a slice of kUnfoldRows rows j of G1; partial sums meet through atomics (DET: the slice's
+// sums go to a.part [4][gridDim.y][D] -- norm_a_w, norm_a_b, norm_b_w, norm_b_b -- zeros where the slice has none)
 constexpr int kUnfoldRows = 16;   // (64 left 288 blocks of 64 dependent row steps each: 38 us of latency for 19 MB)
+template <bool DET>
 __global__ void __launch_bounds__(128) unfold_norm_kernel(UnfoldArgs a, odevit_weights w,
                                                           odevit_weight_grads g) {
   const int D = a.D, hid = a.hid;
@@ -873,6 +887,14 @@ __global__ void __launch_bounds__(128) unfold_norm_kernel(UnfoldArgs a, odevit_w
   }
   const float ma = w.mod_attn_scale ? 1.f + w.mod_attn_scale[i] : 1.f;
   const float mm = w.mod_mlp_scale ? 1.f + w.mod_mlp_scale[i] : 1.f;
+  if constexpr (DET) {
+    const long long slab = (long long)gridDim.y * D, o = (long long)blockIdx.y * D + i;
+    a.part[o] = j0 < 3 * D ? ma * s_cn * dwa : 0.f;
+    a.part[slab + o] = j0 < 3 * D ? ma * dba : 0.f;
+    a.part[2 * slab + o] = j1 > 3 * D ? mm * s_cn * dwm : 0.f;
+    a.part[3 * slab + o] = j1 > 3 * D ? mm * dbm : 0.f;
+    return;
+  }
   if (j0 < 3 * D) {
     if (g.norm_a_w) atomicAdd(g.norm_a_w + i, ma * s_cn * dwa);
     if (g.norm_a_b) atomicAdd(g.norm_a_b + i, ma * dba);
@@ -934,21 +956,60 @@ int softmax_bwd_rows(const float* p, float* dp, const float* dpx, long long rows
   return 0;
 }
 
-int colsum_accum(const void* X, int x_type, long long ld, int rows, int cols, float* acc, cudaStream_t s) {
-  ProfScope prof(KC_BWD_COLSUM, s);
-  if (x_type == DT_BF16 && cols % 8 == 0 && ld % 8 == 0 && (reinterpret_cast<uintptr_t>(X) & 15) == 0) {
-    // rows per block: 256 for wide matrices, fewer for narrow ones so that there are at least two blocks per SM
-    const int col_blocks = (cols + 255) / 256;
-    int rpb = 256;
-    while (rpb > 64 && (long long)col_blocks * ((rows + rpb - 1) / rpb) < 296) rpb >>= 1;
-    dim3 grid(col_blocks, (rows + rpb - 1) / rpb);
-    colsum_bf16_kernel<<<grid, 256, 0, s>>>(reinterpret_cast<const __nv_bfloat16*>(X), ld, rows, cols, rpb, acc);
+// (deterministic mode: at most ceil(rows / 64) row panels of partial sums)
+size_t colsum_part_floats(int rows, int cols) { return (size_t)((rows + 63) / 64) * cols; }
+
+int colsum_accum(const void* X, int x_type, long long ld, int rows, int cols, float* acc, cudaStream_t s, float* part) {
+  const bool det = deterministic();
+  if (det && !part) return set_error(ODEVIT_ERR_WORKSPACE, "colsum_accum: the deterministic mode needs partial-sum scratch");
+  int panels = 0;
+  {
+    ProfScope prof(KC_BWD_COLSUM, s);
+    if (x_type == DT_BF16 && cols % 8 == 0 && ld % 8 == 0 && (reinterpret_cast<uintptr_t>(X) & 15) == 0) {
+      // rows per block: 256 for wide matrices, fewer for narrow ones so that there are at least two blocks per SM
+      const int col_blocks = (cols + 255) / 256;
+      int rpb = 256;
+      while (rpb > 64 && (long long)col_blocks * ((rows + rpb - 1) / rpb) < 296) rpb >>= 1;
+      dim3 grid(col_blocks, (rows + rpb - 1) / rpb);
+      panels = grid.y;
+      if (det) colsum_bf16_kernel<true><<<grid, 256, 0, s>>>(reinterpret_cast<const __nv_bfloat16*>(X), ld, rows, cols, rpb, part);
+      else colsum_bf16_kernel<false><<<grid, 256, 0, s>>>(reinterpret_cast<const __nv_bfloat16*>(X), ld, rows, cols, rpb, acc);
+    } else {
+      const int rpb = 256;
+      dim3 grid((cols + 127) / 128, (rows + rpb - 1) / rpb);
+      panels = grid.y;
+      if (det) colsum_kernel<true><<<grid, 128, 0, s>>>(X, x_type, ld, rows, cols, rpb, part);
+      else colsum_kernel<false><<<grid, 128, 0, s>>>(X, x_type, ld, rows, cols, rpb, acc);
+    }
     ODV_LAUNCH_CHECK();
-    return 0;
   }
-  const int rpb = 256;
-  dim3 grid((cols + 127) / 128, (rows + rpb - 1) / rpb);
-  colsum_kernel<<<grid, 128, 0, s>>>(X, x_type, ld, rows, cols, rpb, acc);
+  if (det) ODV_TRY(det_sum(acc, 0, part, panels, cols, 1, cols, s));
+  return 0;
+}
+
+// one thread per element, slabs added in index order (fp32 adds in a fixed order: the result does not depend on which
+// block or CTA produced which slab, nor when)
+__global__ void __launch_bounds__(256) det_sum_kernel(float* __restrict__ dst, long long ld_dst, const float* __restrict__ part,
+                                                      int n_slab, long long slab, int rows, int cols) {
+  const long long n = (long long)rows * cols;
+  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) {
+    float t = part[i];
+    for (int k = 1; k < n_slab; ++k) t += part[k * slab + i];
+    const long long r = i / cols, c = i - r * cols;
+    dst[r * ld_dst + c] += t;
+  }
+}
+
+int det_sum(float* dst, long long ld_dst, const float* part, int n_slab, long long slab_stride, int rows, int cols,
+            cudaStream_t s, bool own_class) {
+  if (!dst || n_slab <= 0 || rows <= 0 || cols <= 0) return 0;
+  if (own_class) {
+    ProfScope prof(KC_DET_SUM, s);
+    return det_sum(dst, ld_dst, part, n_slab, slab_stride, rows, cols, s, false);
+  }
+  const long long n = (long long)rows * cols;
+  const long long blocks = (n + 255) / 256 < 148 * 8 ? (n + 255) / 256 : 148 * 8;
+  det_sum_kernel<<<(unsigned)blocks, 256, 0, s>>>(dst, ld_dst, part, n_slab, slab_stride, rows, cols);
   ODV_LAUNCH_CHECK();
   return 0;
 }
@@ -1153,9 +1214,21 @@ int ln_bwd_rows(const LnBwdArgs& a, int rows, int D, cudaStream_t s) {
   ProfScope prof(KC_COMBINE, s);
   if (D > 32 * MAX_PER_LANE) return set_error(ODEVIT_ERR_UNSUPPORTED, "ln_bwd_rows: D=%d > 1024", D);
   const int blocks = (rows + 7) / 8 < 148 * 4 ? (rows + 7) / 8 : 148 * 4;
-  ln_bwd_rows_kernel<<<blocks, 256, 0, s>>>(a, rows, D);
+  if (!deterministic()) {
+    ln_bwd_rows_kernel<false><<<blocks, 256, 0, s>>>(a, rows, D);
+    ODV_LAUNCH_CHECK();
+    return 0;
+  }
+  if (!a.part) return set_error(ODEVIT_ERR_WORKSPACE, "ln_bwd_rows: the deterministic mode needs partial-sum scratch");
+  ln_bwd_rows_kernel<true><<<blocks, 256, 0, s>>>(a, rows, D);
   ODV_LAUNCH_CHECK();
-  return 0;
+  ODV_TRY(det_sum(a.dw, 0, a.part, blocks, 2LL * D, 1, D, s));
+  return det_sum(a.db, 0, a.part + D, blocks, 2LL * D, 1, D, s);
+}
+
+size_t ln_bwd_part_floats(int rows, int D) {
+  const int blocks = (rows + 7) / 8 < 148 * 4 ? (rows + 7) / 8 : 148 * 4;
+  return (size_t)blocks * 2 * D;
 }
 
 int rk_apply_rows(const Epi& e, const float* v, int rows, int D, cudaStream_t s) {
@@ -1203,9 +1276,20 @@ int unfold_grads_macaron(const UnfoldArgs& a, cudaStream_t s) {
   ProfScope prof(KC_WEIGHTS, s);
   unfold_w1_kernel<<<3 * a.D + a.hid, 128, 0, s>>>(a, *a.w, *a.gw);
   ODV_LAUNCH_CHECK();
-  unfold_w2_macaron_kernel<<<a.D, 128, 0, s>>>(a, *a.w, *a.gw);
+  if (!deterministic()) {
+    unfold_w2_macaron_kernel<false><<<a.D, 128, 0, s>>>(a, *a.w, *a.gw);
+    ODV_LAUNCH_CHECK();
+    return 0;
+  }
+  if (!a.part) return set_error(ODEVIT_ERR_WORKSPACE, "unfold_grads_macaron: the deterministic mode needs partial-sum scratch");
+  unfold_w2_macaron_kernel<true><<<a.D, 128, 0, s>>>(a, *a.w, *a.gw);
   ODV_LAUNCH_CHECK();
-  return 0;
+  return det_sum(a.gw->res_scale, 0, a.part, a.D, 1, 1, 1, s);
+}
+
+size_t unfold_part_floats(int D, int hid) {
+  const size_t norm = (size_t)4 * ((3 * D + hid + kUnfoldRows - 1) / kUnfoldRows) * D;
+  return norm > (size_t)D ? norm : (size_t)D;
 }
 
 int fold_weights_parallel(const FoldArgs& a, cudaStream_t s) {
@@ -1230,8 +1314,18 @@ int unfold_grads_parallel(const UnfoldArgs& a, cudaStream_t s) {
   ProfScope prof(KC_WEIGHTS, s);
   unfold_w1_kernel<<<3 * a.D + a.hid, 128, 0, s>>>(a, *a.w, *a.gw);
   ODV_LAUNCH_CHECK();
-  unfold_norm_kernel<<<dim3((a.D + 127) / 128, (3 * a.D + a.hid + kUnfoldRows - 1) / kUnfoldRows), 128, 0, s>>>(a, *a.w, *a.gw);
-  ODV_LAUNCH_CHECK();
+  const dim3 ngrid((a.D + 127) / 128, (3 * a.D + a.hid + kUnfoldRows - 1) / kUnfoldRows);
+  if (!deterministic()) {
+    unfold_norm_kernel<false><<<ngrid, 128, 0, s>>>(a, *a.w, *a.gw);
+    ODV_LAUNCH_CHECK();
+  } else {
+    if (!a.part) return set_error(ODEVIT_ERR_WORKSPACE, "unfold_grads_parallel: the deterministic mode needs partial-sum scratch");
+    unfold_norm_kernel<true><<<ngrid, 128, 0, s>>>(a, *a.w, *a.gw);
+    ODV_LAUNCH_CHECK();
+    const long long slab = (long long)ngrid.y * a.D;
+    float* dst[4] = {a.gw->norm_a_w, a.gw->norm_a_b, a.gw->norm_b_w, a.gw->norm_b_b};
+    for (int k = 0; k < 4; ++k) ODV_TRY(det_sum(dst[k], 0, a.part + k * slab, ngrid.y, a.D, 1, a.D, s));
+  }
   unfold_w2_kernel<<<a.D, 128, 0, s>>>(a, *a.gw);
   ODV_LAUNCH_CHECK();
   return 0;

@@ -109,22 +109,23 @@ def _ptr(t: Optional[torch.Tensor]):
     return _vp(t.data_ptr()) if t is not None else None
 
 
-_WS_CACHE: Dict[Tuple[int, int, int], torch.Tensor] = {}
+_WS_CACHE: Dict[Tuple[int, int, int, bool], torch.Tensor] = {}
 
 
 def _workspace(desc: _lib.Desc, kind: int, method: int, device: torch.device):
-    """A cached, 1024-byte aligned device workspace per (device, kind, STREAM).
+    """A cached, 1024-byte aligned device workspace per (device, kind, STREAM, deterministic mode).
 
     Keyed by the current stream so that (a) two streams never share scratch memory and (b) a CUDA-graph capture
     -- which runs on its own capture stream -- allocates its workspace from the graph's private pool: the graph
     then owns the buffer its kernels have baked in, and nothing an eager call does later (a larger batch, another
     method) can free or reuse it under a replay.  A buffer that must grow is replaced, never resized in place;
     `GraphedTrainStep` additionally pins the buffers that were live when it captured."""
+    det = _sync_deterministic()   # (the deterministic mode's backward layouts carry partial-sum scratch)
     n = _lib.lib().odevit_workspace_bytes(ctypes.byref(desc), kind, method)
     if n == 0:
         _lib.check(-1, "odevit_workspace_bytes")
     dev = device.index if device.index is not None else torch.cuda.current_device()
-    key = (dev, kind, int(torch.cuda.current_stream(device).cuda_stream))
+    key = (dev, kind, int(torch.cuda.current_stream(device).cuda_stream), det)
     buf = _WS_CACHE.get(key)
     if buf is None or buf.numel() < n + 1024:
         buf = torch.empty(int(n * 1.05) + 2048, dtype=torch.uint8, device=device)
@@ -186,7 +187,23 @@ def _aligned(buf: Optional[torch.Tensor]):
     return _vp(al), buf.numel() - (al - base)
 
 
+_DETERMINISTIC = [False]   # what the library was last told
+
+
+def _sync_deterministic() -> bool:
+    """Mirror torch.are_deterministic_algorithms_enabled() into the library (odevit_set_deterministic), calling the
+    setter only when the value changes.  On, the backward kernels sum their reductions in a fixed order instead of
+    through atomics: identical inputs give bitwise-identical gradients (same build, GPU model and SM count)."""
+    on = torch.are_deterministic_algorithms_enabled()
+    if on != _DETERMINISTIC[0]:
+        _lib.check(_lib.lib().odevit_set_deterministic(int(on)), "odevit_set_deterministic")
+        _DETERMINISTIC[0] = on
+    return on
+
+
 def _stream() -> _vp:
+    # every library call takes its stream from here: the place to bring the deterministic mode up to date
+    _sync_deterministic()
     return _vp(torch.cuda.current_stream().cuda_stream)
 
 
