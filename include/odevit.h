@@ -17,14 +17,15 @@
  *   odevit_solve_bwd   <-  loss.backward() through that call     train.py:57-67, loss_trainer.py:365
  *                          (reference gradient mode: autograd through the unrolled solver; here a
  *                           reverse sweep that recomputes each step from the stored trajectory row)
- *   odevit_solve_adaptive[_record] / odevit_solve_adaptive_bwd
+ *   odevit_solve_adaptive[_record|_attn] / odevit_solve_adaptive_bwd[_attn]
  *                      <-  odeint(..., method="dopri5") with the error norm taken per image, and loss.backward()
- *                          through it with the accepted steps frozen (not part of the reference)
+ *                          through it with the accepted steps frozen (not part of the reference); _attn: with
+ *                          block.attentions and the JaSMin window of attention_trajectory
  *
  * Conventions (SURVEY.md section 8b):
  *   - plain pointers and sizes only; no torch types; every device buffer, including the workspace,
  *     is owned by the caller; the library never allocates device memory and never synchronises
- *     (except odevit_solve_adaptive[_record], which cannot know its number of rounds in advance;
+ *     (except odevit_solve_adaptive[_record|_attn], which cannot know its number of rounds in advance;
  *     odevit_solve_adaptive_resident decides them on the device and does not synchronise);
  *   - all work is enqueued on `stream` and is asynchronous with respect to the host;
  *   - `t_grid` is a HOST pointer (the per-step dt = t[i+1]-t[i] is formed on the host in fp32,
@@ -152,8 +153,8 @@ typedef enum {
   ODEVIT_WS_SOLVE_FWD = 1, /* odevit_solve_fwd                                                 */
   ODEVIT_WS_SOLVE_BWD = 2, /* odevit_solve_bwd                                                 */
   ODEVIT_WS_ENCODER_FWD = 3, /* odevit_encoder_fwd (method ignored)                            */
-  ODEVIT_WS_SOLVE_ADAPTIVE = 4, /* odevit_solve_adaptive[_record] (method ignored)              */
-  ODEVIT_WS_SOLVE_ADAPTIVE_BWD = 5, /* odevit_solve_adaptive_bwd (method ignored)               */
+  ODEVIT_WS_SOLVE_ADAPTIVE = 4, /* odevit_solve_adaptive[_record|_attn] (method ignored)        */
+  ODEVIT_WS_SOLVE_ADAPTIVE_BWD = 5, /* odevit_solve_adaptive_bwd[_attn] (method ignored)        */
   ODEVIT_WS_SOLVE_ADAPTIVE_RESIDENT = 6 /* odevit_solve_adaptive_resident (method ignored)      */
 } odevit_ws_kind;
 
@@ -321,6 +322,27 @@ int odevit_solve_adaptive_record(const odevit_desc* desc, const odevit_weights* 
                                  int32_t* rejected, int32_t step_cap, double* step_t0, double* step_dt,
                                  int32_t* step_out, void* workspace, size_t workspace_bytes, odevit_stream_t stream);
 
+/* odevit_solve_adaptive_record with the attention outputs torchdiffeq's dopri5 leaves in the reference's field, taken
+ * per image.  The record is optional here: step_t0, step_dt, step_out all NULL (step_cap ignored) or all given.
+ *   p_last [B,H,N,N] fp32 device, or NULL: the map of image b's LAST field evaluation, k7 = f(y1) of its last accepted
+ *     step (t1 >= t_out[-1]; never a rejected attempt's, and not the map at the interpolated states[-1]).  Formed by one
+ *     extra evaluation at every image's end state after the last round: bitwise the in-solve map, not counted in nfe.
+ *   jas_ring [jas_window,B,H] fp32 device, or NULL (jas_count, jas_k, jas_window then ignored): the JaSMin window.
+ *     Every evaluation of image b -- f(x0), the initial-step probe when first_step <= 0, the 6 stages of every attempted
+ *     step, rejected ones included; not the identity rounds after b has finished -- writes its per-head statistic
+ *     max over query rows of log(g_1 / (g_k + 1e-12) + 1e-12) (k = 0: log(g_1 + 1e-12); as odevit_jasmin_rowmax) into
+ *     slot (e mod jas_window) of b's ring, e = its 0-based evaluation index.  jas_count [B] int32 device gets the count
+ *     (= nfe).  Image b's window, its last min(jas_window, jas_count[b]) evaluations, is therefore the first
+ *     min(jas_window, jas_count[b]) slots; slots past that are 0.  0 <= jas_k <= N, jas_window >= 1.
+ * MACARON exposes no map: p_last or jas_ring with it is ODEVIT_ERR_INVALID_ARG.  The states, counts and record are
+ * bitwise those of odevit_solve_adaptive_record.  Workspace kind ODEVIT_WS_SOLVE_ADAPTIVE. */
+int odevit_solve_adaptive_attn(const odevit_desc* desc, const odevit_weights* w, const float* x0,
+                               const float* t_out_host, int32_t n_out, double rtol, double atol, double first_step,
+                               int32_t max_num_steps, float* states, int32_t* nfe, int32_t* accepted, int32_t* rejected,
+                               int32_t step_cap, double* step_t0, double* step_dt, int32_t* step_out, float* p_last,
+                               int32_t jas_k, int32_t jas_window, float* jas_ring, int32_t* jas_count, void* workspace,
+                               size_t workspace_bytes, odevit_stream_t stream);
+
 /* Bytes of the tape of odevit_solve_adaptive_bwd for S = max accepted steps: 6 S + 1 field evaluations. */
 size_t odevit_adaptive_tape_bytes(const odevit_desc* desc, int32_t S);
 
@@ -346,6 +368,16 @@ int odevit_solve_adaptive_bwd(const odevit_desc* desc, const odevit_weights* w, 
                               const float* g_states, float* g_x0, const odevit_weight_grads* gw, float* ckpt,
                               void* tape, size_t tape_bytes, void* workspace, size_t workspace_bytes,
                               odevit_stream_t stream);
+
+/* odevit_solve_adaptive_bwd with a cotangent g_p_last [B,H,N,N] (fp32 device, required) of odevit_solve_adaptive_attn's
+ * p_last: reverse step S, the VJP of f(ckpt[S]) at every image's end state, is the VJP of that map's evaluation and
+ * takes it through its attention VJP.  PARALLEL and PARALLEL_L2 fields; MACARON has no map (ODEVIT_ERR_INVALID_ARG). */
+int odevit_solve_adaptive_bwd_attn(const odevit_desc* desc, const odevit_weights* w, const float* x0,
+                                   const float* t_out_host, int32_t n_out, const double* step_t0, const double* step_dt,
+                                   const int32_t* step_out, int32_t step_cap, const int32_t* n_steps_host,
+                                   const float* g_states, const float* g_p_last, float* g_x0,
+                                   const odevit_weight_grads* gw, float* ckpt, void* tape, size_t tape_bytes,
+                                   void* workspace, size_t workspace_bytes, odevit_stream_t stream);
 
 /* The per-image Dormand-Prince solve of odevit_solve_adaptive run inside the on-chip-state kernel: ONE launch, one
  * persistent CTA per image at a time (images dealt to CTAs as they become free), the state in shared memory, the stage

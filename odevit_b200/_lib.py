@@ -124,6 +124,12 @@ def lib() -> ctypes.CDLL:
                                                ctypes.POINTER(ctypes.c_float), ctypes.c_int32, ctypes.c_double,
                                                ctypes.c_double, ctypes.c_double, ctypes.c_int32, _vp, _vp, _vp, _vp,
                                                ctypes.c_int32, _vp, _vp, _vp, _vp, ctypes.c_size_t, _vp]
+    L.odevit_solve_adaptive_attn.restype = ctypes.c_int
+    L.odevit_solve_adaptive_attn.argtypes = [ctypes.POINTER(Desc), ctypes.POINTER(Weights), _vp,
+                                             ctypes.POINTER(ctypes.c_float), ctypes.c_int32, ctypes.c_double,
+                                             ctypes.c_double, ctypes.c_double, ctypes.c_int32, _vp, _vp, _vp, _vp,
+                                             ctypes.c_int32, _vp, _vp, _vp, _vp, ctypes.c_int32, ctypes.c_int32, _vp, _vp,
+                                             _vp, ctypes.c_size_t, _vp]
     L.odevit_solve_adaptive_resident.restype = ctypes.c_int
     L.odevit_solve_adaptive_resident.argtypes = [ctypes.POINTER(Desc), ctypes.POINTER(Weights), _vp,
                                                  ctypes.POINTER(ctypes.c_float), ctypes.c_int32, ctypes.c_double,
@@ -137,6 +143,12 @@ def lib() -> ctypes.CDLL:
                                             ctypes.c_int32, ctypes.POINTER(ctypes.c_int32), _vp, _vp,
                                             ctypes.POINTER(WeightGrads), _vp, _vp, ctypes.c_size_t, _vp,
                                             ctypes.c_size_t, _vp]
+    L.odevit_solve_adaptive_bwd_attn.restype = ctypes.c_int
+    L.odevit_solve_adaptive_bwd_attn.argtypes = [ctypes.POINTER(Desc), ctypes.POINTER(Weights), _vp,
+                                                 ctypes.POINTER(ctypes.c_float), ctypes.c_int32, _vp, _vp, _vp,
+                                                 ctypes.c_int32, ctypes.POINTER(ctypes.c_int32), _vp, _vp, _vp,
+                                                 ctypes.POINTER(WeightGrads), _vp, _vp, ctypes.c_size_t, _vp,
+                                                 ctypes.c_size_t, _vp]
     L.odevit_solve_uses_resident.restype = ctypes.c_int
     L.odevit_solve_uses_resident.argtypes = [ctypes.POINTER(Desc), ctypes.c_int32, ctypes.c_int32]
     L.odevit_tokens_fwd.restype = ctypes.c_int
@@ -217,6 +229,6 @@ def profile_read() -> dict:
 
 DECLARED_SYMBOLS = ("odevit_abi_version", "odevit_build_info", "odevit_last_error_string",
                     "odevit_workspace_bytes", "odevit_field_fwd", "odevit_solve_fwd", "odevit_solve_bwd",
-                    "odevit_field_bwd", "odevit_tape_bytes", "odevit_fd_curvature", "odevit_jasmin_rowmax", "odevit_encoder_cache_bytes", "odevit_encoder_fwd", "odevit_launch_count", "odevit_reset_launch_count", "odevit_drop_state_advance", "odevit_solve_fwd_lean", "odevit_solve_adaptive", "odevit_solve_adaptive_record", "odevit_solve_adaptive_resident", "odevit_adaptive_tape_bytes", "odevit_solve_adaptive_bwd", "odevit_solve_uses_resident", "odevit_tokens_fwd", "odevit_head_ce_fwd", "odevit_head_ce_bwd", "odevit_extract_mass_fwd", "odevit_extract_mass_bwd", "odevit_pil_bilinear_ksize", "odevit_pil_bilinear_tables", "odevit_preprocess_u8",
+                    "odevit_field_bwd", "odevit_tape_bytes", "odevit_fd_curvature", "odevit_jasmin_rowmax", "odevit_encoder_cache_bytes", "odevit_encoder_fwd", "odevit_launch_count", "odevit_reset_launch_count", "odevit_drop_state_advance", "odevit_solve_fwd_lean", "odevit_solve_adaptive", "odevit_solve_adaptive_record", "odevit_solve_adaptive_attn", "odevit_solve_adaptive_resident", "odevit_adaptive_tape_bytes", "odevit_solve_adaptive_bwd", "odevit_solve_adaptive_bwd_attn", "odevit_solve_uses_resident", "odevit_tokens_fwd", "odevit_head_ce_fwd", "odevit_head_ce_bwd", "odevit_extract_mass_fwd", "odevit_extract_mass_bwd", "odevit_pil_bilinear_ksize", "odevit_pil_bilinear_tables", "odevit_preprocess_u8",
                     "odevit_gemm_bf16", "odevit_profile_enable", "odevit_profile_reserve", "odevit_profile_num_classes", "odevit_profile_class_name",
                     "odevit_profile_read", "odevit_set_deterministic", "odevit_deterministic")

@@ -1,5 +1,5 @@
-// Adaptive Dormand-Prince 5(4) solve with per-image step control (odevit_solve_adaptive[_record]) and its reverse
-// sweep over the accepted steps (odevit_solve_adaptive_bwd).
+// Adaptive Dormand-Prince 5(4) solve with per-image step control (odevit_solve_adaptive[_record|_attn]) and its reverse
+// sweep over the accepted steps (odevit_solve_adaptive_bwd[_attn]).
 //
 // Every image b runs torchdiffeq's dopri5 (_impl/dopri5.py, rk_common.py, interp.py, misc.py) on its own N*D
 // elements: its own t, dt, error norm, accept/reject decision and dense output.  A batch of one is the published
@@ -22,6 +22,12 @@
 // The host cannot know the number of rounds: after enqueuing round r + 1 it waits for round r's active-image count
 // (copied to pinned host memory right after round r, before round r + 1's launches), so the GPU always has the next
 // round queued while the host decides.
+//
+// Attention outputs (odevit_solve_adaptive_attn), torchdiffeq's meaning taken per image: p_last[b] is the map of image
+// b's last field evaluation, k7 = f(y1) of its last accepted step (one extra evaluation at y0 after the last round
+// repeats it bit for bit); the JaSMin window of b is the statistic of b's own last min(W, nfe_b) evaluations -- f(x0),
+// the probe, the 6 stages of every attempted step, rejected ones included, not the identity rounds after b finished --
+// filed per evaluation by ad_jas_push_kernel into a ring [W, B, H].
 //
 // odevit_solve_adaptive_record also records every image's accepted steps (ad_control_kernel); odevit_solve_adaptive_bwd
 // differentiates the solve along them, frozen: it replays the steps into checkpoints (optionally onto a tape), then runs
@@ -62,6 +68,7 @@ struct AdBufs {
   double* t_out;            // [kMaxOut]
   int *accept, *attempts, *n_acc, *n_rej;   // [B]
   int* sync;                // [4]
+  float* jas;               // [B, H] JaSMin statistic of one evaluation
 };
 
 AdBufs layout_adaptive(const Plan& p, Arena& a) {
@@ -89,6 +96,7 @@ AdBufs layout_adaptive(const Plan& p, Arena& a) {
   f.n_rej = f.accept ? f.accept + 3 * p.B : nullptr;
   f.sync = reinterpret_cast<int*>(a.take(16));
   split_scratch(p, a);
+  f.jas = a.f32((size_t)p.B * p.H);
   return f;
 }
 
@@ -102,6 +110,19 @@ __global__ void ad_init_kernel(double* t, double* dt, int* out_next, int* counte
   dt[b] = first_step;     // <= 0: replaced by the initial-step selection
   out_next[b] = 1;
   for (int i = 0; i < 4; ++i) counters[i * B + b] = 0;
+}
+
+// JaSMin window: the statistic of one evaluation (jas [B, H]) goes to slot count[b] mod W of image b's ring [W, B, H],
+// then count[b] += 1 -- for the images that took part in it: all (dt == null: f(x0), the probe) or those with dt_b != 0
+// (a round's stages; a finished image's identity rounds are not evaluations of it).
+__global__ void ad_jas_push_kernel(const float* __restrict__ jas, const double* dt, float* ring, int* count, int B,
+                                   int H, int W) {
+  const int b = blockIdx.x * blockDim.x + threadIdx.x;
+  if (b >= B || (dt && dt[b] == 0.0)) return;
+  const int c = count[b];
+  float* dst = ring + ((long long)(c % W) * B + b) * H;
+  for (int h = 0; h < H; ++h) dst[h] = jas[(long long)b * H + h];
+  count[b] = c + 1;
 }
 
 enum { RS_INIT = 0, RS_D2 = 1, RS_ERR = 2 };
@@ -352,26 +373,44 @@ int row_axpy(const Plan& p, const float* y0, const float* v, float c, const doub
   return rk_apply_rows(e, v, p.M, p.D, s);
 }
 
-// f(u) -> out (plain store)
-int eval_plain(const Plan& p, AdBufs& f, const float* u, float* out, cudaStream_t s) {
+// The JaSMin window of the forward solve: every evaluation forms its statistic in `tmp` (inside the fused attention
+// kernel, else from the exported map: attention_forward) and push() files it in the evaluating images' rings.
+struct JasWindow {
+  float* tmp;
+  float* ring;   // [W, B, H]
+  int* count;    // [B]
+  int k, W, B, H;
+  int push(const double* dt, cudaStream_t s) const {
+    ad_jas_push_kernel<<<(B + 127) / 128, 128, 0, s>>>(tmp, dt, ring, count, B, H, W);
+    ODV_LAUNCH_CHECK();
+    return 0;
+  }
+};
+
+// f(u) -> out (plain store); with a window, filed for the images with dt_b != 0 (dt == null: all)
+int eval_plain(const Plan& p, AdBufs& f, const float* u, float* out, cudaStream_t s, const JasWindow* jw = nullptr,
+               const double* dt = nullptr) {
   Epi e;
   e.out = out; e.c_new = 1.f;
-  return eval_forward(p, f.w, f.ctx, u, f.P, nullptr, f.sq, nullptr, 0, &e, s);
+  ODV_TRY(eval_forward(p, f.w, f.ctx, u, f.P, nullptr, f.sq, nullptr, 0, &e, s, jw ? jw->tmp : nullptr, jw ? jw->k : 0));
+  return jw ? jw->push(dt, s) : 0;
 }
 
 // The stages k2..k6 of one step of every image from y0 and k[0] = k1 (FSAL): u2 by a row pass, then the evaluation of
 // u_{m+1} stores k_{m+1} and its epilogue forms u_{m+2} in u (y1 after k6).  ctx(m): the intermediates of that
-// evaluation.  y1 == nullptr recomputes the intermediates only: k6's output GEMM is skipped.
+// evaluation.  y1 == nullptr recomputes the intermediates only: k6's output GEMM is skipped.  jw: the forward solve's
+// JaSMin window (null in the reverse sweep).
 template <class Ctx>
 int dp_stages(const Plan& p, const WeightBufs& w, Ctx ctx, float* P, float* sq, const float* y0, float* const* k,
-              const double* dt, float* u, float* y1, cudaStream_t s) {
+              const double* dt, float* u, float* y1, cudaStream_t s, const JasWindow* jw = nullptr) {
   ODV_TRY(row_axpy(p, y0, k[0], kDopri5.a[1][0], dt, u, s));
   for (int m = 1; m <= 5; ++m) {
     if (!y1 && m == 5) return eval_forward(p, w, ctx(m), u, P, nullptr, sq, nullptr, 0, nullptr, s);
     Epi e = rk_epilogue(kDopri5, m, 1.f, y0, k, m == 5 ? y1 : u);   // dt_b is applied per image in the epilogue
     e.row_dt = dt; e.rows_per_image = p.N;
     e.k_store = k[m];
-    ODV_TRY(eval_forward(p, w, ctx(m), u, P, nullptr, sq, nullptr, 0, &e, s));
+    ODV_TRY(eval_forward(p, w, ctx(m), u, P, nullptr, sq, nullptr, 0, &e, s, jw ? jw->tmp : nullptr, jw ? jw->k : 0));
+    if (jw) ODV_TRY(jw->push(dt, s));
   }
   return 0;
 }
@@ -463,14 +502,33 @@ struct StepRecord {
   int cap = 0;
 };
 
+// The attention outputs of odevit_solve_adaptive_attn (all null: none).
+struct AttnOut {
+  float* p_last = nullptr;    // [B, H, N, N]
+  float* ring = nullptr;      // [W, B, H]
+  int32_t* count = nullptr;   // [B]
+  int k = 0, window = 0;
+};
+
 int solve_adaptive_impl(const odevit_desc* desc, const odevit_weights* w, const float* x0, const float* t_out_host,
                         int32_t n_out, double rtol, double atol, double first_step, int32_t max_num_steps,
                         float* states, int32_t* nfe, int32_t* accepted, int32_t* rejected, const StepRecord& rec,
-                        void* workspace, size_t workspace_bytes, odevit_stream_t stream) {
+                        const AttnOut& at, void* workspace, size_t workspace_bytes, odevit_stream_t stream) {
   Plan p{};
   ODV_TRY(make_plan(desc, &p));
   ODV_TRY(check_weights(p, w));
   if (p.any_drop) return set_error(ODEVIT_ERR_INVALID_ARG, "the adaptive solve is inference-only: dropout must be 0");
+  if ((at.p_last || at.ring) && p.variant == ODEVIT_FIELD_MACARON)
+    return set_error(ODEVIT_ERR_INVALID_ARG, "MACARON exposes no attention map (need_weights=False, macaron.py:60-65)");
+  if (at.p_last) ODV_TRY(check_device_ptr(at.p_last, "p_last"));
+  if (at.ring) {
+    ODV_TRY(check_device_ptr(at.ring, "jas_ring"));
+    if (!at.count) return set_error(ODEVIT_ERR_INVALID_ARG, "jas_count is NULL");
+    ODV_TRY(check_device_ptr(at.count, "jas_count"));
+    if (at.k < 0 || at.k > p.N || at.window < 1)
+      return set_error(ODEVIT_ERR_INVALID_ARG, "jas_k %d (0..tokens) / jas_window %d (>= 1) out of range", at.k,
+                       at.window);
+  }
   ODV_TRY(check_device_ptr(x0, "x0"));
   ODV_TRY(check_device_ptr(states, "states"));
   if (nfe) ODV_TRY(check_device_ptr(nfe, "nfe"));
@@ -514,10 +572,16 @@ int solve_adaptive_impl(const odevit_desc* desc, const odevit_weights* w, const 
     ODV_CUDA(cudaMemsetAsync(rec.dt, 0, n * 8, s));
     ODV_CUDA(cudaMemsetAsync(rec.out, 0, n * 4, s));
   }
+  const JasWindow jas{f.jas, at.ring, at.count, at.k, at.window, B, p.H};
+  const JasWindow* jw = at.ring ? &jas : nullptr;
+  if (jw) {
+    ODV_CUDA(cudaMemsetAsync(at.ring, 0, (size_t)at.window * B * p.H * 4, s));
+    ODV_CUDA(cudaMemsetAsync(at.count, 0, (size_t)B * 4, s));
+  }
   ad_init_kernel<<<(B + 255) / 256, 256, 0, s>>>(f.t, f.dt, f.out_next, f.accept, f.sync, f.t_out,
                                                   first_step > 0 ? first_step : 0.0, B);
   ODV_LAUNCH_CHECK();
-  ODV_TRY(eval_plain(p, f, f.y0, f.k[0], s));   // f0
+  ODV_TRY(eval_plain(p, f, f.y0, f.k[0], s, jw));   // f0
   const int row_blocks = (p.M + 7) / 8;
   if (!(first_step > 0)) {
     ad_rowsq_kernel<RS_INIT><<<row_blocks, 256, 0, s>>>(f.y0, nullptr, f.k[0], nullptr, nullptr, nullptr, nullptr,
@@ -526,7 +590,7 @@ int solve_adaptive_impl(const odevit_desc* desc, const odevit_weights* w, const 
     ad_init_step_kernel<<<B, kRedThreads, 0, s>>>(0, f.row0, f.row1, N, D, f.h0, f.d1, f.dt);
     ODV_LAUNCH_CHECK();
     ODV_TRY(row_axpy(p, f.y0, f.k[0], 1.f, f.h0, f.u, s));   // probe y0 + h0 f0
-    ODV_TRY(eval_plain(p, f, f.u, f.k[1], s));
+    ODV_TRY(eval_plain(p, f, f.u, f.k[1], s, jw));
     ad_rowsq_kernel<RS_D2><<<row_blocks, 256, 0, s>>>(f.y0, nullptr, f.k[0], f.k[1], nullptr, nullptr, nullptr, nullptr,
                                                      nullptr, nullptr, frtol, fatol, p.M, N, D, f.row0, nullptr);
     ODV_LAUNCH_CHECK();
@@ -540,8 +604,8 @@ int solve_adaptive_impl(const odevit_desc* desc, const odevit_weights* w, const 
     const int c = (int)(r & 1), n = c ^ 1;
     const double* dt = f.dt + (size_t)c * B;
     ODV_CUDA(cudaMemsetAsync(f.sync + c, 0, sizeof(int), s));
-    ODV_TRY(dp_stages(p, f.w, [&](int) { return f.ctx; }, f.P, f.sq, f.y0, f.k, dt, f.u, f.y1, s));
-    ODV_TRY(eval_plain(p, f, f.y1, f.k[6], s));   // k7 = f(y1)
+    ODV_TRY(dp_stages(p, f.w, [&](int) { return f.ctx; }, f.P, f.sq, f.y0, f.k, dt, f.u, f.y1, s, jw));
+    ODV_TRY(eval_plain(p, f, f.y1, f.k[6], s, jw, dt));   // k7 = f(y1)
     ad_rowsq_kernel<RS_ERR><<<row_blocks, 256, 0, s>>>(f.y0, f.y1, f.k[0], nullptr, f.k[2], f.k[3], f.k[4], f.k[5],
                                                        f.k[6], dt, frtol, fatol, p.M, N, D, f.row0, nullptr);
     ODV_LAUNCH_CHECK();
@@ -589,6 +653,10 @@ int solve_adaptive_impl(const odevit_desc* desc, const odevit_weights* w, const 
       return set_error(ODEVIT_ERR_CUDA, "adaptive solve: %d images still active after %lld rounds", active, r + 1);
     }
   }
+  // block.attentions is the map of each image's last evaluation, k7 = f(y1) of its last accepted step; y0 holds that y1
+  // (finished images repeat it).  The forward's kernels have no order-dependent reduction, so this evaluation repeats
+  // that map bit for bit.  It is not counted in nfe and not filed in the window.
+  if (at.p_last) ODV_TRY(eval_forward(p, f.w, f.ctx, f.y0, f.P, at.p_last, f.sq, nullptr, 0, nullptr, s));
   return 0;
 }
 }  // namespace
@@ -599,7 +667,7 @@ extern "C" int odevit_solve_adaptive(const odevit_desc* desc, const odevit_weigh
                                      int32_t* accepted, int32_t* rejected, void* workspace, size_t workspace_bytes,
                                      odevit_stream_t stream) {
   return solve_adaptive_impl(desc, w, x0, t_out_host, n_out, rtol, atol, first_step, max_num_steps, states, nfe,
-                             accepted, rejected, StepRecord{}, workspace, workspace_bytes, stream);
+                             accepted, rejected, StepRecord{}, AttnOut{}, workspace, workspace_bytes, stream);
 }
 
 extern "C" int odevit_solve_adaptive_record(const odevit_desc* desc, const odevit_weights* w, const float* x0,
@@ -612,7 +680,27 @@ extern "C" int odevit_solve_adaptive_record(const odevit_desc* desc, const odevi
   StepRecord rec;
   rec.t0 = step_t0; rec.dt = step_dt; rec.out = step_out; rec.cap = step_cap;
   return solve_adaptive_impl(desc, w, x0, t_out_host, n_out, rtol, atol, first_step, max_num_steps, states, nfe,
-                             accepted, rejected, rec, workspace, workspace_bytes, stream);
+                             accepted, rejected, rec, AttnOut{}, workspace, workspace_bytes, stream);
+}
+
+extern "C" int odevit_solve_adaptive_attn(const odevit_desc* desc, const odevit_weights* w, const float* x0,
+                                          const float* t_out_host, int32_t n_out, double rtol, double atol,
+                                          double first_step, int32_t max_num_steps, float* states, int32_t* nfe,
+                                          int32_t* accepted, int32_t* rejected, int32_t step_cap, double* step_t0,
+                                          double* step_dt, int32_t* step_out, float* p_last, int32_t jas_k,
+                                          int32_t jas_window, float* jas_ring, int32_t* jas_count, void* workspace,
+                                          size_t workspace_bytes, odevit_stream_t stream) {
+  StepRecord rec;
+  if (step_t0 || step_dt || step_out) {
+    if (!step_t0 || !step_dt || !step_out)
+      return set_error(ODEVIT_ERR_INVALID_ARG, "step_t0 / step_dt / step_out: give all three or none");
+    rec.t0 = step_t0; rec.dt = step_dt; rec.out = step_out; rec.cap = step_cap;
+  }
+  AttnOut at;
+  at.p_last = p_last;
+  at.ring = jas_ring; at.count = jas_count; at.k = jas_k; at.window = jas_window;
+  return solve_adaptive_impl(desc, w, x0, t_out_host, n_out, rtol, atol, first_step, max_num_steps, states, nfe,
+                             accepted, rejected, rec, at, workspace, workspace_bytes, stream);
 }
 
 namespace {
@@ -689,17 +777,23 @@ extern "C" size_t odevit_adaptive_tape_bytes(const odevit_desc* desc, int32_t S)
 //   VJP of f(ckpt[s]) with lambda_1 + g_k7 of step s - 1 (the same evaluation):  G <- G + sum mu + g of row s
 // where the g_* are the dense output's cotangents (ad_interp_vjp_kernel).  Reverse step S is that last VJP alone, at each
 // image's end state.  A finished image has dt_b = 0 and no outputs in its remaining steps: lambda = 0 there.
-extern "C" int odevit_solve_adaptive_bwd(const odevit_desc* desc, const odevit_weights* w, const float* x0,
-                                         const float* t_out_host, int32_t n_out, const double* step_t0,
-                                         const double* step_dt, const int32_t* step_out, int32_t step_cap,
-                                         const int32_t* n_steps_host, const float* g_states, float* g_x0,
-                                         const odevit_weight_grads* gw, float* ckpt, void* tape, size_t tape_bytes,
-                                         void* workspace, size_t workspace_bytes, odevit_stream_t stream) {
+// f(ckpt[S]) is also the evaluation whose map is p_last (each image's last one): g_p_last enters its attention VJP.
+namespace {
+int solve_adaptive_bwd_impl(const odevit_desc* desc, const odevit_weights* w, const float* x0, const float* t_out_host,
+                            int32_t n_out, const double* step_t0, const double* step_dt, const int32_t* step_out,
+                            int32_t step_cap, const int32_t* n_steps_host, const float* g_states,
+                            const float* g_p_last, float* g_x0, const odevit_weight_grads* gw, float* ckpt, void* tape,
+                            size_t tape_bytes, void* workspace, size_t workspace_bytes, odevit_stream_t stream) {
   Plan p{};
   ODV_TRY(make_plan(desc, &p));
   ODV_TRY(check_weights(p, w));
   if (p.any_drop) return set_error(ODEVIT_ERR_INVALID_ARG, "the adaptive solve has no dropout: dropout must be 0");
   if (!gw) return set_error(ODEVIT_ERR_INVALID_ARG, "weight-gradient struct is NULL");
+  if (g_p_last) {
+    if (p.variant == ODEVIT_FIELD_MACARON)
+      return set_error(ODEVIT_ERR_INVALID_ARG, "MACARON exposes no attention map (need_weights=False, macaron.py:60-65)");
+    ODV_TRY(check_device_ptr(g_p_last, "g_p_last"));
+  }
   ODV_TRY(check_device_ptr(x0, "x0"));
   ODV_TRY(check_device_ptr(g_states, "g_states"));
   ODV_TRY(check_device_ptr(g_x0, "g_x0"));
@@ -784,7 +878,7 @@ extern "C" int odevit_solve_adaptive_bwd(const odevit_desc* desc, const odevit_w
   {   // reverse step S: f(ckpt[S]) alone, G <- G + its mu + g of row S
     Epi e = rk_vjp_row_epilogue(G, f.mu, 0, &f.cot[S & 1].y, 1, G);
     e.aux_type = p.dd_type;
-    ODV_TRY(eval_vjp(p, b.w, ctx_of(S, 0), b, nullptr, need_c2, gw, 6LL * S, e, s));
+    ODV_TRY(eval_vjp(p, b.w, ctx_of(S, 0), b, g_p_last, need_c2, gw, 6LL * S, e, s));
   }
   for (int st = S - 1; st >= 0; --st) {
     ODV_TRY(seed(f.cot[st & 1].k[3], tb.b[5], dt_of(st)));   // lambda_6
@@ -802,4 +896,27 @@ extern "C" int odevit_solve_adaptive_bwd(const odevit_desc* desc, const odevit_w
                         rk_vjp_row_epilogue(G, f.mu, 5, &cot.y, 1, st == 0 ? g_x0 : G), s));
   }
   return finish_grads(p, w, gw, b, s);
+}
+}  // namespace
+
+extern "C" int odevit_solve_adaptive_bwd(const odevit_desc* desc, const odevit_weights* w, const float* x0,
+                                         const float* t_out_host, int32_t n_out, const double* step_t0,
+                                         const double* step_dt, const int32_t* step_out, int32_t step_cap,
+                                         const int32_t* n_steps_host, const float* g_states, float* g_x0,
+                                         const odevit_weight_grads* gw, float* ckpt, void* tape, size_t tape_bytes,
+                                         void* workspace, size_t workspace_bytes, odevit_stream_t stream) {
+  return solve_adaptive_bwd_impl(desc, w, x0, t_out_host, n_out, step_t0, step_dt, step_out, step_cap, n_steps_host,
+                                 g_states, nullptr, g_x0, gw, ckpt, tape, tape_bytes, workspace, workspace_bytes, stream);
+}
+
+extern "C" int odevit_solve_adaptive_bwd_attn(const odevit_desc* desc, const odevit_weights* w, const float* x0,
+                                              const float* t_out_host, int32_t n_out, const double* step_t0,
+                                              const double* step_dt, const int32_t* step_out, int32_t step_cap,
+                                              const int32_t* n_steps_host, const float* g_states,
+                                              const float* g_p_last, float* g_x0, const odevit_weight_grads* gw,
+                                              float* ckpt, void* tape, size_t tape_bytes, void* workspace,
+                                              size_t workspace_bytes, odevit_stream_t stream) {
+  if (!g_p_last) return set_error(ODEVIT_ERR_INVALID_ARG, "g_p_last is NULL (odevit_solve_adaptive_bwd takes none)");
+  return solve_adaptive_bwd_impl(desc, w, x0, t_out_host, n_out, step_t0, step_dt, step_out, step_cap, n_steps_host,
+                                 g_states, g_p_last, g_x0, gw, ckpt, tape, tape_bytes, workspace, workspace_bytes, stream);
 }

@@ -544,9 +544,27 @@ DOPRI5_MAX_NUM_STEPS = 2 ** 31 - 1   # torchdiffeq's default
 ADAPTIVE_STEP_CAP = 1024   # first size of the accepted-step record of a differentiable adaptive solve (grown 4x on demand)
 
 
+def _adaptive_attn_outputs(x0, spec: FieldSpec, want_p_last: bool, jasmin: Optional[Tuple[int, int]]):
+    """The attention outputs of an adaptive solve: (p_last [B,H,N,N] | None, (jas_ring [W,B,H], jas_count [B] int32, W,
+    k) | None) for jasmin = (W, k)."""
+    B, N, _ = x0.shape
+    if (want_p_last or jasmin is not None) and spec.variant == _lib.FIELD_MACARON:
+        raise OdevitError("MACARON exposes no attention map (macaron.py:60-65): no p_last / JaSMin window")
+    p_last = torch.empty(B, spec.heads, N, N, device=x0.device, dtype=torch.float32) if want_p_last else None
+    jas = None
+    if jasmin is not None:
+        W, k = int(jasmin[0]), int(jasmin[1])
+        if W < 1:
+            raise ValueError(f"jasmin window must be >= 1, got {W}")
+        jas = (torch.empty(W, B, spec.heads, device=x0.device, dtype=torch.float32),
+               torch.empty(B, device=x0.device, dtype=torch.int32), W, k)
+    return p_last, jas
+
+
 def _adaptive_call(x0, t_c, T: int, spec: FieldSpec, names, weights, rtol: float, atol: float, fs: float,
-                   max_num_steps: int, record=None):
-    """One odevit_solve_adaptive call, or odevit_solve_adaptive_record with record = (cap, t0, dt, out).
+                   max_num_steps: int, record=None, attn=None):
+    """One odevit_solve_adaptive call, or odevit_solve_adaptive_record with record = (cap, t0, dt, out), or, with
+    attn = (p_last | None, jas | None) from _adaptive_attn_outputs, odevit_solve_adaptive_attn (record optional).
     Returns (status, states [T,B,N,D], counts [3,B] int32 = nfe, accepted, rejected)."""
     B, N, D = x0.shape
     desc = spec.desc(B, N)
@@ -555,7 +573,16 @@ def _adaptive_call(x0, t_c, T: int, spec: FieldSpec, names, weights, rtol: float
     counts = torch.zeros(3, B, device=x0.device, dtype=torch.int32)
     buf, ws, ws_bytes = _workspace(desc, _lib.WS_SOLVE_ADAPTIVE, 0, x0.device)
     with torch.cuda.device(x0.device):
-        if record is None:
+        if attn is not None:
+            p_last, jas = attn
+            cap, t0, dt, out = record if record is not None else (0, None, None, None)
+            ring, jcount, W, k = jas if jas is not None else (None, None, 0, 0)
+            st = _lib.lib().odevit_solve_adaptive_attn(ctypes.byref(desc), ctypes.byref(w), _ptr(x0), t_c, T,
+                                                       float(rtol), float(atol), fs, int(max_num_steps), _ptr(states),
+                                                       _ptr(counts[0]), _ptr(counts[1]), _ptr(counts[2]), int(cap),
+                                                       _ptr(t0), _ptr(dt), _ptr(out), _ptr(p_last), int(k), int(W),
+                                                       _ptr(ring), _ptr(jcount), ws, ws_bytes, _stream())
+        elif record is None:
             st = _lib.lib().odevit_solve_adaptive(ctypes.byref(desc), ctypes.byref(w), _ptr(x0), t_c, T, float(rtol),
                                                   float(atol), fs, int(max_num_steps), _ptr(states), _ptr(counts[0]),
                                                   _ptr(counts[1]), _ptr(counts[2]), ws, ws_bytes, _stream())
@@ -599,20 +626,24 @@ def _adaptive_check(st: int, what: str) -> None:
 
 
 class _AdaptiveSolve(torch.autograd.Function):
-    """(states, counts) = the adaptive solve of x0; its backward is odevit_solve_adaptive_bwd over the accepted steps
-    the forward recorded (frozen: the step sizes, the output times' positions in them and the rejected attempts carry
-    no gradient)."""
+    """(states, counts, p_last, jas_ring, jas_count) = the adaptive solve of x0; its backward is
+    odevit_solve_adaptive_bwd (odevit_solve_adaptive_bwd_attn with a cotangent of p_last) over the accepted steps the
+    forward recorded (frozen: the step sizes, the output times' positions in them and the rejected attempts carry no
+    gradient).  p_last, jas_ring, jas_count are empty unless asked for (want_p_last, jasmin); the window is not
+    differentiable."""
 
     @staticmethod
     def forward(ctx, x0, spec: FieldSpec, t_c, T: int, rtol: float, atol: float, fs: float, max_num_steps: int,
-                names: Tuple[str, ...], *weights):
+                want_p_last: bool, jasmin: Optional[Tuple[int, int]], names: Tuple[str, ...], *weights):
         B = x0.shape[0]
         cap = max(1, min(int(max_num_steps), int(ADAPTIVE_STEP_CAP)))
         while True:
             rec = (cap, torch.empty(cap, B, device=x0.device, dtype=torch.float64),
                    torch.empty(cap, B, device=x0.device, dtype=torch.float64),
                    torch.empty(cap, B, device=x0.device, dtype=torch.int32))
-            st, states, counts = _adaptive_call(x0, t_c, T, spec, names, weights, rtol, atol, fs, max_num_steps, rec)
+            attn = _adaptive_attn_outputs(x0, spec, want_p_last, jasmin) if (want_p_last or jasmin) else None
+            st, states, counts = _adaptive_call(x0, t_c, T, spec, names, weights, rtol, atol, fs, max_num_steps, rec,
+                                                attn)
             # a full record: the solve is deterministic, so a larger one gives the same result
             if st == _lib.ERR_WORKSPACE and cap < max_num_steps and b"step record" in _lib.lib().odevit_last_error_string():
                 cap = min(4 * cap, int(max_num_steps))
@@ -622,18 +653,26 @@ class _AdaptiveSolve(torch.autograd.Function):
         ctx.spec, ctx.names, ctx.t_c, ctx.T, ctx.cap = spec, names, t_c, T, cap
         ctx.n_steps = counts[1].cpu().tolist()   # (the solve has synchronised already)
         ctx.save_for_backward(x0, rec[1], rec[2], rec[3], *weights)
-        ctx.mark_non_differentiable(counts)
+        empty = x0.new_empty(0)
+        p_last, jas = attn if attn is not None else (None, None)
+        ctx.has_p_last = p_last is not None
+        ring, jcount = (jas[0], jas[1]) if jas is not None else (empty, empty.int())
+        ctx.mark_non_differentiable(counts, ring, jcount)
         ctx.set_materialize_grads(False)
-        return states, counts
+        return states, counts, (p_last if p_last is not None else empty), ring, jcount
 
     @staticmethod
-    def backward(ctx, g_states, _g_counts):
+    def backward(ctx, g_states, _g_counts, g_p_last, _g_ring, _g_jcount):
         x0, step_t0, step_dt, step_out, *weights = ctx.saved_tensors
         spec, names = ctx.spec, ctx.names
         B, N, D = x0.shape
+        if g_p_last is not None and (not ctx.has_p_last or g_p_last.numel() == 0):
+            g_p_last = None
+        if g_states is None and g_p_last is None:
+            return (None,) * (11 + len(weights))
+        gw, gts = _alloc_grads(names, weights, ctx.needs_input_grad[11:])
         if g_states is None:
-            return (None,) * (9 + len(weights))
-        gw, gts = _alloc_grads(names, weights, ctx.needs_input_grad[9:])
+            g_states = torch.zeros(ctx.T, B, N, D, device=x0.device, dtype=torch.float32)
         g_states = _require_cuda(g_states, "g_states")
         desc = spec.desc(B, N)
         w, keep = _pack_weights(names, weights)
@@ -645,19 +684,28 @@ class _AdaptiveSolve(torch.autograd.Function):
         n_c = (ctypes.c_int32 * B)(*ctx.n_steps)
         buf, ws, ws_bytes = _workspace(desc, _lib.WS_SOLVE_ADAPTIVE_BWD, 0, x0.device)
         with torch.cuda.device(x0.device):
-            st = _lib.lib().odevit_solve_adaptive_bwd(ctypes.byref(desc), ctypes.byref(w), _ptr(x0), ctx.t_c, ctx.T,
-                                                      _vp(step_t0.data_ptr()), _vp(step_dt.data_ptr()),
-                                                      _vp(step_out.data_ptr()), ctx.cap, n_c, _ptr(g_states),
-                                                      _ptr(g_x0), ctypes.byref(gw), _ptr(ckpt), tape_p, tape_n, ws,
-                                                      ws_bytes, _stream())
+            if g_p_last is None:
+                st = _lib.lib().odevit_solve_adaptive_bwd(ctypes.byref(desc), ctypes.byref(w), _ptr(x0), ctx.t_c, ctx.T,
+                                                          _vp(step_t0.data_ptr()), _vp(step_dt.data_ptr()),
+                                                          _vp(step_out.data_ptr()), ctx.cap, n_c, _ptr(g_states),
+                                                          _ptr(g_x0), ctypes.byref(gw), _ptr(ckpt), tape_p, tape_n, ws,
+                                                          ws_bytes, _stream())
+            else:
+                g_p_last = _require_cuda(g_p_last, "g_p_last")
+                st = _lib.lib().odevit_solve_adaptive_bwd_attn(ctypes.byref(desc), ctypes.byref(w), _ptr(x0), ctx.t_c,
+                                                               ctx.T, _vp(step_t0.data_ptr()), _vp(step_dt.data_ptr()),
+                                                               _vp(step_out.data_ptr()), ctx.cap, n_c, _ptr(g_states),
+                                                               _ptr(g_p_last), _ptr(g_x0), ctypes.byref(gw),
+                                                               _ptr(ckpt), tape_p, tape_n, ws, ws_bytes, _stream())
         _lib.check(st, "odevit_solve_adaptive_bwd")
-        return (g_x0 if ctx.needs_input_grad[0] else None,) + (None,) * 8 + tuple(gts)
+        return (g_x0 if ctx.needs_input_grad[0] else None,) + (None,) * 10 + tuple(gts)
 
 
 def ode_solve_adaptive(x0: torch.Tensor, t: torch.Tensor, spec: FieldSpec, weights: Dict[str, Optional[torch.Tensor]],
                        rtol: float, atol: float, first_step: Optional[float] = None,
                        max_num_steps: int = DOPRI5_MAX_NUM_STEPS, differentiable: bool = False,
-                       capturable: bool = False):
+                       capturable: bool = False, want_p_last: bool = False,
+                       jasmin: Optional[Tuple[int, int]] = None):
     """Adaptive Dormand-Prince 5(4) solve with per-image step control (odevit_solve_adaptive).
 
     torchdiffeq's dopri5 run on every image on its own: the error norm, the accept / reject decisions, the step sizes
@@ -679,10 +727,21 @@ def ode_solve_adaptive(x0: torch.Tensor, t: torch.Tensor, spec: FieldSpec, weigh
     only: anything else raises, it never falls back to the synchronising solve.  This is a different contract, not a
     faster setting: the default path is the forward of the differentiable solve and raises at the first failure.
 
+    want_p_last: also `p_last` [B,H,N,N], the attention map of each image's LAST field evaluation (k7 = f(y1) of its last
+    accepted step, torchdiffeq's `block.attentions`), differentiable with differentiable=True.
+    jasmin=(W, k): also the JaSMin window of every image's own last min(W, nfe_b) evaluations (f(x0), the initial-step
+    probe and the 6 stages of every attempted step count, rejected ones included): `jas_ring` [W,B,H], image b's window
+    in slots [0, min(W, jas_count[b])) (evaluation e in slot e mod W), and `jas_count` [B] (= nfe); not differentiable.
+    Neither is built with capturable=True, nor for the MACARON field (it exposes no map).
+
     Returns dict(states [len(t),B,N,D] (row i = solution at t[i]), final [B,N,D], nfe [B], accepted [B], rejected [B]
     (int32, device), rounds (int: rounds with at least one image still stepping = max_b accepted + rejected; with
-    capturable=True a 0-d device tensor) and, with capturable=True, status [B] (int32, device))."""
+    capturable=True a 0-d device tensor), with capturable=True status [B] (int32, device), and the requested attention
+    outputs)."""
     names = tuple(k for k, v in weights.items() if v is not None)
+    if capturable and (want_p_last or jasmin is not None):
+        raise OdevitError("attention outputs (p_last, the JaSMin window) are not built for capturable=True: the on-chip "
+                          "adaptive solve exports no maps")
     if capturable:
         return _ode_solve_adaptive_capturable(x0, t, spec, weights, names, rtol, atol, first_step, max_num_steps,
                                               differentiable)
@@ -700,18 +759,40 @@ def ode_solve_adaptive(x0: torch.Tensor, t: torch.Tensor, spec: FieldSpec, weigh
     fs = 0.0 if first_step is None else float(first_step)
     if first_step is not None and not fs > 0:
         raise ValueError(f"first_step must be > 0, got {first_step}")
+    jasmin = (int(jasmin[0]), int(jasmin[1])) if jasmin is not None else None
+    res = {}
     if track:
         x0 = _require_cuda(x0, "x0")
-        states, counts = _AdaptiveSolve.apply(x0, spec, t_c, T, float(rtol), float(atol), fs, int(max_num_steps),
-                                              names, *[weights[k] for k in names])
+        states, counts, p_last, ring, jcount = _AdaptiveSolve.apply(
+            x0, spec, t_c, T, float(rtol), float(atol), fs, int(max_num_steps), bool(want_p_last), jasmin, names,
+            *[weights[k] for k in names])
+        if want_p_last:
+            res["p_last"] = p_last
+        if jasmin is not None:
+            res["jas_ring"], res["jas_count"] = ring, jcount
     else:
         x0 = _require_cuda(x0.detach(), "x0")
+        attn = _adaptive_attn_outputs(x0, spec, want_p_last, jasmin) if (want_p_last or jasmin is not None) else None
         st, states, counts = _adaptive_call(x0, t_c, T, spec, names, [weights[k].detach() for k in names], rtol, atol,
-                                            fs, max_num_steps)
+                                            fs, max_num_steps, attn=attn)
         _adaptive_check(st, "odevit_solve_adaptive")
+        if want_p_last:
+            res["p_last"] = attn[0]
+        if jasmin is not None:
+            res["jas_ring"], res["jas_count"] = attn[1][0], attn[1][1]
     rounds = int((counts[1] + counts[2]).max().item())
-    return {"states": states, "final": states[-1], "nfe": counts[0], "accepted": counts[1], "rejected": counts[2],
-            "rounds": rounds}
+    res.update({"states": states, "final": states[-1], "nfe": counts[0], "accepted": counts[1], "rejected": counts[2],
+                "rounds": rounds})
+    return res
+
+
+def adaptive_jasmin_mean(jas_ring: torch.Tensor, jas_count: torch.Tensor) -> torch.Tensor:
+    """Per image b: the mean of the JaSMin statistic over the heads and the min(W, jas_count[b]) slots of b's window
+    (ode_solve_adaptive(jasmin=(W, k))): [B], on the device, without a synchronisation."""
+    W = jas_ring.shape[0]
+    n = jas_count.clamp(max=W).to(jas_ring.dtype)
+    valid = torch.arange(W, device=jas_ring.device)[:, None] < jas_count[None, :]
+    return (jas_ring.mean(dim=2) * valid).sum(dim=0) / n
 
 
 def _ode_solve_adaptive_capturable(x0, t, spec: FieldSpec, weights, names, rtol, atol, first_step, max_num_steps,

@@ -236,12 +236,15 @@ def _check_field_module(func, who: str) -> None:
 
 def odeint_adaptive(func, y0: torch.Tensor, t: torch.Tensor, *, rtol: float = 1e-7, atol: float = 1e-9,
                     options: Optional[dict] = None, return_stats: bool = False, differentiable: bool = False,
-                    capturable: bool = False):
+                    capturable: bool = False, record_attention: bool = False):
     """`torchdiffeq.odeint(func, y0, t, method="dopri5", rtol, atol, options)` for the fused vector field, with the
     step size controlled PER IMAGE (ops.ode_solve_adaptive): image b's error norm, steps and dense output depend on
     image b alone, where torchdiffeq takes one norm over the batch.  `t` strictly increasing; options: `first_step`,
-    `max_num_steps` (attempted steps per image over the whole solve, not per output interval).  Exports no attention
-    maps.  Inference only unless `differentiable`: then the trajectory is differentiable with respect to y0 and the
+    `max_num_steps` (attempted steps per image over the whole solve, not per output interval).  `record_attention`
+    leaves `func.block.attentions` as `odeint` does: image b's row is the map of b's own last field evaluation (k7 = f(y1)
+    of its last accepted step), differentiable with `differentiable`; `func.attention_trajectory` (every evaluation's
+    map) is not built and stays as it is (a MACARON field exposes no map: ignored there, as in `odeint`).  Not with
+    `capturable`.  Inference only unless `differentiable`: then the trajectory is differentiable with respect to y0 and the
     field's weights, with each image's accepted steps frozen (not the continuous adjoint, and not autograd through an
     unrolled torchdiffeq solve).  `capturable`: the on-chip, non-synchronising form that a CUDA graph can capture
     (ops.ode_solve_adaptive; stats then also hold `status` and `rounds` is a 0-d device tensor).  Returns the trajectory
@@ -252,10 +255,14 @@ def odeint_adaptive(func, y0: torch.Tensor, t: torch.Tensor, *, rtol: float = 1e
     unknown = set(options) - {"first_step", "max_num_steps"}
     if unknown:
         raise ValueError(f"unsupported dopri5 options {sorted(unknown)}; first_step and max_num_steps are built")
+    if hasattr(func.block, "res_scale"):   # the Macaron block
+        record_attention = False
     res = ops.ode_solve_adaptive(y0, t, func.block.field_spec(func.scaler), func.block.field_weights(), rtol, atol,
                                  first_step=options.get("first_step"),
                                  max_num_steps=options.get("max_num_steps", ops.DOPRI5_MAX_NUM_STEPS),
-                                 differentiable=differentiable, capturable=capturable)
+                                 differentiable=differentiable, capturable=capturable, want_p_last=record_attention)
+    if record_attention:
+        func.block.attentions = res["p_last"]
     if return_stats:
         return res["states"], {k: res[k] for k in ("nfe", "accepted", "rejected", "rounds", "status") if k in res}
     return res["states"]
@@ -263,15 +270,26 @@ def odeint_adaptive(func, y0: torch.Tensor, t: torch.Tensor, *, rtol: float = 1e
 
 def adaptive_solve_args(model: nn.Module, output_flags: Dict[str, bool]) -> dict:
     """Checks a model's `adaptive_solve` request (a dict with rtol, atol and optionally first_step, max_num_steps,
-    differentiable, capturable) and the forward's arguments against what the adaptive solve can give."""
+    differentiable, capturable, attention_outputs) and the forward's arguments against what the adaptive solve can give.
+    `output_attentions` is honoured only when the request opts in with "attention_outputs": True -- the outputs cost one
+    extra field evaluation and one small kernel per evaluation, and a request without the key keeps refusing them."""
     cfg = dict(model.adaptive_solve)
-    unknown = set(cfg) - {"rtol", "atol", "first_step", "max_num_steps", "differentiable", "capturable"}
+    unknown = set(cfg) - {"rtol", "atol", "first_step", "max_num_steps", "differentiable", "capturable",
+                          "attention_outputs"}
     if unknown or "rtol" not in cfg or "atol" not in cfg:
-        raise ValueError(f"adaptive_solve takes rtol, atol [, first_step, max_num_steps, differentiable, capturable], "
-                         f"got {sorted(model.adaptive_solve)}")
-    for name, on in output_flags.items():
-        if on:
-            raise ValueError(f"{name} is not available with adaptive_solve (the adaptive solve exports no attention maps)")
+        raise ValueError(f"adaptive_solve takes rtol, atol [, first_step, max_num_steps, differentiable, capturable, "
+                         f"attention_outputs], got {sorted(model.adaptive_solve)}")
+    if output_flags.get("output_attention_trajectory"):
+        raise ValueError("output_attention_trajectory is not built with adaptive_solve (the per-image list of every "
+                         "evaluation's map); output_attentions is, with \"attention_outputs\": True")
+    if output_flags.get("output_attentions"):
+        if not cfg.get("attention_outputs", False):
+            raise ValueError("output_attentions with adaptive_solve needs \"attention_outputs\": True in it (each image's "
+                             "last-evaluation map and JaSMin window: one extra field evaluation and a small kernel per "
+                             "evaluation)")
+        if cfg.get("capturable", False):
+            raise ValueError("output_attentions is not built with adaptive_solve's capturable=True (the on-chip adaptive "
+                             "solve exports no maps); the default path gives it")
     if (not cfg.get("differentiable", False) and torch.is_grad_enabled()
             and any(p.requires_grad for p in model.parameters())):
         raise RuntimeError("adaptive_solve is inference-only (no backward is built): run the model under torch.no_grad()")
@@ -371,9 +389,10 @@ class ViTNeuralODE(nn.Module):
         self.time_interval = time_interval
         self.num_eval_steps = num_eval_steps
         self.t_grid = torch.linspace(0.0, time_interval, num_eval_steps)  # plain attribute, not a buffer
-        # None, or {"rtol", "atol"[, "first_step", "max_num_steps", "differentiable"]}: forward integrates over t_grid
-        # with the per-image adaptive Dormand-Prince solve (inference only unless "differentiable" is True; a plain
-        # attribute like `precision`, not a config key)
+        # None, or {"rtol", "atol"[, "first_step", "max_num_steps", "differentiable", "capturable", "attention_outputs"]}:
+        # forward integrates over t_grid with the per-image adaptive Dormand-Prince solve (inference only unless
+        # "differentiable" is True; output_attentions only with "attention_outputs": True; a plain attribute like
+        # `precision`, not a config key)
         self.adaptive_solve = None
         self.patch_embed.precision = self.odefunc.block.precision
         self.apply(self._spectral_init)
@@ -501,7 +520,7 @@ class ViTNeuralODE(nn.Module):
             num_eval_steps, t = len(t_grid), t_grid
         if self.adaptive_solve is not None:
             return self._forward_adaptive(tokens, t, num_eval_steps, cfg, labels, output_hidden_states,
-                                          output_control_points, temperature, jasmin_k)
+                                          output_control_points, output_attentions, temperature, jasmin_k)
         stages = _lib.STAGES.get(self.solver)
         if stages is None:
             raise ValueError(f"unsupported solver {self.solver!r}")
@@ -594,16 +613,20 @@ class ViTNeuralODE(nn.Module):
         return out
 
     def _forward_adaptive(self, tokens, t, num_eval_steps, cfg, labels, output_hidden_states, output_control_points,
-                          temperature, jasmin_k):
+                          output_attentions, temperature, jasmin_k):
         """forward() with `adaptive_solve` set: the trajectory over t comes from the dense output of the per-image
-        adaptive solve; the finite-difference bound is taken on it; `nfe` [B] is added to the output."""
+        adaptive solve; the finite-difference bound is taken on it; `nfe` [B] is added to the output.  With
+        output_attentions, `attentions` / `attentions_register_tokens` slice each image's last-evaluation map and
+        `jasmin_loss` is taken over each image's own window (ops.ode_solve_adaptive's want_p_last / jasmin)."""
         R = self.patch_embed.num_register_tokens
+        window = int(self.num_eval_steps * 0.85)                            # :614-618
         res = ops.ode_solve_adaptive(tokens, t, self.odefunc.block.field_spec(self.odefunc.scaler),
                                      self.odefunc.block.field_weights(), cfg["rtol"], cfg["atol"],
                                      first_step=cfg.get("first_step"),
                                      max_num_steps=cfg.get("max_num_steps", ops.DOPRI5_MAX_NUM_STEPS),
                                      differentiable=cfg.get("differentiable", False),
-                                     capturable=cfg.get("capturable", False))
+                                     capturable=cfg.get("capturable", False), want_p_last=output_attentions,
+                                     jasmin=(window, int(jasmin_k)) if (output_attentions and window > 0) else None)
         states, final = res["states"], res["final"]
         logits = self.head(final[:, 0])
         out = {
@@ -613,6 +636,18 @@ class ViTNeuralODE(nn.Module):
                 states.detach(), 0.5, 1 / self.num_eval_steps),
             "nfe": res["nfe"],
         }
+        if output_attentions:
+            # per image: its own last evaluation's map, and the JaSMin statistic over its own last min(W, nfe_b)
+            # evaluations, averaged over heads and window slots, then over images (the reference's formula when
+            # every image has the same evaluations)
+            p_last = res["p_last"]
+            self.odefunc.block.attentions = p_last
+            out["attentions"] = p_last[:, :, :-R, :-R]
+            out["attentions_register_tokens"] = p_last[:, :, -R:, :]
+            if window > 0:
+                out["jasmin_loss"] = ops.adaptive_jasmin_mean(res["jas_ring"], res["jas_count"]).mean()
+            else:
+                out["jasmin_loss"] = self.jasmin_loss([], k=jasmin_k, reduction="mean")
         if self.add_distillation_token:
             out["logits_dist"] = self.dist_head(final[:, 1])
         if labels is not None:
